@@ -2,6 +2,7 @@
 """Benchmark of the batch-SOM training epoch (BASELINE.json metric: training samples/s per epoch).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c4|c2|small] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one full training epoch (BMU search -> per-BMU accumulation -> [all-reduce] ->
 neighbourhood smoothing -> read-back of per-neuron error/count/change) of a fixed side x side map on
@@ -18,6 +19,11 @@ Workloads (SURVEY.md section 8(d)); `c3` is the default at every GPU count (weak
 
 `--impl reference` times the CPU restatement of the reference's epoch (oracle/, numpy + the same
 scikit-learn call the reference makes) on the host cores, on a bounded row sample of the workload.
+
+`--dump-outputs DIR` writes what the last timed epoch computed to DIR/<name>.npy (float64): per-neuron `error`
+and `counts`, `change`, the updated prototypes `weights` and the winners of the samples `winners` (rank 0's shard).
+The inputs depend only on the arguments, so two builds can be compared output for output.  Outputs larger than
+their share of 48 MB are a fixed, seeded row sample; the sampled row indices are written as `<name>_rows.npy`.
 """
 import argparse
 import json
@@ -42,6 +48,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # nothing is written into the tree the benchmark runs from (it may be read-only)
 
 WORKLOADS = {
     #          rows per GPU (None = total/gpus), total rows, D, side, mixture components
@@ -290,6 +297,29 @@ def timed_epochs(torch, eng, m, steps, warmup, device, world, epoch0=0, sampler=
     return res
 
 
+DUMP_WEIGHT_VALUES = 4 << 20   # 32 MB of float64 prototypes
+DUMP_WINNER_ROWS = 1 << 20     # 8 MB of winners + 8 MB of their row indices
+
+
+def dump_outputs(path, eng, out):
+    """Write the result of the engine's last epoch (`out` is what `epoch` returned) to path/<name>.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"error": out["error"], "counts": out["counts"], "change": np.array([out["change"]])}
+    W = eng.weights()
+    if W.size > DUMP_WEIGHT_VALUES:
+        arrays["weights_rows"] = np.sort(np.random.default_rng(1).choice(W.shape[0], DUMP_WEIGHT_VALUES // W.shape[1],
+                                                                        replace=False))
+        W = W[arrays["weights_rows"]]
+    arrays["weights"] = W
+    win = eng.idx.view(-1)[: eng.N]
+    if eng.N > DUMP_WINNER_ROWS:
+        arrays["winners_rows"] = np.sort(np.random.default_rng(2).choice(eng.N, DUMP_WINNER_ROWS, replace=False))
+        win = win[eng.torch.from_numpy(arrays["winners_rows"]).to(win.device)]
+    arrays["winners"] = win.cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def k1_time_ms(phases):
     """Whole BMU search per epoch: candidate kernel(s) + second stage + exact re-score (everything between the
     prototype shadows and the final winner indices)."""
@@ -406,6 +436,8 @@ def run_ours(args, wl):
     res = timed_epochs(torch, eng, m, args.steps, args.warmup, device, world, sampler=ClockSampler(local))
     elapsed_ms, launches, bmu_stats, phases, clocks, out = (res[k_] for k_ in ("elapsed_ms", "launches", "bmu_stats", "phases", "clocks", "out"))
     epoch = res["epoch"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, out)  # before the end-to-end leg trains the map further
     ms_per_step = elapsed_ms / args.steps
     value = n_global * args.steps / (elapsed_ms * 1e-3)
 
@@ -586,7 +618,12 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the config-4 strong-scaling sub-record")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity check of the sharded epoch")
     ap.add_argument("--no-fit", action="store_true", help="skip the config-2 fit-level record")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 0)
     wl = WORKLOADS[args.workload]
     args.out = _stdout_for_json_only()

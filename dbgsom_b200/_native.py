@@ -13,7 +13,8 @@ _LIB = None
 LIB_NAME = "libdbgsom_b200.so"
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), LIB_NAME)
 
-ABI_VERSION = 8
+ABI_VERSION = 9
+COLSTATS_PARTS = 256  # DBGSOM_COLSTATS_PARTS
 SELECT_OFF, SELECT_FLAG, SELECT_REFINE = 0, 1, 2
 MAX_CAND = 8
 BMU_SIMT = 0
@@ -138,7 +139,7 @@ SIGNATURES = {
     "dbgsom_bmu": (c_int, [C.POINTER(BmuArgs), c_void_p]),
     "dbgsom_bmu_candidates": (c_int, [C.POINTER(BmuArgs), c_void_p]),
     "dbgsom_bmu_resolve": (c_int, [C.POINTER(BmuArgs), c_void_p]),
-    "dbgsom_accumulate_workspace_bytes": (c_size_t, [c_int64, c_int32]),
+    "dbgsom_accumulate_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32]),
     "dbgsom_accumulate": (c_int, [C.POINTER(AccumulateArgs), c_void_p]),
     "dbgsom_smooth_workspace_bytes": (c_size_t, [c_int32, c_int32]),
     "dbgsom_smooth": (c_int, [C.POINTER(SmoothArgs), c_void_p]),

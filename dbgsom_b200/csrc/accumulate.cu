@@ -13,9 +13,12 @@
 // The accumulate kernel gives every team of warps one contiguous range of the permutation; the
 // team keeps the current segment's float64 prototype in registers (so the exact distance
 // ||x_i - w_b|| costs no extra memory traffic), accumulates k_i x_i in float64 registers and
-// flushes with float64 atomics whenever the segment changes.  Everything after the fp32 load
-// of x is float64, so the result is independent of the (atomic-ordered) permutation up to
-// 1e-16 and matches the reference to ~1e-13; its convergence test (sum ||dW|| < 1e-5,
+// flushes whenever the segment changes: the segment's first team stores its sums, teams that
+// continue it leave theirs to acc_cont_kernel, which adds them in team order.  With the stable
+// permutation every sum is taken in the same order on every run, so the result is bitwise
+// repeatable (the fit is chaotic where prototypes collapse: a last-bit difference flips a near-tie
+// winner and grows from there).  Everything after the fp32 load of x is float64 and matches the
+// reference to ~1e-13; its convergence test (sum ||dW|| < 1e-5,
 // dbgsom/BaseSom.py:519-522) needs that: with fp32 weights or partial sums the prototypes jitter
 // by ~1e-7 relative from epoch to epoch and the fit stops at a different epoch (or never).
 // B200 has the float64 rate for this (~3 DFMA per sample element, far below the HBM time).  The M x D table is never privatised in
@@ -137,36 +140,109 @@ __global__ void __launch_bounds__(SCAT_THREADS) scatter_kernel(const int32_t* __
   }
 }
 
-// Block-local counting sort for maps of 512 .. 24576 neurons: a CTA takes a chunk of samples, counts
-// its winners in shared memory, reserves one contiguous run per (chunk, winner) with ONE global atomic,
-// then hands out the slots with shared-memory atomics.  The per-sample global atomics of
-// scatter_kernel (10M on 4096 addresses at config 3, 0.53 ms) become <= M per chunk.
-constexpr int SCAT2_THREADS = 1024;
-__global__ void __launch_bounds__(SCAT2_THREADS) scatter_chunk_kernel(const int32_t* __restrict__ bmu, int64_t N, int M,
-                                                                     const int32_t* __restrict__ offsets,
-                                                                     int32_t* __restrict__ cursor,
-                                                                     int32_t* __restrict__ perm, int64_t chunk) {
-  extern __shared__ int32_t sc_smem[];  // [M] local counts / cursors, [M] global base of this chunk's run
-  int32_t* lcount = sc_smem;
-  int32_t* lbase = sc_smem + M;
-  const int64_t c0 = (int64_t)blockIdx.x * chunk;
-  const int64_t c1 = c0 + chunk < N ? c0 + chunk : N;
-  for (int j = threadIdx.x; j < M; j += SCAT2_THREADS) lcount[j] = 0;
-  __syncthreads();
-  for (int64_t i = c0 + threadIdx.x; i < c1; i += SCAT2_THREADS) {
+// Stable counting sort for maps of up to STABLE_MAX_M neurons: perm lists the samples of each winner in
+// ascending sample index, so the order K2 sums in -- and the sample order the selective search rebuilds its
+// shadows in -- is the same on every run.  Each warp owns one contiguous chunk of samples:
+//   stable_count_kernel  T[c][j] = samples of chunk c won by j (per-warp table in shared memory);
+//   stable_base_kernel   T[c][j] = offsets[j] + sum_{c' < c} T[c'][j] (in place, one column per thread);
+//   stable_place_kernel  the warp walks its chunk in index order, 32 samples at a time, and hands out the
+//                        slots of its run per winner (lanes that share a winner: in lane order).
+constexpr int STABLE_MAX_M = 24576;
+constexpr int STABLE_MAX_CHUNKS = 148 * 8;
+constexpr int STABLE_SMEM = 64 * 1024;  // per CTA: warps * M counters
+constexpr int STABLE_PREFETCH = 8;      // 32-sample groups loaded ahead by the placing warp
+
+struct StableChunks {
+  int64_t chunk, n;  // samples per warp, number of warps (chunks)
+  int warps;         // warps per CTA
+};
+__host__ __device__ inline int64_t stable_max_chunks(int64_t N) {
+  const int64_t c = (N + 2047) / 2048;
+  return c < 1 ? 1 : (c > STABLE_MAX_CHUNKS ? STABLE_MAX_CHUNKS : c);
+}
+inline StableChunks stable_chunks(int64_t N, int M) {
+  StableChunks s;
+  const int64_t want = stable_max_chunks(N);
+  s.chunk = round_up<int64_t>(ceil_div<int64_t>(N, want), 32 * STABLE_PREFETCH);
+  s.n = ceil_div<int64_t>(N, s.chunk);
+  if (s.n < 1) s.n = 1;
+  int w = STABLE_SMEM / (M * 4);
+  s.warps = w < 1 ? 1 : (w > 8 ? 8 : w);
+  return s;
+}
+
+__global__ void stable_count_kernel(const int32_t* __restrict__ bmu, int64_t N, int M, int64_t chunk, int64_t n_chunks,
+                                    int32_t* __restrict__ T) {
+  extern __shared__ int32_t st_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t c = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
+  if (c >= n_chunks) return;
+  int32_t* cnt = st_smem + (size_t)warp * M;
+  for (int j = lane; j < M; j += 32) cnt[j] = 0;
+  __syncwarp();
+  const int64_t c0 = c * chunk, c1 = c0 + chunk < N ? c0 + chunk : N;
+  for (int64_t i = c0 + lane; i < c1; i += 32) {
     const int b = bmu[i];
-    if ((unsigned)b < (unsigned)M) atomicAdd(&lcount[b], 1);
+    if ((unsigned)b < (unsigned)M) atomicAdd(&cnt[b], 1);
   }
+  __syncwarp();
+  for (int j = lane; j < M; j += 32) T[c * M + j] = cnt[j];
+}
+
+__global__ void __launch_bounds__(1024) stable_base_kernel(int32_t* __restrict__ T, int64_t n_chunks, int M,
+                                                          const int32_t* __restrict__ offsets) {
+  __shared__ int32_t tot[32][33];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int j = blockIdx.x * 32 + lane;
+  const int64_t r0 = n_chunks * w / 32, r1 = n_chunks * (w + 1) / 32;
+  int32_t s = 0;
+  if (j < M)
+    for (int64_t r = r0; r < r1; ++r) s += T[r * M + j];
+  tot[w][lane] = s;
   __syncthreads();
-  for (int j = threadIdx.x; j < M; j += SCAT2_THREADS) {
-    const int c = lcount[j];
-    lbase[j] = c ? offsets[j] + atomicAdd(&cursor[j], c) : 0;
-    lcount[j] = 0;
+  if (j < M) {
+    int32_t run = offsets[j];
+    for (int q = 0; q < w; ++q) run += tot[q][lane];
+    for (int64_t r = r0; r < r1; ++r) {
+      const int32_t c = T[r * M + j];
+      T[r * M + j] = run;
+      run += c;
+    }
   }
-  __syncthreads();
-  for (int64_t i = c0 + threadIdx.x; i < c1; i += SCAT2_THREADS) {
-    const int b = bmu[i];
-    if ((unsigned)b < (unsigned)M) perm[lbase[b] + atomicAdd(&lcount[b], 1)] = (int32_t)i;
+}
+
+__global__ void stable_place_kernel(const int32_t* __restrict__ bmu, int64_t N, int M, int64_t chunk, int64_t n_chunks,
+                                    const int32_t* __restrict__ T, int32_t* __restrict__ perm) {
+  extern __shared__ int32_t st_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t c = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
+  if (c >= n_chunks) return;
+  int32_t* base = st_smem + (size_t)warp * M;
+  for (int j = lane; j < M; j += 32) base[j] = T[c * M + j];
+  __syncwarp();
+  const int64_t c0 = c * chunk, c1 = c0 + chunk < N ? c0 + chunk : N;
+  const unsigned lt = (1u << lane) - 1u;
+  for (int64_t s = c0; s < c1; s += 32 * STABLE_PREFETCH) {
+    int bb[STABLE_PREFETCH];
+#pragma unroll
+    for (int k = 0; k < STABLE_PREFETCH; ++k) {
+      const int64_t i = s + k * 32 + lane;
+      bb[k] = i < c1 ? bmu[i] : -1;
+    }
+#pragma unroll
+    for (int k = 0; k < STABLE_PREFETCH; ++k) {
+      const int b = (unsigned)bb[k] < (unsigned)M ? bb[k] : -1;
+      const unsigned peers = __match_any_sync(kFullMask, b);
+      const int leader = __ffs(peers) - 1;
+      int pos = 0;
+      if (b >= 0 && lane == leader) {
+        pos = base[b];
+        base[b] = pos + __popc(peers);
+      }
+      pos = __shfl_sync(kFullMask, pos, leader);
+      if (b >= 0) perm[pos + __popc(peers & lt)] = (int32_t)(s + k * 32 + lane);
+      __syncwarp();
+    }
   }
 }
 
@@ -215,7 +291,7 @@ template <int VPL, int WPR, int U, int THREADS, int STAGES, bool FULLD, int XU>
 __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     const float* __restrict__ X, int64_t N, int D, int64_t ldx, const int32_t* __restrict__ perm,
     const int32_t* __restrict__ offsets, const double* __restrict__ W, int M, double inv_var,
-    double* __restrict__ part) {
+    double* __restrict__ part, double* __restrict__ cont, int32_t* __restrict__ cont_seg) {
   constexpr int TEAMS = THREADS / 32 / WPR;
   constexpr int SLOT_BYTES = U * VPL * 512;          // one batch of one warp
   constexpr int WARP_BYTES = STAGES * SLOT_BYTES + VPL * 1024 + ACC_WIN_BYTES;
@@ -327,15 +403,21 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     run_d = 0.0;
   };
   auto flush = [&]() {
+    // a segment begun by an earlier team: this team's partial goes to cont[team] and acc_cont_kernel adds the
+    // partials of all continuing teams, in team order, to the one the segment's first team stored (recomputed here,
+    // once per segment, rather than kept live through the row loop)
+    const int64_t t_id = (int64_t)blockIdx.x * TEAMS + (threadIdx.x >> 5) / WPR;
+    const bool to_cont = offsets[seg] < (int32_t)((int64_t)offsets[M] * t_id / ((int64_t)gridDim.x * TEAMS));
+    double* cdst = cont + t_id * (D + 2);
 #pragma unroll
     for (int v = 0; v < VPL; ++v) {
       const int c = col0 + v * 128;
       if (act[v]) {
-        double* dst = Sk + (int64_t)seg * D + c;
-        atomicAdd(dst + 0, acc[v][0]);
-        atomicAdd(dst + 1, acc[v][1]);
-        atomicAdd(dst + 2, acc[v][2]);
-        atomicAdd(dst + 3, acc[v][3]);
+        double* dst = to_cont ? cdst + c : Sk + (int64_t)seg * D + c;
+        dst[0] = acc[v][0];  // the only writer of these entries (part is zeroed before the launch)
+        dst[1] = acc[v][1];
+        dst[2] = acc[v][2];
+        dst[3] = acc[v][3];
       }
     }
     // every row slot is evaluated by 32 / U lanes with identical results: count each slot once
@@ -343,8 +425,14 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     const double tk = warp_sum(slot_leader ? run_k : 0.0);
     const double td = warp_sum(slot_leader ? run_d : 0.0);
     if (tw == 0 && lane == 0) {
-      atomicAdd(part + (int64_t)M * D + seg, tk);              // sk
-      atomicAdd(part + (int64_t)M * D + 2 * (int64_t)M + seg, td);  // E
+      if (to_cont) {
+        cdst[D] = tk;
+        cdst[D + 1] = td;
+        cont_seg[t_id] = seg;
+      } else {
+        part[(int64_t)M * D + seg] = tk;                      // sk
+        part[(int64_t)M * D + 2 * (int64_t)M + seg] = td;     // E
+      }
     }
   };
 
@@ -450,8 +538,38 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
   if (seg >= 0) flush();
 }
 
+// part[seg] += the partials of the teams that continued segment seg, summed in team order; one CTA per segment (the
+// CTA of its first continuing team).  cont_seg is -1 for a team that continued nothing, which includes teams with an
+// empty range (fewer samples than teams): those may sit between two teams that continue the same segment and must not
+// split its run.  Segments only grow with the team index, so skipping -1 entries never joins two different segments.
+__global__ void __launch_bounds__(256) acc_cont_kernel(const double* __restrict__ cont, const int32_t* __restrict__ cont_seg,
+                                                      int64_t n_teams, int M, int D, double* __restrict__ part) {
+  const int64_t t = blockIdx.x;
+  const int seg = cont_seg[t];
+  if (seg < 0) return;
+  for (int64_t u = t - 1; u >= 0; --u) {
+    const int q = cont_seg[u];
+    if (q == seg) return;  // an earlier team continues seg: its CTA sums the run
+    if (q >= 0) break;
+  }
+  for (int c = threadIdx.x; c < D + 2; c += blockDim.x) {
+    double sum = 0.0;
+    for (int64_t u = t; u < n_teams; ++u) {
+      const int q = cont_seg[u];
+      if (q == seg) sum += cont[u * (D + 2) + c];
+      else if (q >= 0) break;
+    }
+    double* dst = c < D ? part + (int64_t)seg * D + c
+                        : part + (int64_t)M * D + (c == D ? 0 : 2 * (int64_t)M) + seg;
+    *dst += sum;
+  }
+}
+
+constexpr int64_t ACC_MAX_TEAMS = 148 * 2 * 8;  // CTAs (<= 2 per SM) x teams per CTA (<= 8)
+
 template <int VPL, int WPR, int U, int XU = 1>
-int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, const int32_t* offsets, cudaStream_t s) {
+int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, const int32_t* offsets, double* cont,
+                      int32_t* cont_seg, cudaStream_t s) {
   // one warp per row (WPR = 1): 6 warps per CTA leave 168 registers per thread at two CTAs per SM, enough
   // for the U * VPL * 4 converted elements + prototype + sums without spilling (at 128 registers the
   // loop-carried cursors spilled and every iteration stalled on local-memory loads); teams need 8 warps
@@ -470,8 +588,13 @@ int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, cons
   const int64_t useful = ceil_div<int64_t>(ceil_div<int64_t>(a.N, 4 * U), TEAMS);  // >= 4 batches per team
   if (blocks > useful) blocks = useful;
   if (blocks < 1) blocks = 1;
+  const int64_t n_teams = blocks * TEAMS;
+  static_assert(TEAMS <= 8, "ACC_MAX_TEAMS");
+  DBGSOM_CUDA_TRY(cudaMemsetAsync(cont_seg, 0xff, (size_t)n_teams * 4, s));
   kern<<<(unsigned)blocks, THREADS, smem, s>>>(a.d_X, a.N, a.D, a.ldx, perm, offsets, a.d_W, a.M,
-                                              a.inv_total_variance, a.d_part);
+                                              a.inv_total_variance, a.d_part, cont, cont_seg);
+  DBGSOM_LAUNCH_CHECK();
+  acc_cont_kernel<<<(unsigned)n_teams, 256, 0, s>>>(cont, cont_seg, n_teams, a.M, a.D, a.d_part);
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
 }
@@ -480,10 +603,18 @@ int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, cons
 
 struct AccWorkspace {
   int32_t *counts, *offsets, *cursor, *perm;
-  static size_t bytes(int64_t N, int M) {
-    return 3 * round_up<size_t>((size_t)(M + 1) * 4, 256) + round_up<size_t>((size_t)N * 4, 256);
+  int32_t* chunk_table;  // stable scatter: [chunks, M] (dead once perm is built; shares its space with cont)
+  double* cont;          // [ACC_MAX_TEAMS, D + 2] partials of teams that continue a segment
+  int32_t* cont_seg;     // [ACC_MAX_TEAMS]
+  static size_t shared_bytes(int64_t N, int M, int D) {
+    const size_t table = M <= STABLE_MAX_M ? (size_t)stable_max_chunks(N) * M * 4 : 0;
+    const size_t c = round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 2) * 8, 256) + (size_t)ACC_MAX_TEAMS * 4;
+    return round_up<size_t>(table > c ? table : c, 256);
   }
-  static AccWorkspace carve(void* base, int64_t N, int M) {
+  static size_t bytes(int64_t N, int M, int D) {
+    return 3 * round_up<size_t>((size_t)(M + 1) * 4, 256) + round_up<size_t>((size_t)N * 4, 256) + shared_bytes(N, M, D);
+  }
+  static AccWorkspace carve(void* base, int64_t N, int M, int D) {
     AccWorkspace w;
     uint8_t* p = reinterpret_cast<uint8_t*>(base);
     const size_t sm = round_up<size_t>((size_t)(M + 1) * 4, 256);
@@ -491,18 +622,22 @@ struct AccWorkspace {
     w.offsets = reinterpret_cast<int32_t*>(p + sm);
     w.cursor = reinterpret_cast<int32_t*>(p + 2 * sm);
     w.perm = reinterpret_cast<int32_t*>(p + 3 * sm);
+    uint8_t* q = p + 3 * sm + round_up<size_t>((size_t)N * 4, 256);
+    w.chunk_table = reinterpret_cast<int32_t*>(q);
+    w.cont = reinterpret_cast<double*>(q);
+    w.cont_seg = reinterpret_cast<int32_t*>(q + round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 2) * 8, 256));
     return w;
   }
 };
 
-size_t accumulate_workspace_bytes(int64_t N, int M) { return AccWorkspace::bytes(N, M); }
+size_t accumulate_workspace_bytes(int64_t N, int M, int D) { return AccWorkspace::bytes(N, M, D); }
 size_t accumulate_perm_offset(int64_t N, int M) {
   (void)N;
   return 3 * round_up<size_t>((size_t)(M + 1) * 4, 256);
 }
 
 int run_accumulate(const dbgsom_accumulate_args& a, cudaStream_t s) {
-  const AccWorkspace ws = AccWorkspace::carve(a.d_workspace, a.N, a.M);
+  const AccWorkspace ws = AccWorkspace::carve(a.d_workspace, a.N, a.M, a.D);
   const int64_t M = a.M, D = a.D;
   DBGSOM_CUDA_TRY(cudaMemsetAsync(a.d_part, 0, (size_t)(M * D + 3 * M) * sizeof(double), s));
   DBGSOM_CUDA_TRY(cudaMemsetAsync(ws.counts, 0, (size_t)(M + 1) * 4, s));
@@ -525,17 +660,19 @@ int run_accumulate(const dbgsom_accumulate_args& a, cudaStream_t s) {
   }
   scan_kernel<<<1, SCAN_THREADS, 0, s>>>(ws.counts, a.M, ws.offsets, ws.cursor, a.d_part + M * D + M);
   DBGSOM_LAUNCH_CHECK();
-  if (a.M >= 512 && a.M <= 24576 && a.N >= (1 << 18)) {
-    const size_t smem = (size_t)a.M * 8;
-    DBGSOM_CUDA_TRY(cudaFuncSetAttribute(scatter_chunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // one wave: two resident CTAs per SM (one when the tables need more than half the shared memory)
-    const int64_t slots = 148 * (smem <= 100 * 1024 ? 2 : 1);
-    int64_t chunk = round_up<int64_t>(ceil_div<int64_t>(a.N, slots), SCAT2_THREADS);
-    if (chunk < 16384) chunk = 16384;
-    scatter_chunk_kernel<<<(unsigned)ceil_div<int64_t>(a.N, chunk), SCAT2_THREADS, smem, s>>>(
-        a.d_bmu, a.N, a.M, ws.offsets, ws.cursor, ws.perm, chunk);
+  if (a.M <= STABLE_MAX_M) {
+    const StableChunks sc = stable_chunks(a.N, a.M);
+    const size_t smem = (size_t)sc.warps * a.M * 4;
+    const unsigned ctas = (unsigned)ceil_div<int64_t>(sc.n, sc.warps);
+    DBGSOM_CUDA_TRY(cudaFuncSetAttribute(stable_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DBGSOM_CUDA_TRY(cudaFuncSetAttribute(stable_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    stable_count_kernel<<<ctas, sc.warps * 32, smem, s>>>(a.d_bmu, a.N, a.M, sc.chunk, sc.n, ws.chunk_table);
     DBGSOM_LAUNCH_CHECK();
-  } else {
+    stable_base_kernel<<<(unsigned)ceil_div(a.M, 32), 1024, 0, s>>>(ws.chunk_table, sc.n, a.M, ws.offsets);
+    DBGSOM_LAUNCH_CHECK();
+    stable_place_kernel<<<ctas, sc.warps * 32, smem, s>>>(a.d_bmu, a.N, a.M, sc.chunk, sc.n, ws.chunk_table, ws.perm);
+    DBGSOM_LAUNCH_CHECK();
+  } else {  // maps too large for the per-warp tables: slots in arrival order
     int64_t blocks = ceil_div<int64_t>(a.N, SCAT_THREADS * 4);
     if (blocks > 148 * 16) blocks = 148 * 16;
     scatter_kernel<<<(unsigned)blocks, SCAT_THREADS, 0, s>>>(a.d_bmu, a.N, a.M, ws.offsets, ws.cursor, ws.perm);
@@ -551,23 +688,23 @@ int run_accumulate(const dbgsom_accumulate_args& a, cudaStream_t s) {
   static const char* tune_xu = getenv("DBGSOM_ACC_XU");
   const int xu = tune_xu ? atoi(tune_xu) : 4;
   if (D4 <= 128) {
-    if (u_small == 4) return launch_accumulate<1, 1, 4>(a, ws.perm, ws.offsets, s);
-    if (xu >= 4) return launch_accumulate<1, 1, 8, 4>(a, ws.perm, ws.offsets, s);
-    if (xu == 3) return launch_accumulate<1, 1, 8, 3>(a, ws.perm, ws.offsets, s);
-    if (xu == 2) return launch_accumulate<1, 1, 8, 2>(a, ws.perm, ws.offsets, s);
-    return launch_accumulate<1, 1, 8>(a, ws.perm, ws.offsets, s);
+    if (u_small == 4) return launch_accumulate<1, 1, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu >= 4) return launch_accumulate<1, 1, 8, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 3) return launch_accumulate<1, 1, 8, 3>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 2) return launch_accumulate<1, 1, 8, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    return launch_accumulate<1, 1, 8>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   }
   if (D4 <= 256) {
-    if (u_small == 2) return launch_accumulate<2, 1, 2>(a, ws.perm, ws.offsets, s);
-    if (xu >= 4) return launch_accumulate<2, 1, 4, 4>(a, ws.perm, ws.offsets, s);
-    if (xu == 3) return launch_accumulate<2, 1, 4, 3>(a, ws.perm, ws.offsets, s);
-    if (xu == 2) return launch_accumulate<2, 1, 4, 2>(a, ws.perm, ws.offsets, s);
-    return launch_accumulate<2, 1, 4>(a, ws.perm, ws.offsets, s);
+    if (u_small == 2) return launch_accumulate<2, 1, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu >= 4) return launch_accumulate<2, 1, 4, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 3) return launch_accumulate<2, 1, 4, 3>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 2) return launch_accumulate<2, 1, 4, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    return launch_accumulate<2, 1, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   }
-  if (D4 <= 512) return launch_accumulate<4, 1, 2>(a, ws.perm, ws.offsets, s);
-  if (D4 <= 1024) return launch_accumulate<4, 2, 2>(a, ws.perm, ws.offsets, s);
-  if (D4 <= 2048) return launch_accumulate<4, 4, 2>(a, ws.perm, ws.offsets, s);
-  if (D4 <= 4096) return launch_accumulate<4, 8, 2>(a, ws.perm, ws.offsets, s);
+  if (D4 <= 512) return launch_accumulate<4, 1, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 1024) return launch_accumulate<4, 2, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 2048) return launch_accumulate<4, 4, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 4096) return launch_accumulate<4, 8, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   return DBGSOM_E_UNSUPPORTED;
 }
 

@@ -14,7 +14,7 @@ int run_tile_bounds(const double*, int, int, const double*, float, const int32_t
 int run_prepare_bias(const float*, int, const float*, uint16_t*, float*, cudaStream_t);
 int run_row_ops(double*, int, const int32_t*, int, cudaStream_t);
 int run_gather_rows(const float*, int64_t, int, const int64_t*, int, double*, cudaStream_t);
-size_t accumulate_workspace_bytes(int64_t, int);
+size_t accumulate_workspace_bytes(int64_t, int, int);
 int run_accumulate(const dbgsom_accumulate_args&, cudaStream_t);
 size_t smooth_workspace_bytes(int, int);
 int run_smooth(const dbgsom_smooth_args&, cudaStream_t);
@@ -160,7 +160,7 @@ int dbgsom_bmu(const dbgsom_bmu_args* a, void* stream) {
   return dbgsom_bmu_resolve(a, stream);
 }
 
-size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M) { return accumulate_workspace_bytes(N, M); }
+size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M, int32_t D) { return accumulate_workspace_bytes(N, M, D); }
 size_t dbgsom_accumulate_perm_offset(int64_t N, int32_t M) { return accumulate_perm_offset(N, M); }
 
 int dbgsom_accumulate(const dbgsom_accumulate_args* a, void* stream) {
@@ -169,7 +169,7 @@ int dbgsom_accumulate(const dbgsom_accumulate_args* a, void* stream) {
     return DBGSOM_E_BADARG;
   if (a->N > 0x7fffffffLL) return DBGSOM_E_UNSUPPORTED;  // int32 permutation
   if (a->D % 4 != 0 || a->ldx % 4 != 0 || !aligned16(a->d_X) || !aligned16(a->d_W)) return DBGSOM_E_UNSUPPORTED;
-  if (a->workspace_bytes < accumulate_workspace_bytes(a->N, a->M)) return DBGSOM_E_WORKSPACE;
+  if (a->workspace_bytes < accumulate_workspace_bytes(a->N, a->M, a->D)) return DBGSOM_E_WORKSPACE;
   return run_accumulate(*a, as_stream(stream));
 }
 

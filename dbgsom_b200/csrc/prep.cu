@@ -6,8 +6,9 @@ namespace dbgsom {
 namespace {
 
 // ------------------------------------------------------------------------------------------ K4
-// moments[d] += sum_i (x_id - c_d), moments[D + d] += sum_i (x_id - c_d)^2 (float64),
-// moments[2D] = max |x_id - c_d|.
+// Part r = blockIdx.y of moments ([DBGSOM_COLSTATS_PARTS][2D + 1]) gets the rows of row block r:
+// [d] = sum_i (x_id - c_d), [D + d] = sum_i (x_id - c_d)^2 (float64), [2D] = max |x_id - c_d| over its columns.
+// No atomics: the caller adds the parts in order, so the statistics are the same on every run.
 // Replaces np.var(data, axis=0) / np.std(data, axis=0, ddof=1), dbgsom/BaseSom.py:363, :380.
 // Shifting by a data row keeps the one-pass variance free of cancellation.
 constexpr int CS_COLS = 32, CS_ROWS = 8;
@@ -41,10 +42,11 @@ __global__ void __launch_bounds__(CS_COLS * CS_ROWS) colstats_kernel(const float
       a2 += s2[q][cx];
       a3 = fmax(a3, s3[q][cx]);
     }
-    atomicAdd(&moments[d], a1);
-    atomicAdd(&moments[D + d], a2);
-    // non-negative doubles order like their bit patterns
-    atomicMax(reinterpret_cast<long long*>(&moments[2 * D]), __double_as_longlong(a3));
+    double* part = moments + (int64_t)blockIdx.y * (2 * D + 1);
+    part[d] = a1;
+    part[D + d] = a2;
+    // non-negative doubles order like their bit patterns (the column blocks of a part share this entry)
+    atomicMax(reinterpret_cast<long long*>(&part[2 * D]), __double_as_longlong(a3));
   }
 }
 
@@ -341,8 +343,7 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restric
 int run_colstats(const float* X, int64_t N, int D, int64_t ldx, const float* shift, double* moments, cudaStream_t s) {
   int64_t row_blocks = ceil_div<int64_t>(N, 4096);
   const int col_blocks = ceil_div(D, CS_COLS);
-  const int64_t cap = ceil_div<int64_t>(148 * 16, col_blocks);
-  if (row_blocks > cap) row_blocks = cap;
+  if (row_blocks > DBGSOM_COLSTATS_PARTS) row_blocks = DBGSOM_COLSTATS_PARTS;
   if (row_blocks < 1) row_blocks = 1;
   const int64_t rows_per_block = ceil_div<int64_t>(N, row_blocks);
   colstats_kernel<<<dim3(col_blocks, (unsigned)row_blocks), CS_COLS * CS_ROWS, 0, s>>>(X, N, D, ldx, shift, moments,

@@ -190,9 +190,9 @@ __global__ void __launch_bounds__(256, 2) smooth_gemm_kernel(const uint16_t* __r
   }
 }
 
-// change += ||W_in[i] - W_out[i]||_2, one warp per row
+// row_norm[i] = ||W_in[i] - W_out[i]||_2, one warp per row
 __global__ void __launch_bounds__(256) change_kernel(const double* __restrict__ W_in, const double* __restrict__ W_out,
-                                                    int row_begin, int row_end, int D, double* __restrict__ change) {
+                                                    int row_begin, int row_end, int D, double* __restrict__ row_norm) {
   const int lane = threadIdx.x & 31;
   const int i = row_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
   if (i >= row_end) return;
@@ -202,7 +202,25 @@ __global__ void __launch_bounds__(256) change_kernel(const double* __restrict__ 
     acc = fma(t, t, acc);
   }
   acc = warp_sum(acc);
-  if (lane == 0) atomicAdd(change, sqrt(acc));
+  if (lane == 0) row_norm[i] = sqrt(acc);
+}
+
+// change += sum of row_norm[row_begin:row_end], one CTA, in a fixed order (the same value on every run)
+constexpr int CHANGE_SUM_THREADS = 1024;
+__global__ void __launch_bounds__(CHANGE_SUM_THREADS) change_sum_kernel(const double* __restrict__ row_norm,
+                                                                       int row_begin, int row_end,
+                                                                       double* __restrict__ change) {
+  __shared__ double part[CHANGE_SUM_THREADS / 32];
+  double acc = 0.0;
+  for (int i = row_begin + threadIdx.x; i < row_end; i += CHANGE_SUM_THREADS) acc += row_norm[i];
+  acc = warp_sum(acc);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double total = 0.0;
+    for (int w = 0; w < CHANGE_SUM_THREADS / 32; ++w) total += part[w];
+    *change += total;
+  }
 }
 
 }  // namespace
@@ -258,7 +276,10 @@ int run_smooth(const dbgsom_smooth_args& a, cudaStream_t s) {
                                             r0, r1, D, a.d_W_out);
     DBGSOM_LAUNCH_CHECK();
   }
-  change_kernel<<<ceil_div(rows, 8), 256, 0, s>>>(a.d_W_in, a.d_W_out, r0, r1, D, a.d_change);
+  // the row norms go to ws.B (the GEMM above was its last reader)
+  change_kernel<<<ceil_div(rows, 8), 256, 0, s>>>(a.d_W_in, a.d_W_out, r0, r1, D, ws.B);
+  DBGSOM_LAUNCH_CHECK();
+  change_sum_kernel<<<1, CHANGE_SUM_THREADS, 0, s>>>(ws.B, r0, r1, a.d_change);
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
 }

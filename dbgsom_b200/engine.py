@@ -258,14 +258,17 @@ class DeviceEngine:
         # K4: moments about a common data row (rank 0's first row)
         shift_row = self.X[0].clone()
         self.comm.broadcast_(shift_row, 0)
-        moments = torch.zeros(2 * self.ldx + 1, dtype=torch.float64, device=self.dev)
+        parts = torch.zeros((nat.COLSTATS_PARTS, 2 * self.ldx + 1), dtype=torch.float64, device=self.dev)
         nat.check(
             self.lib.dbgsom_colstats(
-                self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), moments.data_ptr(), self._stream()
+                self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), parts.data_ptr(), self._stream()
             ),
             "dbgsom_colstats",
         )
         self.launches += 1
+        # the row-block parts are added on the host in a fixed order: the same statistics on every run
+        p = parts.cpu().numpy()
+        moments = torch.from_numpy(np.append(p[:, : 2 * self.ldx].sum(axis=0), p[:, 2 * self.ldx].max())).to(self.dev)
         self.comm.allreduce_(moments[: 2 * self.ldx])
         self.comm.allreduce_(moments[2 * self.ldx :], "max")
         m = moments.cpu().numpy()
@@ -770,11 +773,11 @@ class DeviceEngine:
         acc.d_labels = self.labels.data_ptr() if use_hist else None
         acc.n_classes = self.n_classes if use_hist else 0
         acc.d_class_hist = self.class_hist.data_ptr() if use_hist else None
-        ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(self.N, m))
+        ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(self.N, m, self.ldx))
         acc.d_workspace, acc.workspace_bytes = ws.data_ptr(), ws.numel()
         with self._Phase(self, "accumulate"):
             nat.check(self.lib.dbgsom_accumulate(acc, self._stream()), "dbgsom_accumulate")
-        self.launches += 6 + (1 if use_hist else 0)
+        self.launches += (10 if m <= 24576 else 8) + (1 if use_hist else 0)  # stable scatter: 3 kernels
         if resort and self.X16_hi is not None:
             self._sort_age += 1
             if self.row_perm is None or self._sort_age >= self.resort_every:
@@ -811,7 +814,7 @@ class DeviceEngine:
                 nat.check(self.lib.dbgsom_smooth(sm, self._stream()), "dbgsom_smooth")
             else:
                 self.change.zero_()
-        self.launches += 6
+        self.launches += 7
         if shard_rows:
             with self._Phase(self, "allgather"):
                 flat = out[: rows_per * world]

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define DBGSOM_ABI_VERSION 8
+#define DBGSOM_ABI_VERSION 9
 
 #define DBGSOM_OK 0
 #define DBGSOM_E_BADARG (-1)      /* null pointer, non-positive size, bad enum             */
@@ -64,12 +64,14 @@ int dbgsom_check_device(int device);
  * K4  column statistics (once per fit)
  * replaces  np.var(data, axis=0).sum()           dbgsom/BaseSom.py:363
  *           np.std(data, axis=0, ddof=1)         dbgsom/BaseSom.py:380
- * d_moments[0:D]  += sum_i (x_id - c_d),  d_moments[D:2D] += sum_i (x_id - c_d)^2 in float64,
- * d_moments[2D] = max(d_moments[2D], max_id |x_id - c_d|), with c = d_shift_row (float32 [D],
- * device; any data row works, all ranks must use the same one).  The caller zeroes d_moments
- * (2D+1 doubles), all-reduces it across GPUs when sharded (sum, max for the last entry) and
- * finishes the scalars on the host.
+ * d_moments is [DBGSOM_COLSTATS_PARTS][2D+1]; part r covers a fixed block of rows:
+ * part[0:D] = sum_i (x_id - c_d),  part[D:2D] = sum_i (x_id - c_d)^2 in float64,
+ * part[2D] = max(part[2D], max_id |x_id - c_d|), with c = d_shift_row (float32 [D],
+ * device; any data row works, all ranks must use the same one).  The caller zeroes d_moments,
+ * adds the parts in order (max for the last entry; a fixed order makes the result the same on
+ * every run), all-reduces the sum across GPUs when sharded and finishes the scalars on the host.
  */
+#define DBGSOM_COLSTATS_PARTS 256
 int dbgsom_colstats(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift_row,
                     double* d_moments, void* stream);
 
@@ -278,9 +280,11 @@ typedef struct dbgsom_accumulate_args {
   size_t workspace_bytes;
 } dbgsom_accumulate_args;
 
-size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M);
+size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M, int32_t D);
 /* Byte offset, inside the workspace of dbgsom_accumulate(N, M), of the int32 [N] sample permutation grouped by
- * winner (ascending winner index) that the call leaves behind. */
+ * winner (ascending winner index) that the call leaves behind.  For M <= 24576 the samples of a winner are in
+ * ascending sample index and the call's sums are the same on every run; above that the samples of a winner are
+ * in the order the scatter's atomics hand out, which varies between runs, and so do the last bits of the sums. */
 size_t dbgsom_accumulate_perm_offset(int64_t N, int32_t M);
 int dbgsom_accumulate(const dbgsom_accumulate_args* args, void* stream);
 

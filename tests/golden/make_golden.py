@@ -140,14 +140,16 @@ TRAJ_CASES = [
 
 # BASELINE.json configs[1] (SURVEY.md section 8(d)): SomClassifier on the Fashion-MNIST-shaped 70000 x 784 mixture
 # with ten classes.  n_iter is kept small enough for CI (the reference needs ~0.5 s per epoch here); the states of
-# `capture` epochs are stored in full, everything else as per-epoch records like the traj_* files.
+# `capture` epochs are stored in full, everything else as per-epoch records like the traj_* files.  A captured state
+# costs 0.2-0.6 MB (its float64 prototypes do not compress), so two are kept to hold the file under 1 MB: epoch 5 of
+# the growth phase and epoch 30 of the fine phase (sigma 0.7, near-equal prototypes, dead neurons below live ones).
 FITSTEP_CASES = [
     # cast float64 (float32-representable values, like the other fixtures): with float32 input the reference's
     # total variance is a float32 row-by-row accumulation over 70000 rows (np.var, dbgsom/BaseSom.py:363) whose ~1e-5
     # rounding noise this fit amplifies by flipping samples between near-equidistant prototypes -- from epoch 2 on the
     # trajectory then depends on numpy's summation order, which no other implementation can reproduce
     dict(name="c2_gmm784_clf", est="clf", data="gmm:70000:784:10:21:float32", cast="float64",
-         params=dict(random_state=7, n_iter=36, max_neurons=400), capture=[5, 11, 17, 18, 30]),
+         params=dict(random_state=7, n_iter=36, max_neurons=400), capture=[5, 30]),
 ]
 
 

@@ -51,7 +51,7 @@ def test_argument_errors_do_not_touch_the_gpu(lib):
     assert lib.dbgsom_apply_row_ops(None, 4, None, 0, None) == -1
     assert lib.dbgsom_gather_rows(None, 4, 4, None, 0, None, None) == -1
     assert lib.dbgsom_bmu_workspace_bytes(1000, 1) >= 1000 * (4 * nat.MAX_CAND + 1)
-    assert lib.dbgsom_accumulate_workspace_bytes(1000, 16) >= 4000
+    assert lib.dbgsom_accumulate_workspace_bytes(1000, 16, 4) >= 4000
     assert lib.dbgsom_smooth_workspace_bytes(16, 8) >= 16 * 8 * 8
 
 

@@ -686,6 +686,63 @@ def test_config2_fit_follows_the_reference_trajectory(path, backend):
     assert est.score(X[:5000], y[:5000]) >= 0.0  # the sparse-coding inference path runs at this shape
 
 
+@pytest.mark.parametrize("n", [3, 4])
+@pytest.mark.parametrize("backend", ["simt", "tensor"])
+def test_one_prototype_wins_every_sample_of_a_tiny_set(n, backend):
+    """Fewer samples than K2 has teams of warps: most teams have an empty range, and the teams that continue the one
+    segment sit between empty ones.  Counts, errors and prototypes must still be the oracle's."""
+    rng = np.random.default_rng(n)
+    X = rng.normal(size=(n, 8)).astype(np.float32).astype(np.float64)
+    W = np.concatenate([X.mean(axis=0, keepdims=True), 50.0 + rng.normal(size=(3, 8))])
+    hop = O.hop_matrix_grid(2, 2).astype(np.float64)
+    stats, r, W_new = run_epoch(X, W, hop, 1.0, True, backend)
+    assert np.array_equal(r["winners"], np.zeros(n, dtype=np.int64))
+    ref = O.epoch_step(X, W, hop, 1.0, stats["total_variance"], pack=True)
+    np.testing.assert_array_equal(r["counts"], ref["n"])
+    np.testing.assert_allclose(r["error"], ref["E"], rtol=1e-12, atol=1e-12)
+    assert np.abs(W_new - ref["W_new"]).max() / np.abs(ref["W_new"]).max() < 1e-12
+
+
+@pytest.mark.parametrize("n,d,gx,gy", [
+    (300_000, 64, 16, 16),    # the sorted sample order feeds the selective search from the second epoch on
+    (20_000, 768, 8, 8),      # D > 512: teams of several warps in K2
+    (60_000, 16, 100, 100),   # M > 8192: one warp per CTA in the stable scatter
+    (5, 8, 2, 2),             # fewer samples than K2 has teams
+], ids=["selective", "wide_teams", "large_map", "tiny"])
+def test_epochs_repeat_bit_for_bit(n, d, gx, gy):
+    """Two engines on the same data and start produce the same prototypes, errors and counts, bit for bit, epoch after
+    epoch: every sum is taken in a fixed order, and K2's permutation lists the samples of each winner in ascending
+    sample index (maps of up to 24576 neurons)."""
+    import torch
+
+    from dbgsom_b200.topology import MapTopology
+
+    X = _datasets.gmm(n, d, 16, 7)
+    m = gx * gy
+    runs = []
+    for _ in range(2):
+        e = engine(bmu_backend="tensor")
+        stats = e.load_data(X, None, 0)
+        e.init_map_from_rows(np.random.default_rng(3).choice(n, m, replace=n < m), capacity=m)
+        e.set_hops_from_topology(MapTopology.full_grid(gx, gy))
+        outs = []
+        for ep in range(4):
+            # sigma grows with the map, as in a fit: too narrow a neighbourhood leaves far rows with no weight (NaN)
+            r = e.epoch(max(2.0, 0.1 * gx) - 0.3 * ep, True, False)
+            outs.append((e.weights(), r["error"], r["counts"], r["change"]))
+        win = e.last_winners_host()
+        assert (win >= 0).all()
+        off = int(e.lib.dbgsom_accumulate_perm_offset(e.N, e.M))
+        perm = e._ws["acc"][off : off + 4 * e.N].view(torch.int32).cpu().numpy()
+        np.testing.assert_array_equal(perm, np.argsort(win, kind="stable"))
+        runs.append((stats["total_variance"], outs))
+        e.close()
+    assert runs[0][0] == runs[1][0]
+    for a, b in zip(runs[0][1], runs[1][1]):
+        for x, y in zip(a, b):
+            np.testing.assert_array_equal(x, y)
+
+
 def test_tile_bounds_are_the_column_tile_maxima():
     """dbgsom_tile_bounds: max ||u_j|| and max |wnorm_j| per 128 shadow columns, in the column order of the search,
     without padding columns and without prototypes taken out of the search (wnorm = +inf)."""

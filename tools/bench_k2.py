@@ -22,7 +22,7 @@ for s in range(0, n, 1 << 20):
 bmu = (torch.randint(0, live, (n,), device=dev, generator=g) * (m // live)).to(torch.int32)
 W = torch.randn(m, d, device=dev, generator=g, dtype=torch.float64)
 part = torch.zeros(m * d + 3 * m, dtype=torch.float64, device=dev)
-ws = torch.empty(lib.dbgsom_accumulate_workspace_bytes(n, m), dtype=torch.uint8, device=dev)
+ws = torch.empty(lib.dbgsom_accumulate_workspace_bytes(n, m, d), dtype=torch.uint8, device=dev)
 a = nat.AccumulateArgs()
 a.d_X, a.N, a.D, a.ldx = X.data_ptr(), n, d, d
 a.d_bmu, a.d_W, a.M = bmu.data_ptr(), W.data_ptr(), m
