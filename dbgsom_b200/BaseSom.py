@@ -20,7 +20,7 @@ from typing import Any
 import numpy as np
 from sklearn.base import BaseEstimator
 from sklearn.utils import check_array, check_random_state
-from sklearn.utils.validation import check_is_fitted
+from sklearn.utils.validation import _check_sample_weight, check_is_fitted
 
 from .topology import MapTopology
 
@@ -70,6 +70,11 @@ class BaseSom(BaseEstimator):
         SPMD multi-GPU: every rank calls `fit` with its own shard of the samples; only the
         per-neuron partial sums are all-reduced each epoch (`torch.distributed`, NCCL).  The start
         rows are drawn on rank 0 and broadcast, and `classes_` is the union over all shards.
+
+    `fit(X, y, sample_weight)` takes frequency weights like scikit-learn's `KMeans`: a sample of integer
+    weight w counts like w copies of it (fractional weights extend the same sums), zero removes it from
+    every sum of the fit while it still gets a winner in `labels_`.  The start prototypes are drawn among
+    the samples with positive weight.
     """
 
     def __init__(
@@ -168,10 +173,16 @@ class BaseSom(BaseEstimator):
             raise NotImplementedError("vertical_growth is not supported (broken in the reference, out of scope)")
 
     # ------------------------------------------------------------------ fit
-    def fit(self, X, y=None):
-        """Train the map on X (and y).  Same contract as dbgsom/BaseSom.py:88-131."""
+    def fit(self, X, y=None, sample_weight=None):
+        """Train the map on X (and y).  Same contract as dbgsom/BaseSom.py:88-131.
+
+        sample_weight : array of shape (n_samples,), default None
+            Frequency weights (finite, >= 0, at least four positive); None weighs every sample 1.
+        """
         self._check_arguments()
         X, y = self._check_input_data(X, y)
+        if sample_weight is not None:
+            sample_weight = self._check_sample_weight(sample_weight, X)
         if y is None and self.growth_criterion == "entropy":
             # the reference indexes `y[winners == j]` with y = None here (dbgsom/BaseSom.py:547-551) and dies with
             # a TypeError in the first epoch; say what is wrong instead of silently growing on another criterion
@@ -195,7 +206,7 @@ class BaseSom(BaseEstimator):
         self._host_hops_s = 0.0
         try:
             t0 = time.perf_counter()
-            self._initialize_som(engine, X, y)
+            self._initialize_som(engine, X, y, sample_weight)
             t1 = time.perf_counter()
             self._grow_som(engine)
             t2 = time.perf_counter()
@@ -216,25 +227,61 @@ class BaseSom(BaseEstimator):
         self.n_iter_ = self._current_epoch
         return self
 
-    def _initialize_som(self, engine, X: np.ndarray, y) -> None:
+    @staticmethod
+    def _check_sample_weight(sample_weight, X) -> np.ndarray:
+        """float64 weights of the rows of X: the right length, finite and non-negative."""
+        w = _check_sample_weight(sample_weight, X, dtype=np.float64, ensure_non_negative=True,
+                                 allow_all_zero_weights=True)
+        if not np.isfinite(w).all():
+            raise ValueError("sample_weight must be finite")
+        return np.ascontiguousarray(w, dtype=np.float64)
+
+    def _initialize_som(self, engine, X: np.ndarray, y, sample_weight=None) -> None:
         """`_initialize_som` + `_create_som`, dbgsom/BaseSom.py:352-369, :419-444."""
         self._current_epoch = 0
         self.converged_ = False
         self._training_phase = "coarse"
         self._neurons_added = True
         n_classes = len(self.classes_) if y is not None else 0
-        stats = engine.load_data(X, y, n_classes)
+        if sample_weight is None:
+            stats = engine.load_data(X, y, n_classes)
+        else:
+            stats = engine.load_data(X, y, n_classes, sample_weight=sample_weight)
+        # the amount of data the error means are taken over: the total weight of a weighted fit
+        self._n_total = stats.get("total_weight")
         self._total_variance = stats["total_variance"]
         self.growing_threshold_ = self._growing_threshold(stats, X.shape[1])
-        # identical draw to `rng.choice(a=data, size=4, replace=False)` (row choice)
-        rng = np.random.default_rng(seed=self.random_state)
-        rows = rng.choice(stats["n_samples"], size=4, replace=False)
-        if self._comm is not None:
-            # an unseeded (or per-rank different) generator would give every rank its own four rows
-            rows = np.asarray(self._comm.broadcast_object(rows, src=0))
+        rows = self._start_rows(stats["n_samples"], sample_weight, engine)
         self._topology = MapTopology.initial_square()
         engine.init_map_from_rows(rows, capacity=self._capacity_hint())
         self._hops_dirty = True
+
+    def _start_rows(self, n_samples: int, sample_weight, engine) -> np.ndarray:
+        """Global sample indices of the four start prototypes (dbgsom/BaseSom.py:423-430).
+
+        Unweighted: the draw of `rng.choice(a=data, size=4, replace=False)` (row choice).  Weighted: the same draw
+        over the rows with positive weight (in global order), so zero-weight rows never become prototypes and
+        all-positive weights give exactly the unweighted rows.  When sharded, rank 0 draws and every rank
+        resolves the positions that fall into its own shard; the others are -1 (owned by another rank)."""
+        rng = np.random.default_rng(seed=self.random_state)
+        if sample_weight is None:
+            rows = rng.choice(n_samples, size=4, replace=False)
+            if self._comm is not None:
+                # an unseeded (or per-rank different) generator would give every rank its own four rows
+                rows = np.asarray(self._comm.broadcast_object(rows, src=0))
+            return rows
+        positive = np.flatnonzero(sample_weight > 0)
+        pos_offset, n_pos = 0, positive.size
+        if self._comm is not None:
+            pos_offset, n_pos = self._comm.exclusive_offset(positive.size, getattr(self._comm, "device", None))
+        if n_pos < 4:
+            raise ValueError(f"sample_weight has {n_pos} positive entries; at least 4 are needed (one per start prototype)")
+        pick = rng.choice(n_pos, size=4, replace=False)
+        if self._comm is not None:
+            pick = np.asarray(self._comm.broadcast_object(pick, src=0))
+        local = pick - pos_offset
+        own = (local >= 0) & (local < positive.size)
+        return np.where(own, positive[np.where(own, local, 0)] + getattr(engine, "sample_offset", 0), -1)
 
     def _capacity_hint(self) -> int:
         # growth is only tested before a growth step (quirk Q8) so the map can overshoot
@@ -331,7 +378,7 @@ class BaseSom(BaseEstimator):
         # error and node statistics are measured against the prototypes BEFORE the final
         # update, while the graph (and the final `weights_`) carry the updated ones.
         st = engine.final_statistics(topo.positions(), topo.degrees())
-        n_total = engine.n_samples_global
+        n_total = engine.n_samples_global if self._n_total is None else self._n_total
         tf.append(time.perf_counter())
         # topographic error: grid distance of the two BMUs > 1.5 (dbgsom/BaseSom.py:924-953)
         self.topographic_error_ = st["te_count"] / n_total
@@ -408,12 +455,16 @@ class BaseSom(BaseEstimator):
         """Node attribute as an array in node order (dbgsom/BaseSom.py:237-239)."""
         return np.array([data[attribute] for _, data in self.som_.nodes.data()])
 
-    def calculate_quantization_error(self, X) -> float:
-        """Mean distance to the nearest prototype (dbgsom/BaseSom.py:904-922)."""
+    def calculate_quantization_error(self, X, sample_weight=None) -> float:
+        """Mean distance to the nearest prototype (dbgsom/BaseSom.py:904-922); weighted mean with `sample_weight`."""
         check_is_fitted(self)
         X = check_array(X)
+        if sample_weight is not None:
+            sample_weight = self._check_sample_weight(sample_weight, X)
         dist, _ = self._get_winning_neurons(X, n_bmu=1)
-        return float(np.mean(dist))
+        if sample_weight is None:
+            return float(np.mean(dist))
+        return float(np.average(dist, weights=sample_weight))
 
     def transform(self, X, y=None) -> np.ndarray:
         """Non-negative sparse code of each sample over the normalised prototypes.

@@ -13,7 +13,7 @@ _LIB = None
 LIB_NAME = "libdbgsom_b200.so"
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), LIB_NAME)
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 COLSTATS_PARTS = 256  # DBGSOM_COLSTATS_PARTS
 SELECT_OFF, SELECT_FLAG, SELECT_REFINE = 0, 1, 2
 MAX_CAND = 8
@@ -115,6 +115,7 @@ SIGNATURES = {
     "dbgsom_status_string": (C.c_char_p, [c_int]),
     "dbgsom_check_device": (c_int, [c_int]),
     "dbgsom_colstats": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
+    "dbgsom_colstats_weighted": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dbgsom_prepare_x16": (
         c_int,
         [c_void_p, c_int64, c_int, c_int64, c_void_p, c_float, c_void_p, c_void_p, c_int64, c_void_p, c_void_p],
@@ -141,6 +142,7 @@ SIGNATURES = {
     "dbgsom_bmu_resolve": (c_int, [C.POINTER(BmuArgs), c_void_p]),
     "dbgsom_accumulate_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32]),
     "dbgsom_accumulate": (c_int, [C.POINTER(AccumulateArgs), c_void_p]),
+    "dbgsom_accumulate_weighted": (c_int, [C.POINTER(AccumulateArgs), c_void_p, c_void_p, c_void_p]),
     "dbgsom_smooth_workspace_bytes": (c_size_t, [c_int32, c_int32]),
     "dbgsom_smooth": (c_int, [C.POINTER(SmoothArgs), c_void_p]),
     "dbgsom_apply_row_ops": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p]),
@@ -148,9 +150,19 @@ SIGNATURES = {
     "dbgsom_node_stats": (
         c_int, [c_void_p, c_int32, c_void_p, c_int32, c_int64, c_void_p, c_int32, c_double, c_void_p, c_void_p]
     ),
+    "dbgsom_node_stats_weighted": (
+        c_int,
+        [c_void_p, c_int32, c_void_p, c_int32, c_int64, c_void_p, c_int32, c_double, c_void_p, c_void_p, c_void_p],
+    ),
     "dbgsom_umatrix": (c_int, [c_void_p, c_int32, c_int32, c_int64, c_void_p, c_void_p, c_void_p]),
     "dbgsom_label_hist": (
         c_int, [c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
+    ),
+    "dbgsom_label_hist_weighted_workspace_bytes": (c_size_t, [c_int64, c_int32]),
+    "dbgsom_label_hist_weighted": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_size_t,
+         c_void_p],
     ),
     "dbgsom_hops": (c_int, [c_void_p, c_int32, c_void_p, c_int64, c_void_p]),
     "dbgsom_sparse_code_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32]),

@@ -72,7 +72,7 @@ __global__ void __launch_bounds__(HIST_THREADS) hist_kernel(const int32_t* __res
 }
 
 // ------------------------------------------------------------------------------------------ scan
-// single CTA: offsets[j] = sum_{i<j} counts[i], offsets[M] = total; n_j -> part_n as float64; cursor = 0
+// single CTA: offsets[j] = sum_{i<j} counts[i], offsets[M] = total; n_j -> part_n (if given) as float64; cursor = 0
 constexpr int SCAN_THREADS = 1024;
 __global__ void __launch_bounds__(SCAN_THREADS) scan_kernel(const int32_t* __restrict__ counts, int M,
                                                            int32_t* __restrict__ offsets,
@@ -108,7 +108,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_kernel(const int32_t* __res
     if (j < M) {
       offsets[j] = excl;
       cursor[j] = 0;
-      part_n[j] = (double)c;
+      if (part_n) part_n[j] = (double)c;
     }
     __syncthreads();
     if (threadIdx.x == SCAN_THREADS - 1) carry_sh = carry + warp_tot[31];
@@ -287,18 +287,27 @@ __device__ __forceinline__ double f32_as_f64(float f) {
 // instructions per 4-row batch were loop control.
 // All arithmetic is float64: distances by direct differences, k = 1 - sqrt(1 - exp(-d^2 / V))
 // literally as dbgsom/BaseSom.py:536-537, sums in float64 registers.
-template <int VPL, int WPR, int U, int THREADS, int STAGES, bool FULLD, int XU>
+// WGT (frequency weights, `weight` [N] float64): row i counts w_i times -- k_i, d_i and the count 1 of the row are
+// multiplied by w_i, and the segment's weight sum is flushed into the n slot of `part` (the scan's integer count is
+// overwritten).  Lane u of the issuing warp copies the weight of row u of the batch next to the staged rows, so the
+// weight arrives with the batch's commit group; its sample index is the ring's byte offset / row bytes (exact in
+// float64 for any N that fits the int32 permutation).
+template <int VPL, int WPR, int U, int THREADS, int STAGES, bool FULLD, int XU, bool WGT>
 __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     const float* __restrict__ X, int64_t N, int D, int64_t ldx, const int32_t* __restrict__ perm,
     const int32_t* __restrict__ offsets, const double* __restrict__ W, int M, double inv_var,
-    double* __restrict__ part, double* __restrict__ cont, int32_t* __restrict__ cont_seg) {
+    const double* __restrict__ weight, double* __restrict__ part, double* __restrict__ cont,
+    int32_t* __restrict__ cont_seg) {
   constexpr int TEAMS = THREADS / 32 / WPR;
   constexpr int SLOT_BYTES = U * VPL * 512;          // one batch of one warp
-  constexpr int WARP_BYTES = STAGES * SLOT_BYTES + VPL * 1024 + ACC_WIN_BYTES;
+  constexpr int WGT_BYTES = WGT ? STAGES * U * 8 : 0;
+  constexpr int WARP_BYTES = STAGES * SLOT_BYTES + VPL * 1024 + ACC_WIN_BYTES + WGT_BYTES;
+  constexpr int CW = WGT ? 3 : 2;                    // sums per segment besides Sk in a continuation partial
   // per warp: [STAGES][U][VPL][32 lanes x 16 B] staged samples, then [VPL][32 lanes x 32 B] the current
   // segment's float64 prototype (each lane keeps the 4 columns it owns; in registers it cost 16 of them),
   // then the ring of row offsets: slot (p & 63) = byte offset of the row at position p; slots 0..7 are
-  // mirrored at 64..71 so a batch reads its <= 8 consecutive slots without wrapping
+  // mirrored at 64..71 so a batch reads its <= 8 consecutive slots without wrapping; WGT: then [STAGES][U]
+  // float64 row weights
   static_assert(U <= 8 && STAGES >= 2 && STAGES <= 4, "offset ring mirror / byte FIFO");
   extern __shared__ __align__(16) uint8_t stage_smem[];
   __shared__ double red[TEAMS][2][WPR][U];  // cross-warp partial squared distances (double buffered)
@@ -336,6 +345,8 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
   int32_t perm_nxt = perm_at(filled + lane);  // always one window ahead of the ring
   const uint32_t row_bytes = (uint32_t)ldx * 4u;
   const char* __restrict__ my_src = reinterpret_cast<const char*>(X + col0);
+  const uint32_t my_wgt = my_win + ACC_WIN_BYTES;  // WGT: [STAGES][U] weights of the staged rows
+  const double inv_row_bytes = 1.0 / (double)row_bytes;
   uint32_t fifo = 0;  // one byte per batch in flight, oldest lowest: rows | 0x80 if the batch starts a segment
 
   auto issue = [&](int stage, int fifo_pos) {  // every lane copies its own 16-byte pieces of the next batch
@@ -373,6 +384,18 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
                            : "memory");
         }
       }
+      if constexpr (WGT) {
+        if (lane < nb) {
+          uint64_t o = off[0];
+#pragma unroll
+          for (int u = 1; u < U; ++u)
+            if (lane == u) o = off[u];
+          const uint32_t i = (uint32_t)__double2uint_rn((double)o * inv_row_bytes);
+          asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(my_wgt + (uint32_t)(stage * U + lane) * 8),
+                       "l"(weight + i)
+                       : "memory");
+        }
+      }
       fifo |= (uint32_t)(nb | (pnew ? 0x80 : 0)) << (8 * fifo_pos);
       pnew = false;
       pp += nb;
@@ -384,7 +407,7 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
 
   double* __restrict__ Sk = part;
   double acc[VPL][4];
-  double run_k = 0.0, run_d = 0.0;  // sums of the rows this lane evaluates (row slot row_of_lane)
+  double run_k = 0.0, run_d = 0.0, run_n = 0.0;  // sums of the rows this lane evaluates (row slot row_of_lane)
   int seg = ~lo;  // < 0: nothing accumulated yet, the first segment is ~seg
   auto load_w = [&](int sgm) {
     seg = sgm;
@@ -401,6 +424,7 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     }
     run_k = 0.0;
     run_d = 0.0;
+    run_n = 0.0;
   };
   auto flush = [&]() {
     // a segment begun by an earlier team: this team's partial goes to cont[team] and acc_cont_kernel adds the
@@ -408,7 +432,7 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     // once per segment, rather than kept live through the row loop)
     const int64_t t_id = (int64_t)blockIdx.x * TEAMS + (threadIdx.x >> 5) / WPR;
     const bool to_cont = offsets[seg] < (int32_t)((int64_t)offsets[M] * t_id / ((int64_t)gridDim.x * TEAMS));
-    double* cdst = cont + t_id * (D + 2);
+    double* cdst = cont + t_id * (D + CW);
 #pragma unroll
     for (int v = 0; v < VPL; ++v) {
       const int c = col0 + v * 128;
@@ -424,14 +448,17 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     const bool slot_leader = (lane % (32 / U)) == 0;
     const double tk = warp_sum(slot_leader ? run_k : 0.0);
     const double td = warp_sum(slot_leader ? run_d : 0.0);
+    const double tn = WGT ? warp_sum(slot_leader ? run_n : 0.0) : 0.0;
     if (tw == 0 && lane == 0) {
       if (to_cont) {
         cdst[D] = tk;
         cdst[D + 1] = td;
+        if (WGT) cdst[D + 2] = tn;
         cont_seg[t_id] = seg;
       } else {
         part[(int64_t)M * D + seg] = tk;                      // sk
         part[(int64_t)M * D + 2 * (int64_t)M + seg] = td;     // E
+        if (WGT) part[(int64_t)M * D + M + seg] = tn;         // n (the scan wrote the count)
       }
     }
   };
@@ -451,6 +478,7 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
     fifo >>= 8;
     issue(stage == 0 ? STAGES - 1 : stage - 1, STAGES - 2);  // refill the slot consumed in the previous iteration
     asm volatile("cp.async.wait_group %0;" ::"n"(STAGES - 1) : "memory");
+    if constexpr (WGT) __syncwarp();  // the weights are read by the lanes of their row slot, not by the copying lane
     const uint32_t rows = my_smem + (uint32_t)stage * SLOT_BYTES;
 
     // ALL: the batch has all U rows (the common case) -> no per-row predicates in the unrolled code
@@ -509,8 +537,16 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
       // each lane evaluates the weight and the distance of its row slot (32 / U lanes per slot, redundantly)
       // dbgsom/BaseSom.py:536 squares the distance again; d2 itself is that square to one rounding, and the
       // exponential no longer waits for the square root
-      const double my_dist = sqrt(my_d2);
-      const double my_k = 1.0 - sqrt(1.0 - exp(-inv_var * my_d2));
+      double my_dist = sqrt(my_d2);
+      double my_k = 1.0 - sqrt(1.0 - exp(-inv_var * my_d2));
+      if constexpr (WGT) {
+        double w = 0.0;
+        if (ALL || row_of_lane<U>(lane) < nb)
+          asm volatile("ld.shared.f64 %0, [%1];" : "=d"(w) : "r"(my_wgt + (uint32_t)(stage * U + row_of_lane<U>(lane)) * 8));
+        my_k *= w;  // the k * x sums below take the weighted k
+        my_dist *= w;
+        run_n += w;
+      }
       if (ALL || row_of_lane<U>(lane) < nb) {
         run_k += my_k;
         run_d += my_dist;
@@ -542,8 +578,9 @@ __global__ void __launch_bounds__(THREADS, 2) accumulate_kernel(
 // CTA of its first continuing team).  cont_seg is -1 for a team that continued nothing, which includes teams with an
 // empty range (fewer samples than teams): those may sit between two teams that continue the same segment and must not
 // split its run.  Segments only grow with the team index, so skipping -1 entries never joins two different segments.
+// A partial is [Sk (D) | sk | E] or, weighted, [Sk | sk | E | n]: cw = D + 2 or D + 3 entries.
 __global__ void __launch_bounds__(256) acc_cont_kernel(const double* __restrict__ cont, const int32_t* __restrict__ cont_seg,
-                                                      int64_t n_teams, int M, int D, double* __restrict__ part) {
+                                                      int64_t n_teams, int M, int D, int cw, double* __restrict__ part) {
   const int64_t t = blockIdx.x;
   const int seg = cont_seg[t];
   if (seg < 0) return;
@@ -552,33 +589,34 @@ __global__ void __launch_bounds__(256) acc_cont_kernel(const double* __restrict_
     if (q == seg) return;  // an earlier team continues seg: its CTA sums the run
     if (q >= 0) break;
   }
-  for (int c = threadIdx.x; c < D + 2; c += blockDim.x) {
+  for (int c = threadIdx.x; c < cw; c += blockDim.x) {
     double sum = 0.0;
     for (int64_t u = t; u < n_teams; ++u) {
       const int q = cont_seg[u];
-      if (q == seg) sum += cont[u * (D + 2) + c];
+      if (q == seg) sum += cont[u * cw + c];
       else if (q >= 0) break;
     }
     double* dst = c < D ? part + (int64_t)seg * D + c
-                        : part + (int64_t)M * D + (c == D ? 0 : 2 * (int64_t)M) + seg;
+                        : part + (int64_t)M * D + (c == D ? 0 : c == D + 1 ? 2 * (int64_t)M : (int64_t)M) + seg;
     *dst += sum;
   }
 }
 
 constexpr int64_t ACC_MAX_TEAMS = 148 * 2 * 8;  // CTAs (<= 2 per SM) x teams per CTA (<= 8)
 
-template <int VPL, int WPR, int U, int XU = 1>
-int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, const int32_t* offsets, double* cont,
-                      int32_t* cont_seg, cudaStream_t s) {
+template <int VPL, int WPR, int U, int XU, bool WGT>
+int launch_accumulate_t(const dbgsom_accumulate_args& a, const double* weight, const int32_t* perm,
+                        const int32_t* offsets, double* cont, int32_t* cont_seg, cudaStream_t s) {
   // one warp per row (WPR = 1): 6 warps per CTA leave 168 registers per thread at two CTAs per SM, enough
   // for the U * VPL * 4 converted elements + prototype + sums without spilling (at 128 registers the
   // loop-carried cursors spilled and every iteration stalled on local-memory loads); teams need 8 warps
   constexpr int THREADS = WPR == 1 ? 192 : 256;
   constexpr int STAGES = WPR == 1 ? 4 : 3;
   constexpr int TEAMS = THREADS / 32 / WPR;
-  const size_t smem = (size_t)(THREADS / 32) * (STAGES * U * VPL * 512 + VPL * 1024 + ACC_WIN_BYTES);
-  auto kern = a.D == 128 * VPL * WPR ? accumulate_kernel<VPL, WPR, U, THREADS, STAGES, true, XU>
-                                     : accumulate_kernel<VPL, WPR, U, THREADS, STAGES, false, XU>;
+  const size_t smem =
+      (size_t)(THREADS / 32) * (STAGES * U * VPL * 512 + VPL * 1024 + ACC_WIN_BYTES + (WGT ? STAGES * U * 8 : 0));
+  auto kern = a.D == 128 * VPL * WPR ? accumulate_kernel<VPL, WPR, U, THREADS, STAGES, true, XU, WGT>
+                                     : accumulate_kernel<VPL, WPR, U, THREADS, STAGES, false, XU, WGT>;
   DBGSOM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 1;  // resident CTAs per SM: 2 by registers (__launch_bounds__) if the staging rings fit twice
   DBGSOM_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, THREADS, smem));
@@ -592,11 +630,56 @@ int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, cons
   static_assert(TEAMS <= 8, "ACC_MAX_TEAMS");
   DBGSOM_CUDA_TRY(cudaMemsetAsync(cont_seg, 0xff, (size_t)n_teams * 4, s));
   kern<<<(unsigned)blocks, THREADS, smem, s>>>(a.d_X, a.N, a.D, a.ldx, perm, offsets, a.d_W, a.M,
-                                              a.inv_total_variance, a.d_part, cont, cont_seg);
+                                              a.inv_total_variance, weight, a.d_part, cont, cont_seg);
   DBGSOM_LAUNCH_CHECK();
-  acc_cont_kernel<<<(unsigned)n_teams, 256, 0, s>>>(cont, cont_seg, n_teams, a.M, a.D, a.d_part);
+  acc_cont_kernel<<<(unsigned)n_teams, 256, 0, s>>>(cont, cont_seg, n_teams, a.M, a.D, a.D + (WGT ? 3 : 2), a.d_part);
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
+}
+
+// the weighted kernels exist for the default variant of each width only (the DBGSOM_ACC_* tuning switches select
+// among unweighted variants)
+template <int VPL, int WPR, int U, int XU = 1>
+int launch_accumulate(const dbgsom_accumulate_args& a, const double* weight, const int32_t* perm, const int32_t* offsets,
+                      double* cont, int32_t* cont_seg, cudaStream_t s) {
+  if (weight) return DBGSOM_E_UNSUPPORTED;
+  return launch_accumulate_t<VPL, WPR, U, XU, false>(a, nullptr, perm, offsets, cont, cont_seg, s);
+}
+template <int VPL, int WPR, int U, int XU = 1>
+int launch_accumulate_w(const dbgsom_accumulate_args& a, const double* weight, const int32_t* perm,
+                        const int32_t* offsets, double* cont, int32_t* cont_seg, cudaStream_t s) {
+  if (weight) return launch_accumulate_t<VPL, WPR, U, XU, true>(a, weight, perm, offsets, cont, cont_seg, s);
+  return launch_accumulate_t<VPL, WPR, U, XU, false>(a, nullptr, perm, offsets, cont, cont_seg, s);
+}
+
+// Weighted class histogram per winner, out[j, c] = sum of weight[i] (1 if weight == NULL) over the samples i of
+// segment j with label c (float64 [M, n_classes], every cell written).  One warp per segment: lane l adds the weights of positions
+// offsets[j] + l, + 32, ... into its own row of shared-memory bins, then the 32 rows are added in lane order -- with
+// the stable permutation the sums are the same on every run.  Classes are taken CC at a time.
+constexpr int CH_WARPS = 4;
+constexpr int CH_CLASSES = 48;
+__global__ void __launch_bounds__(CH_WARPS * 32) seg_class_hist_kernel(
+    const int32_t* __restrict__ perm, const int32_t* __restrict__ offsets, const int32_t* __restrict__ labels,
+    const double* __restrict__ weight, int M, int n_classes, int c0, int cc, double* __restrict__ out) {
+  extern __shared__ double ch_bins[];  // [CH_WARPS][32][cc]
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int j = blockIdx.x * CH_WARPS + warp;
+  if (j >= M) return;
+  double* bins = ch_bins + (size_t)warp * 32 * cc;
+  for (int q = lane; q < 32 * cc; q += 32) bins[q] = 0.0;
+  __syncwarp();
+  double* mine = bins + lane * cc;
+  for (int32_t p = offsets[j] + lane; p < offsets[j + 1]; p += 32) {
+    const int32_t i = perm[p];
+    const int y = labels[i] - c0;
+    if ((unsigned)y < (unsigned)cc) mine[y] += weight ? weight[i] : 1.0;
+  }
+  __syncwarp();
+  for (int c = lane; c < cc; c += 32) {
+    double t = 0.0;
+    for (int l = 0; l < 32; ++l) t += bins[l * cc + c];
+    out[(int64_t)j * n_classes + c0 + c] = t;
+  }
 }
 
 }  // namespace
@@ -604,11 +687,11 @@ int launch_accumulate(const dbgsom_accumulate_args& a, const int32_t* perm, cons
 struct AccWorkspace {
   int32_t *counts, *offsets, *cursor, *perm;
   int32_t* chunk_table;  // stable scatter: [chunks, M] (dead once perm is built; shares its space with cont)
-  double* cont;          // [ACC_MAX_TEAMS, D + 2] partials of teams that continue a segment
+  double* cont;          // [ACC_MAX_TEAMS, D + 2 (+1 weighted)] partials of teams that continue a segment
   int32_t* cont_seg;     // [ACC_MAX_TEAMS]
   static size_t shared_bytes(int64_t N, int M, int D) {
     const size_t table = M <= STABLE_MAX_M ? (size_t)stable_max_chunks(N) * M * 4 : 0;
-    const size_t c = round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 2) * 8, 256) + (size_t)ACC_MAX_TEAMS * 4;
+    const size_t c = round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 3) * 8, 256) + (size_t)ACC_MAX_TEAMS * 4;
     return round_up<size_t>(table > c ? table : c, 256);
   }
   static size_t bytes(int64_t N, int M, int D) {
@@ -625,7 +708,7 @@ struct AccWorkspace {
     uint8_t* q = p + 3 * sm + round_up<size_t>((size_t)N * 4, 256);
     w.chunk_table = reinterpret_cast<int32_t*>(q);
     w.cont = reinterpret_cast<double*>(q);
-    w.cont_seg = reinterpret_cast<int32_t*>(q + round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 2) * 8, 256));
+    w.cont_seg = reinterpret_cast<int32_t*>(q + round_up<size_t>((size_t)ACC_MAX_TEAMS * (D + 3) * 8, 256));
     return w;
   }
 };
@@ -636,47 +719,87 @@ size_t accumulate_perm_offset(int64_t N, int M) {
   return 3 * round_up<size_t>((size_t)(M + 1) * 4, 256);
 }
 
-int run_accumulate(const dbgsom_accumulate_args& a, cudaStream_t s) {
-  const AccWorkspace ws = AccWorkspace::carve(a.d_workspace, a.N, a.M, a.D);
-  const int64_t M = a.M, D = a.D;
-  DBGSOM_CUDA_TRY(cudaMemsetAsync(a.d_part, 0, (size_t)(M * D + 3 * M) * sizeof(double), s));
+// counts per winner (+ the int32 class histogram when class_hist != NULL) -> offsets -> permutation of the samples
+// grouped by winner (ascending sample index for M <= STABLE_MAX_M); part_n (may be NULL) receives the counts
+static int build_winner_perm(const int32_t* bmu, int64_t N, int M, const int32_t* labels, int n_classes,
+                             int32_t* class_hist, const AccWorkspace& ws, double* part_n, cudaStream_t s) {
   DBGSOM_CUDA_TRY(cudaMemsetAsync(ws.counts, 0, (size_t)(M + 1) * 4, s));
-  const bool with_labels = a.d_labels != nullptr && a.d_class_hist != nullptr && a.n_classes > 0;
-  if (with_labels) DBGSOM_CUDA_TRY(cudaMemsetAsync(a.d_class_hist, 0, (size_t)M * a.n_classes * 4, s));
-
+  if (class_hist) DBGSOM_CUDA_TRY(cudaMemsetAsync(class_hist, 0, (size_t)M * n_classes * 4, s));
   // histogram
   {
-    const int64_t bins = M + (with_labels ? M * a.n_classes : 0);
+    const int64_t bins = M + (class_hist ? (int64_t)M * n_classes : 0);
     const bool smem = bins <= HIST_SMEM_BINS;
     const int64_t rows_per_block = smem ? 16384 : 4096;
-    const unsigned blocks = (unsigned)ceil_div<int64_t>(a.N, rows_per_block);
+    const unsigned blocks = (unsigned)ceil_div<int64_t>(N, rows_per_block);
     if (smem)
-      hist_kernel<true><<<blocks, HIST_THREADS, (size_t)bins * 4, s>>>(a.d_bmu, a.N, a.M, with_labels ? a.d_labels : nullptr,
-                                                                     a.n_classes, ws.counts, a.d_class_hist, rows_per_block);
+      hist_kernel<true><<<blocks, HIST_THREADS, (size_t)bins * 4, s>>>(bmu, N, M, class_hist ? labels : nullptr,
+                                                                     n_classes, ws.counts, class_hist, rows_per_block);
     else
-      hist_kernel<false><<<blocks, HIST_THREADS, 0, s>>>(a.d_bmu, a.N, a.M, with_labels ? a.d_labels : nullptr,
-                                                        a.n_classes, ws.counts, a.d_class_hist, rows_per_block);
+      hist_kernel<false><<<blocks, HIST_THREADS, 0, s>>>(bmu, N, M, class_hist ? labels : nullptr, n_classes, ws.counts,
+                                                        class_hist, rows_per_block);
     DBGSOM_LAUNCH_CHECK();
   }
-  scan_kernel<<<1, SCAN_THREADS, 0, s>>>(ws.counts, a.M, ws.offsets, ws.cursor, a.d_part + M * D + M);
+  scan_kernel<<<1, SCAN_THREADS, 0, s>>>(ws.counts, M, ws.offsets, ws.cursor, part_n);
   DBGSOM_LAUNCH_CHECK();
-  if (a.M <= STABLE_MAX_M) {
-    const StableChunks sc = stable_chunks(a.N, a.M);
-    const size_t smem = (size_t)sc.warps * a.M * 4;
+  if (M <= STABLE_MAX_M) {
+    const StableChunks sc = stable_chunks(N, M);
+    const size_t smem = (size_t)sc.warps * M * 4;
     const unsigned ctas = (unsigned)ceil_div<int64_t>(sc.n, sc.warps);
     DBGSOM_CUDA_TRY(cudaFuncSetAttribute(stable_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     DBGSOM_CUDA_TRY(cudaFuncSetAttribute(stable_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    stable_count_kernel<<<ctas, sc.warps * 32, smem, s>>>(a.d_bmu, a.N, a.M, sc.chunk, sc.n, ws.chunk_table);
+    stable_count_kernel<<<ctas, sc.warps * 32, smem, s>>>(bmu, N, M, sc.chunk, sc.n, ws.chunk_table);
     DBGSOM_LAUNCH_CHECK();
-    stable_base_kernel<<<(unsigned)ceil_div(a.M, 32), 1024, 0, s>>>(ws.chunk_table, sc.n, a.M, ws.offsets);
+    stable_base_kernel<<<(unsigned)ceil_div(M, 32), 1024, 0, s>>>(ws.chunk_table, sc.n, M, ws.offsets);
     DBGSOM_LAUNCH_CHECK();
-    stable_place_kernel<<<ctas, sc.warps * 32, smem, s>>>(a.d_bmu, a.N, a.M, sc.chunk, sc.n, ws.chunk_table, ws.perm);
+    stable_place_kernel<<<ctas, sc.warps * 32, smem, s>>>(bmu, N, M, sc.chunk, sc.n, ws.chunk_table, ws.perm);
     DBGSOM_LAUNCH_CHECK();
   } else {  // maps too large for the per-warp tables: slots in arrival order
-    int64_t blocks = ceil_div<int64_t>(a.N, SCAT_THREADS * 4);
+    int64_t blocks = ceil_div<int64_t>(N, SCAT_THREADS * 4);
     if (blocks > 148 * 16) blocks = 148 * 16;
-    scatter_kernel<<<(unsigned)blocks, SCAT_THREADS, 0, s>>>(a.d_bmu, a.N, a.M, ws.offsets, ws.cursor, ws.perm);
+    scatter_kernel<<<(unsigned)blocks, SCAT_THREADS, 0, s>>>(bmu, N, M, ws.offsets, ws.cursor, ws.perm);
     DBGSOM_LAUNCH_CHECK();
+  }
+  return DBGSOM_OK;
+}
+
+// float64 [M, n_classes] weighted class histogram over the segments of a permutation built by build_winner_perm
+static int run_seg_class_hist(const AccWorkspace& ws, const int32_t* labels, const double* weight, int M, int n_classes,
+                              double* out, cudaStream_t s) {
+  const int cc_max = n_classes < CH_CLASSES ? n_classes : CH_CLASSES;
+  DBGSOM_CUDA_TRY(cudaFuncSetAttribute(seg_class_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       CH_WARPS * 32 * cc_max * 8));
+  for (int c0 = 0; c0 < n_classes; c0 += CH_CLASSES) {
+    const int cc = n_classes - c0 < CH_CLASSES ? n_classes - c0 : CH_CLASSES;
+    seg_class_hist_kernel<<<(unsigned)ceil_div(M, CH_WARPS), CH_WARPS * 32, (size_t)CH_WARPS * 32 * cc * 8, s>>>(
+        ws.perm, ws.offsets, labels, weight, M, n_classes, c0, cc, out);
+    DBGSOM_LAUNCH_CHECK();
+  }
+  return DBGSOM_OK;
+}
+
+size_t label_hist_weighted_workspace_bytes(int64_t N, int M) { return AccWorkspace::bytes(N, M, 1); }
+
+int run_label_counts_weighted(const int32_t* idx, const int32_t* labels, const double* weight, int64_t N, int M,
+                              int n_classes, double* counts, void* workspace, cudaStream_t s) {
+  const AccWorkspace ws = AccWorkspace::carve(workspace, N, M, 1);
+  const int rc = build_winner_perm(idx, N, M, nullptr, 0, nullptr, ws, nullptr, s);
+  if (rc != DBGSOM_OK) return rc;
+  return run_seg_class_hist(ws, labels, weight, M, n_classes, counts, s);
+}
+
+int run_accumulate(const dbgsom_accumulate_args& a, const double* weight, double* class_hist_w, cudaStream_t s) {
+  const AccWorkspace ws = AccWorkspace::carve(a.d_workspace, a.N, a.M, a.D);
+  const int64_t M = a.M, D = a.D;
+  DBGSOM_CUDA_TRY(cudaMemsetAsync(a.d_part, 0, (size_t)(M * D + 3 * M) * sizeof(double), s));
+  const bool with_labels = a.d_labels != nullptr && a.n_classes > 0 &&
+                           (weight ? class_hist_w != nullptr : a.d_class_hist != nullptr);
+  // weighted: the class histogram is summed per segment after the scatter (float64, fixed order)
+  int rc = build_winner_perm(a.d_bmu, a.N, a.M, a.d_labels, a.n_classes,
+                             with_labels && !weight ? a.d_class_hist : nullptr, ws, a.d_part + M * D + M, s);
+  if (rc != DBGSOM_OK) return rc;
+  if (with_labels && weight) {
+    rc = run_seg_class_hist(ws, a.d_labels, weight, a.M, a.n_classes, class_hist_w, s);
+    if (rc != DBGSOM_OK) return rc;
   }
   const int D4 = a.D;
   static const char* tune_u = getenv("DBGSOM_ACC_ROWS");  // tuning switch: rows per batch for D <= 256
@@ -686,25 +809,26 @@ int run_accumulate(const dbgsom_accumulate_args& a, cudaStream_t s) {
   // cycles (ncu: XU 20 % busy at two in four).  10M x 256 rows stand-alone 1.80 (one) / 1.76 (two) / 1.72 ms (four);
   // in the bench epoch, at the clock K1 leaves, 2.21 / 2.17 / 2.12 ms.  DBGSOM_ACC_XU=1..4 selects.
   static const char* tune_xu = getenv("DBGSOM_ACC_XU");
-  const int xu = tune_xu ? atoi(tune_xu) : 4;
+  const int xu = weight ? 4 : (tune_xu ? atoi(tune_xu) : 4);
+  const double* w = weight;
   if (D4 <= 128) {
-    if (u_small == 4) return launch_accumulate<1, 1, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu >= 4) return launch_accumulate<1, 1, 8, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu == 3) return launch_accumulate<1, 1, 8, 3>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu == 2) return launch_accumulate<1, 1, 8, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    return launch_accumulate<1, 1, 8>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (u_small == 4 && !w) return launch_accumulate<1, 1, 4>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu >= 4) return launch_accumulate_w<1, 1, 8, 4>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 3) return launch_accumulate<1, 1, 8, 3>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 2) return launch_accumulate<1, 1, 8, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    return launch_accumulate<1, 1, 8>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   }
   if (D4 <= 256) {
-    if (u_small == 2) return launch_accumulate<2, 1, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu >= 4) return launch_accumulate<2, 1, 4, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu == 3) return launch_accumulate<2, 1, 4, 3>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    if (xu == 2) return launch_accumulate<2, 1, 4, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-    return launch_accumulate<2, 1, 4>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (u_small == 2 && !w) return launch_accumulate<2, 1, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu >= 4) return launch_accumulate_w<2, 1, 4, 4>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 3) return launch_accumulate<2, 1, 4, 3>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    if (xu == 2) return launch_accumulate<2, 1, 4, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+    return launch_accumulate<2, 1, 4>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   }
-  if (D4 <= 512) return launch_accumulate<4, 1, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-  if (D4 <= 1024) return launch_accumulate<4, 2, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-  if (D4 <= 2048) return launch_accumulate<4, 4, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
-  if (D4 <= 4096) return launch_accumulate<4, 8, 2>(a, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 512) return launch_accumulate_w<4, 1, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 1024) return launch_accumulate_w<4, 2, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 2048) return launch_accumulate_w<4, 4, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
+  if (D4 <= 4096) return launch_accumulate_w<4, 8, 2>(a, w, ws.perm, ws.offsets, ws.cont, ws.cont_seg, s);
   return DBGSOM_E_UNSUPPORTED;
 }
 

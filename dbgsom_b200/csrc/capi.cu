@@ -2,7 +2,7 @@
 #include "common.cuh"
 
 namespace dbgsom {
-int run_colstats(const float*, int64_t, int, int64_t, const float*, double*, cudaStream_t);
+int run_colstats(const float*, int64_t, int, int64_t, const float*, const double*, double*, cudaStream_t);
 int run_prepare_x16(const float*, int64_t, int, int64_t, const float*, float, const int32_t*, uint16_t*, uint16_t*, int64_t,
                     float*, cudaStream_t);
 size_t accumulate_perm_offset(int64_t, int);
@@ -15,11 +15,15 @@ int run_prepare_bias(const float*, int, const float*, uint16_t*, float*, cudaStr
 int run_row_ops(double*, int, const int32_t*, int, cudaStream_t);
 int run_gather_rows(const float*, int64_t, int, const int64_t*, int, double*, cudaStream_t);
 size_t accumulate_workspace_bytes(int64_t, int, int);
-int run_accumulate(const dbgsom_accumulate_args&, cudaStream_t);
+int run_accumulate(const dbgsom_accumulate_args&, const double*, double*, cudaStream_t);
+size_t label_hist_weighted_workspace_bytes(int64_t, int);
+int run_label_counts_weighted(const int32_t*, const int32_t*, const double*, int64_t, int, int, double*, void*, cudaStream_t);
 size_t smooth_workspace_bytes(int, int);
 int run_smooth(const dbgsom_smooth_args&, cudaStream_t);
-int run_node_stats(const int32_t*, int, const double*, int, int64_t, const int32_t*, int, double, double*, cudaStream_t);
-int run_label_hist(const int32_t*, int, const int32_t*, int64_t, int64_t, int, int, int32_t*, int64_t*, cudaStream_t);
+int run_node_stats(const int32_t*, int, const double*, int, int64_t, const int32_t*, int, double, const double*, double*,
+                   cudaStream_t);
+int run_label_hist(const int32_t*, int, const int32_t*, const double*, int64_t, int64_t, int, int, int32_t*, int64_t*,
+                   cudaStream_t);
 int run_umatrix(const double*, int, int, int64_t, const double*, double*, cudaStream_t);
 int run_hops(const int32_t*, int, uint16_t*, int64_t, cudaStream_t);
 size_t sparse_code_workspace_bytes(int64_t, int, int);
@@ -59,7 +63,13 @@ int dbgsom_check_device(int device) {
 int dbgsom_colstats(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift_row, double* d_moments,
                     void* stream) {
   if (!d_X || !d_shift_row || !d_moments || N <= 0 || D <= 0 || ldx < D) return DBGSOM_E_BADARG;
-  return run_colstats(d_X, N, D, ldx, d_shift_row, d_moments, as_stream(stream));
+  return run_colstats(d_X, N, D, ldx, d_shift_row, nullptr, d_moments, as_stream(stream));
+}
+
+int dbgsom_colstats_weighted(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift_row,
+                             const double* d_weight, double* d_moments, void* stream) {
+  if (!d_X || !d_shift_row || !d_moments || N <= 0 || D <= 0 || ldx < D) return DBGSOM_E_BADARG;
+  return run_colstats(d_X, N, D, ldx, d_shift_row, d_weight, d_moments, as_stream(stream));
 }
 
 int dbgsom_prepare_x16(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift, float scale,
@@ -164,13 +174,19 @@ size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M, int32_t D) { retu
 size_t dbgsom_accumulate_perm_offset(int64_t N, int32_t M) { return accumulate_perm_offset(N, M); }
 
 int dbgsom_accumulate(const dbgsom_accumulate_args* a, void* stream) {
+  return dbgsom_accumulate_weighted(a, nullptr, nullptr, stream);
+}
+
+int dbgsom_accumulate_weighted(const dbgsom_accumulate_args* a, const double* d_weight, double* d_class_hist_w,
+                               void* stream) {
   if (!a || !a->d_X || !a->d_bmu || !a->d_W || !a->d_part || !a->d_workspace) return DBGSOM_E_BADARG;
+  if (d_weight && a->d_labels && a->n_classes > 0 && !d_class_hist_w) return DBGSOM_E_BADARG;
   if (a->N <= 0 || a->D <= 0 || a->M <= 0 || a->ldx < a->D || !(a->inv_total_variance == a->inv_total_variance))
     return DBGSOM_E_BADARG;
   if (a->N > 0x7fffffffLL) return DBGSOM_E_UNSUPPORTED;  // int32 permutation
   if (a->D % 4 != 0 || a->ldx % 4 != 0 || !aligned16(a->d_X) || !aligned16(a->d_W)) return DBGSOM_E_UNSUPPORTED;
   if (a->workspace_bytes < accumulate_workspace_bytes(a->N, a->M, a->D)) return DBGSOM_E_WORKSPACE;
-  return run_accumulate(*a, as_stream(stream));
+  return run_accumulate(*a, d_weight, d_class_hist_w, as_stream(stream));
 }
 
 size_t dbgsom_smooth_workspace_bytes(int32_t M, int32_t D) { return smooth_workspace_bytes(M, D); }
@@ -200,7 +216,18 @@ int dbgsom_node_stats(const int32_t* d_idx, int32_t idx_stride, const double* d_
   if (!d_idx || !d_dist || !d_pos || !d_out || N <= 0 || M <= 0 || idx_stride < 1 || dist_stride < 1)
     return DBGSOM_E_BADARG;
   if (!(bandwidth > 0.0)) return DBGSOM_E_BADARG;
-  return run_node_stats(d_idx, idx_stride, d_dist, dist_stride, N, d_pos, M, bandwidth, d_out, as_stream(stream));
+  return run_node_stats(d_idx, idx_stride, d_dist, dist_stride, N, d_pos, M, bandwidth, nullptr, d_out,
+                        as_stream(stream));
+}
+
+int dbgsom_node_stats_weighted(const int32_t* d_idx, int32_t idx_stride, const double* d_dist, int32_t dist_stride,
+                               int64_t N, const int32_t* d_pos, int32_t M, double bandwidth, const double* d_weight,
+                               double* d_out, void* stream) {
+  if (!d_idx || !d_dist || !d_pos || !d_out || N <= 0 || M <= 0 || idx_stride < 1 || dist_stride < 1)
+    return DBGSOM_E_BADARG;
+  if (!(bandwidth > 0.0)) return DBGSOM_E_BADARG;
+  return run_node_stats(d_idx, idx_stride, d_dist, dist_stride, N, d_pos, M, bandwidth, d_weight, d_out,
+                        as_stream(stream));
 }
 
 int dbgsom_umatrix(const double* d_W, int32_t M, int32_t D, int64_t ldw, const double* d_colw, double* d_out,
@@ -214,7 +241,25 @@ int dbgsom_label_hist(const int32_t* d_idx, int32_t idx_stride, const int32_t* d
                       void* stream) {
   if (!d_idx || !d_labels || !d_counts || !d_first || N <= 0 || M <= 0 || n_classes <= 0 || idx_stride < 1)
     return DBGSOM_E_BADARG;
-  return run_label_hist(d_idx, idx_stride, d_labels, N, sample_offset, M, n_classes, d_counts, d_first,
+  return run_label_hist(d_idx, idx_stride, d_labels, nullptr, N, sample_offset, M, n_classes, d_counts, d_first,
+                        as_stream(stream));
+}
+
+size_t dbgsom_label_hist_weighted_workspace_bytes(int64_t N, int32_t M) {
+  return label_hist_weighted_workspace_bytes(N, M);
+}
+
+int dbgsom_label_hist_weighted(const int32_t* d_idx, const int32_t* d_labels, const double* d_weight, int64_t N,
+                               int64_t sample_offset, int32_t M, int32_t n_classes, double* d_counts, int64_t* d_first,
+                               void* d_workspace, size_t workspace_bytes, void* stream) {
+  if (!d_idx || !d_labels || !d_counts || !d_first || !d_workspace || N <= 0 || M <= 0 || n_classes <= 0)
+    return DBGSOM_E_BADARG;
+  if (N > 0x7fffffffLL) return DBGSOM_E_UNSUPPORTED;  // int32 permutation
+  if (workspace_bytes < label_hist_weighted_workspace_bytes(N, M)) return DBGSOM_E_WORKSPACE;
+  const int rc = run_label_counts_weighted(d_idx, d_labels, d_weight, N, M, n_classes, d_counts, d_workspace,
+                                           as_stream(stream));
+  if (rc != DBGSOM_OK) return rc;
+  return run_label_hist(d_idx, 1, d_labels, d_weight, N, sample_offset, M, n_classes, nullptr, d_first,
                         as_stream(stream));
 }
 

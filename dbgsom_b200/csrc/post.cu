@@ -22,10 +22,14 @@ namespace {
 constexpr int NS_THREADS = 256;
 
 // out = [te_count, qe_sum, hits[M], dens_sum[M]]  (float64, atomically accumulated; zeroed by the launcher)
+// WGT: every term of sample i is multiplied by weight[i] (frequency weights)
+template <bool WGT>
 __global__ void __launch_bounds__(NS_THREADS) node_stats_kernel(const int32_t* __restrict__ idx, int idx_stride,
                                                                const double* __restrict__ dist, int dist_stride,
                                                                int64_t N, const int32_t* __restrict__ pos, int M,
-                                                               double inv_two_bw2, double norm, double* __restrict__ out) {
+                                                               double inv_two_bw2, double norm,
+                                                               const double* __restrict__ weight,
+                                                               double* __restrict__ out) {
   double te = 0.0, qe = 0.0;
   double* hits = out + 2;
   double* dens = out + 2 + M;
@@ -34,18 +38,20 @@ __global__ void __launch_bounds__(NS_THREADS) node_stats_kernel(const int32_t* _
     const int b0 = idx[i * idx_stride];
     if ((unsigned)b0 >= (unsigned)M) continue;  // NaN row: no winner
     const double d = dist[i * dist_stride];
-    qe += d;
+    const double w = WGT ? weight[i] : 1.0;
+    qe += WGT ? w * d : d;
     if (idx_stride > 1) {
       const int b1 = idx[i * idx_stride + 1];
       if ((unsigned)b1 < (unsigned)M) {
         const int dx = pos[2 * b0] - pos[2 * b1], dy = pos[2 * b0 + 1] - pos[2 * b1 + 1];
         // grid distance > 1.5  <=>  squared integer distance > 2 (dbgsom/BaseSom.py:951)
-        if (dx * dx + dy * dy > 2) te += 1.0;
+        if (dx * dx + dy * dy > 2) te += w;
       }
     }
-    atomicAdd(hits + b0, 1.0);
+    atomicAdd(hits + b0, w);
     // (np.exp(-(d**2) / (2 * sigma**2))) / (sigma * sqrt(2 * pi))   dbgsom/BaseSom.py:205-208
-    atomicAdd(dens + b0, exp(-(d * d) * inv_two_bw2) * norm);
+    const double kd = exp(-(d * d) * inv_two_bw2) * norm;
+    atomicAdd(dens + b0, WGT ? w * kd : kd);
   }
   te = warp_sum(te);
   qe = warp_sum(qe);
@@ -68,8 +74,11 @@ __global__ void __launch_bounds__(NS_THREADS) node_stats_kernel(const int32_t* _
 }
 
 // ------------------------------------------------------------------------------------------ class histogram
+// weight != NULL: first occurrences over the samples with weight > 0 only.  counts == NULL: first occurrences only (the
+// weighted counts are summed per winner in a fixed order by the segment kernel of accumulate.cu)
 __global__ void __launch_bounds__(NS_THREADS) label_hist_kernel(const int32_t* __restrict__ idx, int idx_stride,
-                                                               const int32_t* __restrict__ labels, int64_t N,
+                                                               const int32_t* __restrict__ labels,
+                                                               const double* __restrict__ weight, int64_t N,
                                                                int64_t sample_offset, int M, int n_classes,
                                                                int32_t* __restrict__ counts,
                                                                long long* __restrict__ first) {
@@ -78,8 +87,9 @@ __global__ void __launch_bounds__(NS_THREADS) label_hist_kernel(const int32_t* _
     const int b = idx[i * idx_stride];
     const int y = labels[i];
     if ((unsigned)b >= (unsigned)M || (unsigned)y >= (unsigned)n_classes) continue;
+    if (weight && !(weight[i] > 0.0)) continue;
     const int64_t cell = (int64_t)b * n_classes + y;
-    atomicAdd(counts + cell, 1);
+    if (counts) atomicAdd(counts + cell, 1);
     atomicMin(first + cell, (long long)(sample_offset + i));
   }
 }
@@ -202,31 +212,36 @@ __global__ void __launch_bounds__(HOP_THREADS) hops_kernel(const int32_t* __rest
 }  // namespace
 
 int run_node_stats(const int32_t* idx, int idx_stride, const double* dist, int dist_stride, int64_t N,
-                   const int32_t* pos, int M, double bandwidth, double* out, cudaStream_t s) {
+                   const int32_t* pos, int M, double bandwidth, const double* weight, double* out, cudaStream_t s) {
   DBGSOM_CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)(2 + 2 * (int64_t)M) * sizeof(double), s));
   int64_t blocks = ceil_div<int64_t>(N, NS_THREADS * 8);
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (blocks < 1) blocks = 1;
   const double inv_two_bw2 = 1.0 / (2.0 * bandwidth * bandwidth);
   const double norm = 1.0 / (bandwidth * 2.5066282746310002);  // sqrt(2 pi)
-  node_stats_kernel<<<(unsigned)blocks, NS_THREADS, 0, s>>>(idx, idx_stride, dist, dist_stride, N, pos, M, inv_two_bw2,
-                                                           norm, out);
+  if (weight)
+    node_stats_kernel<true><<<(unsigned)blocks, NS_THREADS, 0, s>>>(idx, idx_stride, dist, dist_stride, N, pos, M,
+                                                                   inv_two_bw2, norm, weight, out);
+  else
+    node_stats_kernel<false><<<(unsigned)blocks, NS_THREADS, 0, s>>>(idx, idx_stride, dist, dist_stride, N, pos, M,
+                                                                    inv_two_bw2, norm, nullptr, out);
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
 }
 
-int run_label_hist(const int32_t* idx, int idx_stride, const int32_t* labels, int64_t N, int64_t sample_offset, int M,
-                   int n_classes, int32_t* counts, int64_t* first, cudaStream_t s) {
+// weight != NULL: first occurrences among the samples with weight > 0 only; counts may be NULL (see label_hist_kernel)
+int run_label_hist(const int32_t* idx, int idx_stride, const int32_t* labels, const double* weight, int64_t N,
+                   int64_t sample_offset, int M, int n_classes, int32_t* counts, int64_t* first, cudaStream_t s) {
   const int64_t cells = (int64_t)M * n_classes;
-  DBGSOM_CUDA_TRY(cudaMemsetAsync(counts, 0, (size_t)cells * sizeof(int32_t), s));
+  if (counts) DBGSOM_CUDA_TRY(cudaMemsetAsync(counts, 0, (size_t)cells * sizeof(int32_t), s));
   fill_i64_kernel<<<(unsigned)ceil_div<int64_t>(cells, 256), 256, 0, s>>>(reinterpret_cast<long long*>(first), cells,
                                                                          0x7fffffffffffffffLL);
   DBGSOM_LAUNCH_CHECK();
   int64_t blocks = ceil_div<int64_t>(N, NS_THREADS * 8);
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (blocks < 1) blocks = 1;
-  label_hist_kernel<<<(unsigned)blocks, NS_THREADS, 0, s>>>(idx, idx_stride, labels, N, sample_offset, M, n_classes,
-                                                           counts, reinterpret_cast<long long*>(first));
+  label_hist_kernel<<<(unsigned)blocks, NS_THREADS, 0, s>>>(idx, idx_stride, labels, weight, N, sample_offset, M,
+                                                           n_classes, counts, reinterpret_cast<long long*>(first));
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
 }

@@ -11,9 +11,13 @@ namespace {
 // No atomics: the caller adds the parts in order, so the statistics are the same on every run.
 // Replaces np.var(data, axis=0) / np.std(data, axis=0, ddof=1), dbgsom/BaseSom.py:363, :380.
 // Shifting by a data row keeps the one-pass variance free of cancellation.
+// WGT: the moments are weighted, w_i (x_id - c_d) and w_i (x_id - c_d)^2; the maximum stays over every row (all rows,
+// zero-weight ones included, go through the fp16 shadow that it scales).
 constexpr int CS_COLS = 32, CS_ROWS = 8;
+template <bool WGT>
 __global__ void __launch_bounds__(CS_COLS * CS_ROWS) colstats_kernel(const float* __restrict__ X, int64_t N, int D,
                                                                     int64_t ldx, const float* __restrict__ shift,
+                                                                    const double* __restrict__ weight,
                                                                     double* __restrict__ moments,
                                                                     int64_t rows_per_block) {
   __shared__ double s1[CS_ROWS][CS_COLS], s2[CS_ROWS][CS_COLS], s3[CS_ROWS][CS_COLS];
@@ -26,8 +30,9 @@ __global__ void __launch_bounds__(CS_COLS * CS_ROWS) colstats_kernel(const float
     const float c = shift[d];
     for (int64_t r = r0 + ry; r < r1; r += CS_ROWS) {
       const double t = (double)X[r * ldx + d] - (double)c;
-      a1 += t;
-      a2 = fma(t, t, a2);
+      const double wt = WGT ? weight[r] * t : t;
+      a1 += wt;
+      a2 = fma(wt, t, a2);
       a3 = fmax(a3, fabs(t));
     }
   }
@@ -340,14 +345,18 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restric
 
 }  // namespace
 
-int run_colstats(const float* X, int64_t N, int D, int64_t ldx, const float* shift, double* moments, cudaStream_t s) {
+int run_colstats(const float* X, int64_t N, int D, int64_t ldx, const float* shift, const double* weight, double* moments,
+                 cudaStream_t s) {
   int64_t row_blocks = ceil_div<int64_t>(N, 4096);
   const int col_blocks = ceil_div(D, CS_COLS);
   if (row_blocks > DBGSOM_COLSTATS_PARTS) row_blocks = DBGSOM_COLSTATS_PARTS;
   if (row_blocks < 1) row_blocks = 1;
   const int64_t rows_per_block = ceil_div<int64_t>(N, row_blocks);
-  colstats_kernel<<<dim3(col_blocks, (unsigned)row_blocks), CS_COLS * CS_ROWS, 0, s>>>(X, N, D, ldx, shift, moments,
-                                                                                    rows_per_block);
+  const dim3 grid(col_blocks, (unsigned)row_blocks);
+  if (weight)
+    colstats_kernel<true><<<grid, CS_COLS * CS_ROWS, 0, s>>>(X, N, D, ldx, shift, weight, moments, rows_per_block);
+  else
+    colstats_kernel<false><<<grid, CS_COLS * CS_ROWS, 0, s>>>(X, N, D, ldx, shift, nullptr, moments, rows_per_block);
   DBGSOM_LAUNCH_CHECK();
   return DBGSOM_OK;
 }

@@ -169,6 +169,8 @@ class DeviceEngine:
         self.comm = Comm(distributed, self.dev)
         self.sample_offset = 0
         self.n_samples_global = 0
+        self.weight = None        # float64 [N] frequency weights of the samples (None: unweighted)
+        self.weight_total = 0.0   # sum of the weights over all ranks (== n_samples_global when unweighted)
         self.launches = 0  # kernels + memsets enqueued by this engine (bench bookkeeping)
         self.fp32_reruns = 0  # epochs repeated on the fp32 search because a prototype left the fp16 range
         self._prof = None
@@ -233,14 +235,17 @@ class DeviceEngine:
     def close(self) -> None:
         self._ws.clear()
         self._perm_cache.clear()
-        for name in ("X", "X16_hi", "X16_lo", "xnorm16", "W", "W32", "W16_hi", "W16_lo", "Wb16", "_row_hash", "labels",
+        for name in ("X", "X16_hi", "X16_lo", "xnorm16", "W", "W32", "W16_hi", "W16_lo", "Wb16", "_row_hash", "labels", "weight",
                      "part", "hop", "_final_idx", "row_perm", "tile_mask", "tile_bound"):
             if hasattr(self, name):
                 setattr(self, name, None)
 
     # ------------------------------------------------------------------ data
-    def load_data(self, X: np.ndarray, y, n_classes: int) -> dict:
-        """Upload the samples and reduce the column statistics `fit` needs (K4)."""
+    def load_data(self, X: np.ndarray, y, n_classes: int, sample_weight=None) -> dict:
+        """Upload the samples and reduce the column statistics `fit` needs (K4).
+
+        `sample_weight` (float64 [N], finite, >= 0; this rank's shard): frequency weights -- a sample of weight w
+        counts like w copies of it in every sum of the fit.  None runs the unweighted kernels."""
         torch = self.torch
         with torch.cuda.device(self.dev):
             self.N, self.D = int(X.shape[0]), int(X.shape[1])
@@ -251,7 +256,19 @@ class DeviceEngine:
             if y is not None:
                 self.labels = torch.from_numpy(np.ascontiguousarray(y, dtype=np.int32)).to(self.dev)
             self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
+            self._set_weights(None if sample_weight is None else torch.from_numpy(
+                np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev))
             return self._column_statistics()
+
+    def _set_weights(self, weight_dev) -> None:
+        self.weight = weight_dev
+        if weight_dev is None:
+            self.weight_total = float(self.n_samples_global)
+            return
+        if weight_dev.dtype != self.torch.float64 or tuple(weight_dev.shape) != (self.N,) or not weight_dev.is_contiguous():
+            raise ValueError("sample_weight must be a contiguous float64 vector with one entry per sample")
+        total = weight_dev.sum().reshape(1)
+        self.weight_total = float(self.comm.allreduce_(total).item())
 
     def _column_statistics(self) -> dict:
         torch = self.torch
@@ -259,12 +276,21 @@ class DeviceEngine:
         shift_row = self.X[0].clone()
         self.comm.broadcast_(shift_row, 0)
         parts = torch.zeros((nat.COLSTATS_PARTS, 2 * self.ldx + 1), dtype=torch.float64, device=self.dev)
-        nat.check(
-            self.lib.dbgsom_colstats(
-                self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), parts.data_ptr(), self._stream()
-            ),
-            "dbgsom_colstats",
-        )
+        if self.weight is None:
+            nat.check(
+                self.lib.dbgsom_colstats(
+                    self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), parts.data_ptr(), self._stream()
+                ),
+                "dbgsom_colstats",
+            )
+        else:
+            nat.check(
+                self.lib.dbgsom_colstats_weighted(
+                    self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), self.weight.data_ptr(),
+                    parts.data_ptr(), self._stream(),
+                ),
+                "dbgsom_colstats_weighted",
+            )
         self.launches += 1
         # the row-block parts are added on the host in a fixed order: the same statistics on every run
         p = parts.cpu().numpy()
@@ -273,12 +299,16 @@ class DeviceEngine:
         self.comm.allreduce_(moments[2 * self.ldx :], "max")
         m = moments.cpu().numpy()
         s1, s2, maxabs = m[: self.ldx], m[self.ldx : 2 * self.ldx], float(m[2 * self.ldx])
-        stats = column_moments_to_stats(self.n_samples_global, s1, s2)
+        # the amount of data is the total weight (the sample count when unweighted)
+        n_g = self.weight_total if self.weight is not None else self.n_samples_global
+        stats = column_moments_to_stats(n_g, s1, s2)
+        stats["n_samples"] = int(self.n_samples_global)
+        if self.weight is not None:
+            stats["total_weight"] = n_g
         self.total_variance = stats["total_variance"]
         # data mean (centres the fp16 shadow) and a power-of-two scale that keeps it in range
-        mean = shift_row.double().cpu().numpy() + s1 / self.n_samples_global
+        mean = shift_row.double().cpu().numpy() + s1 / n_g
         # the device copy of X is float32: an offset far larger than the spread costs that many digits of the spread
-        n_g = self.n_samples_global
         std = np.sqrt(np.maximum(s2 - s1 * s1 / n_g, 0.0) / max(n_g, 1))
         with np.errstate(divide="ignore", invalid="ignore"):
             ratio = np.where(std > 0, np.abs(mean) / std, 0.0)
@@ -299,8 +329,8 @@ class DeviceEngine:
         self.ld16 = _round_up(self.ldx, 64)
         return stats
 
-    def load_device_data(self, X_dev, labels_dev=None, n_classes: int = 0) -> dict:
-        """Like `load_data` for samples that already live in HBM (float32 [N, D], D % 4 == 0)."""
+    def load_device_data(self, X_dev, labels_dev=None, n_classes: int = 0, weight_dev=None) -> dict:
+        """Like `load_data` for samples that already live in HBM (float32 [N, D], D % 4 == 0; weights float64 [N])."""
         torch = self.torch
         if X_dev.dtype != torch.float32 or X_dev.dim() != 2 or not X_dev.is_contiguous() or X_dev.shape[1] % 4:
             raise ValueError("X_dev must be a contiguous float32 [N, D] CUDA tensor with D % 4 == 0")
@@ -309,6 +339,7 @@ class DeviceEngine:
             self.X, self.ldx = X_dev, int(X_dev.shape[1])
             self.n_classes, self.labels = int(n_classes), labels_dev
             self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
+            self._set_weights(weight_dev)
             return self._column_statistics()
 
     def _ensure_x16(self, need_lo: bool) -> None:
@@ -345,8 +376,10 @@ class DeviceEngine:
         self.change = torch.zeros(1, dtype=torch.float64, device=self.dev)
         self.idx = torch.empty((self.N, 2), dtype=torch.int32, device=self.dev)
         self.bmu_stats = torch.zeros(8, dtype=torch.int64, device=self.dev)
+        # weighted fits sum the class histogram as float64 weights
+        hist_dtype = torch.int32 if self.weight is None else torch.float64
         self.class_hist = (
-            torch.zeros((cap, self.n_classes), dtype=torch.int32, device=self.dev) if self.labels is not None else None
+            torch.zeros((cap, self.n_classes), dtype=hist_dtype, device=self.dev) if self.labels is not None else None
         )
         if old is not None:
             for new, prev in zip(self.W, old):
@@ -772,11 +805,19 @@ class DeviceEngine:
         acc.d_part = part.data_ptr()
         acc.d_labels = self.labels.data_ptr() if use_hist else None
         acc.n_classes = self.n_classes if use_hist else 0
-        acc.d_class_hist = self.class_hist.data_ptr() if use_hist else None
+        acc.d_class_hist = self.class_hist.data_ptr() if use_hist and self.weight is None else None
         ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(self.N, m, self.ldx))
         acc.d_workspace, acc.workspace_bytes = ws.data_ptr(), ws.numel()
         with self._Phase(self, "accumulate"):
-            nat.check(self.lib.dbgsom_accumulate(acc, self._stream()), "dbgsom_accumulate")
+            if self.weight is None:
+                nat.check(self.lib.dbgsom_accumulate(acc, self._stream()), "dbgsom_accumulate")
+            else:
+                nat.check(
+                    self.lib.dbgsom_accumulate_weighted(
+                        acc, self.weight.data_ptr(), self.class_hist.data_ptr() if use_hist else None, self._stream()
+                    ),
+                    "dbgsom_accumulate_weighted",
+                )
         self.launches += (10 if m <= 24576 else 8) + (1 if use_hist else 0)  # stable scatter: 3 kernels
         if resort and self.X16_hi is not None:
             self._sort_age += 1
@@ -927,13 +968,22 @@ class DeviceEngine:
             pos = torch.from_numpy(np.ascontiguousarray(positions[:m], dtype=np.int32)).to(self.dev)
             out = torch.empty(2 + 2 * m, dtype=torch.float64, device=self.dev)
             ok = bandwidth > 0 and math.isfinite(bandwidth)
-            nat.check(
-                self.lib.dbgsom_node_stats(
-                    idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, self.N, pos.data_ptr(), m,
-                    bandwidth if ok else 1.0, out.data_ptr(), self._stream(),
-                ),
-                "dbgsom_node_stats",
-            )
+            if self.weight is None:
+                nat.check(
+                    self.lib.dbgsom_node_stats(
+                        idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, self.N, pos.data_ptr(), m,
+                        bandwidth if ok else 1.0, out.data_ptr(), self._stream(),
+                    ),
+                    "dbgsom_node_stats",
+                )
+            else:
+                nat.check(
+                    self.lib.dbgsom_node_stats_weighted(
+                        idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, self.N, pos.data_ptr(), m,
+                        bandwidth if ok else 1.0, self.weight.data_ptr(), out.data_ptr(), self._stream(),
+                    ),
+                    "dbgsom_node_stats_weighted",
+                )
             self.launches += 2
             self.comm.allreduce_(out)
             o = out.cpu().numpy()
@@ -953,10 +1003,26 @@ class DeviceEngine:
 
     def label_histogram(self, n_classes: int):
         """Class counts [M, C] and first global sample index [M, C] of every (winner, class) cell of the
-        last `final_winners` search, reduced over ranks (dbgsom/SomClassifier.py:130-152)."""
+        last `final_winners` search, reduced over ranks (dbgsom/SomClassifier.py:130-152).  Weighted fits: the
+        counts are weight sums and `first` ignores zero-weight samples."""
         torch = self.torch
         with torch.cuda.device(self.dev):
             m = self.M
+            if self.weight is not None:
+                counts = torch.empty((m, n_classes), dtype=torch.float64, device=self.dev)
+                first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
+                ws = self._workspace("labels", self.lib.dbgsom_label_hist_weighted_workspace_bytes(self.N, m))
+                nat.check(
+                    self.lib.dbgsom_label_hist_weighted(
+                        self._final_idx.data_ptr(), self.labels.data_ptr(), self.weight.data_ptr(), self.N,
+                        self.sample_offset, m, n_classes, counts.data_ptr(), first.data_ptr(), ws.data_ptr(),
+                        ws.numel(), self._stream(),
+                    ),
+                    "dbgsom_label_hist_weighted",
+                )
+                self.comm.allreduce_(counts)
+                self.comm.allreduce_(first, "min")
+                return counts.cpu().numpy(), first.cpu().numpy()
             counts = torch.empty((m, n_classes), dtype=torch.int32, device=self.dev)
             first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
             nat.check(

@@ -15,7 +15,11 @@
  *     or a positive cudaError_t; nothing throws; the library keeps no global state besides
  *     cached device attributes and the resolved cuTensorMapEncodeTiled entry point;
  *   - matrices are row-major; `ld*` are leading dimensions in ELEMENTS;
- *   - sizes: N samples, D features, M prototypes ("neurons").
+ *   - sizes: N samples, D features, M prototypes ("neurons");
+ *   - d_weight (the *_weighted entry points): float64 [N] frequency weights of the samples (sample_weight of
+ *     fit), finite and >= 0; NULL = every weight 1, which is exactly the unweighted entry point.  A sample of
+ *     weight w counts like w copies of it in every sum.  This is unrelated to the per-sample similarity
+ *     k_i of K2, which the reference calls "sample_weights".
  *
  * Data layout in HBM (see DESIGN.md):
  *   X     float32 [N, ldx]      master copy of the samples (read by the update pass)
@@ -37,7 +41,7 @@
 extern "C" {
 #endif
 
-#define DBGSOM_ABI_VERSION 9
+#define DBGSOM_ABI_VERSION 10
 
 #define DBGSOM_OK 0
 #define DBGSOM_E_BADARG (-1)      /* null pointer, non-positive size, bad enum             */
@@ -74,6 +78,11 @@ int dbgsom_check_device(int device);
 #define DBGSOM_COLSTATS_PARTS 256
 int dbgsom_colstats(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift_row,
                     double* d_moments, void* stream);
+/* Same with frequency weights: part[0:D] = sum_i w_i (x_id - c_d), part[D:2D] = sum_i w_i (x_id - c_d)^2; the
+ * maximum stays over ALL rows (zero-weight rows too: every row goes through the fp16 shadow it scales).  The
+ * caller divides by sum_i w_i instead of N. */
+int dbgsom_colstats_weighted(const float* d_X, int64_t N, int D, int64_t ldx, const float* d_shift_row,
+                             const double* d_weight, double* d_moments, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * fp16 shadows for the tensor-core BMU search (X once per fit, W once per epoch)
@@ -287,6 +296,14 @@ size_t dbgsom_accumulate_workspace_bytes(int64_t N, int32_t M, int32_t D);
  * in the order the scatter's atomics hand out, which varies between runs, and so do the last bits of the sums. */
 size_t dbgsom_accumulate_perm_offset(int64_t N, int32_t M);
 int dbgsom_accumulate(const dbgsom_accumulate_args* args, void* stream);
+/* Same with frequency weights w_i = d_weight[i]:  Sk[b,:] += w_i k_i x_i,  sk[b] += w_i k_i,  n[b] += w_i,
+ * E[b] += w_i d_i.  A neuron is live iff n > 0: one that wins only zero-weight samples is dead.  The samples are
+ * still bucketed by integer count; the weight of each row is read with the row.  With d_labels, the class
+ * histogram per winner is summed as float64 weights into d_class_hist_w [M, n_classes] (every cell written;
+ * args->d_class_hist is not used), in a fixed order per winner, so it is the same on every run for M <= 24576
+ * like the other sums.  d_weight == NULL is dbgsom_accumulate (int32 d_class_hist, d_class_hist_w unused). */
+int dbgsom_accumulate_weighted(const dbgsom_accumulate_args* args, const double* d_weight, double* d_class_hist_w,
+                               void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * K3  neighbourhood smoothing
@@ -353,6 +370,11 @@ int dbgsom_gather_rows(const float* d_X, int64_t ldx, int D, const int64_t* d_ro
  */
 int dbgsom_node_stats(const int32_t* d_idx, int32_t idx_stride, const double* d_dist, int32_t dist_stride,
                       int64_t N, const int32_t* d_pos, int32_t M, double bandwidth, double* d_out, void* stream);
+/* Same with frequency weights: every sample's term (topographic-error indicator, distance, hit, density term) is
+ * multiplied by d_weight[i]; the caller divides the first two by sum_i w_i. */
+int dbgsom_node_stats_weighted(const int32_t* d_idx, int32_t idx_stride, const double* d_dist, int32_t dist_stride,
+                               int64_t N, const int32_t* d_pos, int32_t M, double bandwidth, const double* d_weight,
+                               double* d_out, void* stream);
 
 /* replaces  BaseSom._get_u_matrix  dbgsom/BaseSom.py:320-337:
  * d_out[i] = sum_j d_colw[j] * ||W[i,:] - W[j,:]||_2  (float64, direct differences like scipy cdist);
@@ -367,6 +389,15 @@ int dbgsom_umatrix(const double* d_W, int32_t M, int32_t D, int64_t ldw, const d
 int dbgsom_label_hist(const int32_t* d_idx, int32_t idx_stride, const int32_t* d_labels, int64_t N,
                       int64_t sample_offset, int32_t M, int32_t n_classes, int32_t* d_counts, int64_t* d_first,
                       void* stream);
+/* Same with frequency weights, for winners d_idx [N] (stride 1): d_counts float64 [M, n_classes] = sum of the
+ * weights per cell, added per winner in ascending sample order (the same on every run for M <= 24576, so a tie
+ * between two classes cannot flip between runs), and d_first = smallest global sample index among the samples of
+ * the cell with weight > 0 (statistics.mode over the samples that are present).  The samples are grouped by winner
+ * in d_workspace (dbgsom_label_hist_weighted_workspace_bytes(N, M) bytes). */
+size_t dbgsom_label_hist_weighted_workspace_bytes(int64_t N, int32_t M);
+int dbgsom_label_hist_weighted(const int32_t* d_idx, const int32_t* d_labels, const double* d_weight, int64_t N,
+                               int64_t sample_offset, int32_t M, int32_t n_classes, double* d_counts, int64_t* d_first,
+                               void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * hop matrix on the device (SURVEY.md section 8(f) rank 2)
