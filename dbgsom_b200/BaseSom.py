@@ -157,6 +157,7 @@ class BaseSom(BaseEstimator):
             distributed=self.distributed if distributed is None else distributed,
             bound_scale=self.bound_scale,
             strict_ties=self.strict_ties,
+            capacity_hint=self._capacity_hint(),
         )
 
     def _check_arguments(self) -> None:

@@ -18,6 +18,7 @@ from typing import Sequence
 import numpy as np
 
 from . import _native as nat
+from . import streaming
 from .hostmath import class_entropy, column_moments_to_stats
 
 _UPLOAD_ROWS = 1 << 20
@@ -130,6 +131,7 @@ class DeviceEngine:
         distributed: bool = False,
         bound_scale: float = 0.0,
         strict_ties: bool = False,
+        capacity_hint: int = 0,
     ) -> None:
         import torch
 
@@ -180,6 +182,16 @@ class DeviceEngine:
         self.W = None
         self.M = 0
         self.n_previous_rows = 0
+        # Streaming (streaming.py, DESIGN.md "Streaming fits"): samples that do not fit in device memory stay in the
+        # caller's host array and pass through the device in chunks of `stream_rows` rows every epoch.  0 plans
+        # automatically (stream only when the resident fit would not fit); DBGSOM_STREAM_ROWS=n forces chunks of n rows.
+        self.stream_rows = streaming.stream_rows_from_env()
+        self.capacity_hint = int(capacity_hint)  # map capacity the fit will ask for (sizes the plan)
+        self.streaming = False
+        self.chunks = None        # [(c0, c1)] row ranges of the chunks when streaming
+        self._host_X = None
+        self._stager = None
+        self._copy_stream = None
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
@@ -233,10 +245,17 @@ class DeviceEngine:
         return out
 
     def close(self) -> None:
+        if self._stager is not None:
+            # no copy may still read the page-locked ring when it is unregistered
+            self.torch.cuda.synchronize(self.dev)
+            self._stager.close()
+            self._stager = None
+        self._host_X = None
         self._ws.clear()
         self._perm_cache.clear()
         for name in ("X", "X16_hi", "X16_lo", "xnorm16", "W", "W32", "W16_hi", "W16_lo", "Wb16", "_row_hash", "labels", "weight",
-                     "part", "hop", "_final_idx", "row_perm", "tile_mask", "tile_bound"):
+                     "part", "hop", "_final_idx", "row_perm", "tile_mask", "tile_bound", "_slots", "_cx16", "_cpart",
+                     "_chist", "_cidx", "_cdist"):
             if hasattr(self, name):
                 setattr(self, name, None)
 
@@ -249,6 +268,9 @@ class DeviceEngine:
         torch = self.torch
         with torch.cuda.device(self.dev):
             self.N, self.D = int(X.shape[0]), int(X.shape[1])
+            rows = self._plan_rows(self.N, self.D, int(n_classes) if y is not None else 0, sample_weight is not None)
+            if rows is not None:
+                return self._load_streamed(X, y, n_classes, sample_weight, rows)
             self.X = self._upload_matrix(X)
             self.ldx = int(self.X.shape[1])
             self.n_classes = int(n_classes)
@@ -260,6 +282,21 @@ class DeviceEngine:
                 np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev))
             return self._column_statistics()
 
+    def free_device_bytes(self) -> int:
+        """Device bytes a fit may still allocate: free memory plus what torch has cached but not handed out, less
+        `streaming.free_margin`."""
+        free, total = self.torch.cuda.mem_get_info(self.dev)
+        cached = self.torch.cuda.memory_reserved(self.dev) - self.torch.cuda.memory_allocated(self.dev)
+        return int(free) + int(cached) - streaming.free_margin(total)
+
+    def _plan_rows(self, n: int, d: int, n_classes: int, weighted: bool, capacity: int | None = None) -> int | None:
+        """Chunk rows of a streamed fit, or None for the resident one (`streaming.plan_stream`)."""
+        if self.stream_rows > 0:
+            return streaming._round_up(int(self.stream_rows), streaming.ROW_GRANULE)
+        cap = max(int(self.capacity_hint if capacity is None else capacity), 4)
+        return streaming.plan_stream(n, d, cap, n_classes, weighted, self.free_device_bytes(),
+                                     self.lib.dbgsom_accumulate_workspace_bytes, self.lib.dbgsom_bmu_workspace_bytes)
+
     def _set_weights(self, weight_dev) -> None:
         self.weight = weight_dev
         if weight_dev is None:
@@ -270,31 +307,53 @@ class DeviceEngine:
         total = weight_dev.sum().reshape(1)
         self.weight_total = float(self.comm.allreduce_(total).item())
 
-    def _column_statistics(self) -> dict:
-        torch = self.torch
-        # K4: moments about a common data row (rank 0's first row)
-        shift_row = self.X[0].clone()
-        self.comm.broadcast_(shift_row, 0)
-        parts = torch.zeros((nat.COLSTATS_PARTS, 2 * self.ldx + 1), dtype=torch.float64, device=self.dev)
-        if self.weight is None:
+    def _colstats_parts(self, X, n: int, shift_row, weight) -> np.ndarray:
+        """K4 over n rows of X: the [COLSTATS_PARTS, 2 ldx + 1] row-block parts on the host."""
+        parts = self.torch.zeros((nat.COLSTATS_PARTS, 2 * self.ldx + 1), dtype=self.torch.float64, device=self.dev)
+        if weight is None:
             nat.check(
                 self.lib.dbgsom_colstats(
-                    self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), parts.data_ptr(), self._stream()
+                    X.data_ptr(), n, self.ldx, self.ldx, shift_row.data_ptr(), parts.data_ptr(), self._stream()
                 ),
                 "dbgsom_colstats",
             )
         else:
             nat.check(
                 self.lib.dbgsom_colstats_weighted(
-                    self.X.data_ptr(), self.N, self.ldx, self.ldx, shift_row.data_ptr(), self.weight.data_ptr(),
+                    X.data_ptr(), n, self.ldx, self.ldx, shift_row.data_ptr(), weight.data_ptr(),
                     parts.data_ptr(), self._stream(),
                 ),
                 "dbgsom_colstats_weighted",
             )
         self.launches += 1
+        return parts.cpu().numpy()
+
+    def _column_statistics(self) -> dict:
+        torch = self.torch
+        # K4: moments about a common data row (rank 0's first row)
+        if self.streaming:
+            shift_row = torch.zeros(self.ldx, dtype=torch.float32, device=self.dev)
+            shift_row[: self.D] = torch.from_numpy(np.asarray(self._host_X[0], dtype=np.float32)).to(self.dev)
+        else:
+            shift_row = self.X[0].clone()
+        self.comm.broadcast_(shift_row, 0)
         # the row-block parts are added on the host in a fixed order: the same statistics on every run
-        p = parts.cpu().numpy()
-        moments = torch.from_numpy(np.append(p[:, : 2 * self.ldx].sum(axis=0), p[:, 2 * self.ldx].max())).to(self.dev)
+        if not self.streaming:
+            p = self._colstats_parts(self.X, self.N, shift_row, self.weight)
+            sums, maxabs = p[:, : 2 * self.ldx].sum(axis=0), p[:, 2 * self.ldx].max()
+        else:
+            # streamed: each chunk's parts are added, then the chunk sums in chunk order
+            acc = {"sums": np.zeros(2 * self.ldx), "max": 0.0}
+
+            def body(c, c0, c1, x):
+                w = self.weight[c0:c1] if self.weight is not None else None
+                p = self._colstats_parts(x, c1 - c0, shift_row, w)
+                acc["sums"] = acc["sums"] + p[:, : 2 * self.ldx].sum(axis=0)
+                acc["max"] = max(acc["max"], float(p[:, 2 * self.ldx].max()))
+
+            self._stream_pass(body)
+            sums, maxabs = acc["sums"], acc["max"]
+        moments = torch.from_numpy(np.append(sums, maxabs)).to(self.dev)
         self.comm.allreduce_(moments[: 2 * self.ldx])
         self.comm.allreduce_(moments[2 * self.ldx :], "max")
         m = moments.cpu().numpy()
@@ -342,6 +401,99 @@ class DeviceEngine:
             self._set_weights(weight_dev)
             return self._column_statistics()
 
+    # ------------------------------------------------------------------ streamed data
+    def _load_streamed(self, X, y, n_classes: int, sample_weight, rows: int) -> dict:
+        """`load_data` for a streamed fit: only per-sample vectors go to the device (labels, weights; the winners and
+        the chunk-local sort permutation are allocated here), the rows stay in the caller's array."""
+        torch = self.torch
+        if X.dtype not in (np.float32, np.float64):
+            raise ValueError("streamed samples must be float32 or float64")
+        self.streaming = True
+        self._host_X = X
+        self.ldx = _round_up(self.D, 4)
+        self.ld16 = _round_up(self.ldx, 64)
+        self.chunk_rows = int(min(rows, _round_up(max(self.N, 1), streaming.ROW_GRANULE)))
+        self.chunks = streaming.chunk_bounds(self.N, self.chunk_rows)
+        self.n_classes = int(n_classes)
+        self.labels = None
+        if y is not None:
+            self.labels = torch.from_numpy(np.ascontiguousarray(y, dtype=np.int32)).to(self.dev)
+        self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
+        self._set_weights(None if sample_weight is None else torch.from_numpy(
+            np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev))
+        # two float32 chunk slots (one is filled while the other is computed on); every other chunk buffer is single,
+        # because all compute runs on one stream
+        self._slots = [torch.empty((self.chunk_rows, self.ldx), dtype=torch.float32, device=self.dev) for _ in range(2)]
+        self._slot_ready = [torch.cuda.Event() for _ in range(2)]
+        self._slot_free = [torch.cuda.Event() for _ in range(2)]
+        self.row_perm = torch.empty(self.N, dtype=torch.int32, device=self.dev)  # chunk-local K2 order per chunk
+        self._chunks_sorted = False  # row_perm holds every chunk's K2 order (after the first epoch)
+        self._sorted_search = False  # some chunk's search read its samples sorted (the post passes then do too)
+        self._cx16 = None
+        self._copy_stream = torch.cuda.Stream(self.dev)
+        self._stager = streaming.HostStager(torch, streaming.HostStager.piece_rows_for(self.chunk_rows, self.ldx),
+                                            self.D, self.ldx)
+        return self._column_statistics()
+
+    def _stream_pass(self, body) -> None:
+        """One pass over the samples in chunks: body(c, c0, c1, x) enqueues the work on chunk c, whose float32 rows
+        x [c1 - c0, ldx] are in a device slot.  The rows of chunk c + 1 are staged by the host threads and copied on
+        a side stream into the other slot while chunk c is computed; a slot is overwritten only after the work on
+        the chunk before has been enqueued and has run (event `_slot_free`)."""
+        torch = self.torch
+        main = torch.cuda.current_stream(self.dev)
+        copy = self._copy_stream
+        copy.wait_stream(main)  # earlier readers of the slots are done before they are overwritten
+        with self._stager.pieces(self._host_X, self.chunks) as pieces:
+            pieces = iter(pieces)
+
+            def upload(c):
+                s, (c0, c1) = c % 2, self.chunks[c]
+                if c >= 2:
+                    copy.wait_event(self._slot_free[s])
+                done = c0
+                with torch.cuda.stream(copy):
+                    while done < c1:
+                        _, r0, r1, host, release = next(pieces)
+                        self._slots[s][r0 - c0 : r1 - c0].copy_(host, non_blocking=True)
+                        ev = torch.cuda.Event()
+                        ev.record(copy)
+                        release(ev)
+                        done = r1
+                    self._slot_ready[s].record(copy)
+
+            upload(0)
+            for c, (c0, c1) in enumerate(self.chunks):
+                s = c % 2
+                main.wait_event(self._slot_ready[s])
+                body(c, c0, c1, self._slots[s][: c1 - c0])
+                self._slot_free[s].record(main)
+                if c + 1 < len(self.chunks):
+                    upload(c + 1)
+
+    def _chunk_x16(self, x, n: int, need_lo: bool, perm=None):
+        """fp16 shadows of one chunk's rows (in the order `perm`, chunk-local, when given)."""
+        torch = self.torch
+        if self._cx16 is None or (need_lo and self._cx16[1] is None):
+            self._cx16 = (torch.empty((self.chunk_rows, self.ld16), dtype=torch.float16, device=self.dev),
+                          torch.empty((self.chunk_rows, self.ld16), dtype=torch.float16, device=self.dev) if need_lo else None,
+                          torch.empty(self.chunk_rows, dtype=torch.float32, device=self.dev))
+        hi, lo, xn = self._cx16
+        lo_ptr = lo.data_ptr() if need_lo else None
+        with self._Phase(self, "prepare_x16"):
+            if perm is None:
+                nat.check(self.lib.dbgsom_prepare_x16(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(), self.scale,
+                                                      hi.data_ptr(), lo_ptr, self.ld16, xn.data_ptr(), self._stream()),
+                          "dbgsom_prepare_x16")
+                self.launches += 1
+            else:
+                nat.check(self.lib.dbgsom_prepare_x16_sorted(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(),
+                                                             self.scale, perm.data_ptr(), hi.data_ptr(), lo_ptr, self.ld16,
+                                                             xn.data_ptr(), self._stream()),
+                          "dbgsom_prepare_x16_sorted")
+                self.launches += 2
+        return hi[:n], (lo[:n] if need_lo else None), xn[:n]
+
     def _ensure_x16(self, need_lo: bool) -> None:
         torch = self.torch
         if self.X16_hi is not None and (self.X16_lo is not None or not need_lo):
@@ -374,13 +526,18 @@ class DeviceEngine:
         self.wmax = torch.zeros(4, dtype=torch.float32, device=self.dev)  # see dbgsom_prepare_w
         self.part = torch.zeros(cap * self.ldx + 3 * cap, dtype=torch.float64, device=self.dev)
         self.change = torch.zeros(1, dtype=torch.float64, device=self.dev)
-        self.idx = torch.empty((self.N, 2), dtype=torch.int32, device=self.dev)
+        # the epoch's winners (streamed fits keep only the int32 winner of every sample resident)
+        self.idx = torch.empty((self.N, 1 if self.streaming else 2), dtype=torch.int32, device=self.dev)
         self.bmu_stats = torch.zeros(8, dtype=torch.int64, device=self.dev)
         # weighted fits sum the class histogram as float64 weights
         hist_dtype = torch.int32 if self.weight is None else torch.float64
         self.class_hist = (
             torch.zeros((cap, self.n_classes), dtype=hist_dtype, device=self.dev) if self.labels is not None else None
         )
+        if self.streaming:
+            # one chunk's K2 sums and class histogram, added into the epoch's in chunk order
+            self._cpart = torch.empty_like(self.part)
+            self._chist = torch.empty_like(self.class_hist) if self.class_hist is not None else None
         if old is not None:
             for new, prev in zip(self.W, old):
                 new[: prev.shape[0]] = prev
@@ -400,7 +557,13 @@ class DeviceEngine:
             local = rows - self.sample_offset
             owned = (local >= 0) & (local < self.N)
             W0 = self.W[0]
-            if owned.any():
+            if owned.any() and self.streaming:
+                # the rows the device gather would read, rounded through float32 like the device copy of X
+                tmp = np.zeros((len(rows), self.ldx), dtype=np.float64)
+                tmp[:, : self.D] = np.asarray(self._host_X[np.where(owned, local, 0)]).astype(np.float32)
+                tmp[~owned] = 0
+                W0[: len(rows)] = torch.from_numpy(tmp).to(self.dev)
+            elif owned.any():
                 src = torch.from_numpy(np.where(owned, local, 0)).to(self.dev)
                 tmp = torch.zeros((len(rows), self.ldx), dtype=torch.float64, device=self.dev)
                 nat.check(
@@ -757,6 +920,8 @@ class DeviceEngine:
         """One training epoch on the resident data; returns per-neuron error, counts, change."""
         torch = self.torch
         with torch.cuda.device(self.dev):
+            if self.streaming:
+                return self._epoch_streamed(sigma, pack_rows, entropy_error, _force_simt)
             m, cur = self.M, self.W[self.cur]
             be = (nat.BMU_SIMT, 0) if _force_simt else self._pick_backend(self.N, m)
             x16 = None
@@ -791,40 +956,97 @@ class DeviceEngine:
         self.launches += 2
         self._sort_age = 0
 
-    def _update_and_smooth(self, be, idx, sigma: float, pack_rows: bool, entropy_error: bool, resort: bool = False) -> dict:
-        """K2 -> all-reduce -> K3 -> read-back, given the winners of the current prototypes."""
-        torch = self.torch
+    def _accumulate(self, X, n: int, idx, part, labels, weight, hist):
+        """K2 over n rows of X with winners idx into `part` (and the class histogram `hist` when labels are given);
+        returns the workspace, which holds the samples' order grouped by winner."""
         m, cur = self.M, self.W[self.cur]
-        # K2
-        part = self.part[: m * self.ldx + 3 * m]
-        use_hist = entropy_error and self.labels is not None
         acc = nat.AccumulateArgs()
-        acc.d_X, acc.N, acc.D, acc.ldx = self.X.data_ptr(), self.N, self.ldx, self.ldx
+        acc.d_X, acc.N, acc.D, acc.ldx = X.data_ptr(), n, self.ldx, self.ldx
         acc.d_bmu, acc.d_W, acc.M = idx.data_ptr(), cur.data_ptr(), m
         acc.inv_total_variance = 1.0 / self.total_variance if self.total_variance > 0 else float("inf")
         acc.d_part = part.data_ptr()
-        acc.d_labels = self.labels.data_ptr() if use_hist else None
-        acc.n_classes = self.n_classes if use_hist else 0
-        acc.d_class_hist = self.class_hist.data_ptr() if use_hist and self.weight is None else None
-        ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(self.N, m, self.ldx))
+        acc.d_labels = labels.data_ptr() if labels is not None else None
+        acc.n_classes = self.n_classes if labels is not None else 0
+        acc.d_class_hist = hist.data_ptr() if labels is not None and weight is None else None
+        ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(n, m, self.ldx))
         acc.d_workspace, acc.workspace_bytes = ws.data_ptr(), ws.numel()
         with self._Phase(self, "accumulate"):
-            if self.weight is None:
+            if weight is None:
                 nat.check(self.lib.dbgsom_accumulate(acc, self._stream()), "dbgsom_accumulate")
             else:
                 nat.check(
                     self.lib.dbgsom_accumulate_weighted(
-                        acc, self.weight.data_ptr(), self.class_hist.data_ptr() if use_hist else None, self._stream()
+                        acc, weight.data_ptr(), hist.data_ptr() if labels is not None else None, self._stream()
                     ),
                     "dbgsom_accumulate_weighted",
                 )
-        self.launches += (10 if m <= 24576 else 8) + (1 if use_hist else 0)  # stable scatter: 3 kernels
+        self.launches += (10 if m <= 24576 else 8) + (1 if labels is not None else 0)  # stable scatter: 3 kernels
+        return ws
+
+    def _update_and_smooth(self, be, idx, sigma: float, pack_rows: bool, entropy_error: bool, resort: bool = False) -> dict:
+        """K2 -> all-reduce -> K3 -> read-back, given the winners of the current prototypes."""
+        m = self.M
+        # K2
+        part = self.part[: m * self.ldx + 3 * m]
+        use_hist = entropy_error and self.labels is not None
+        ws = self._accumulate(self.X, self.N, idx, part, self.labels if use_hist else None, self.weight,
+                              self.class_hist if use_hist else None)
         if resort and self.X16_hi is not None:
             self._sort_age += 1
             if self.row_perm is None or self._sort_age >= self.resort_every:
                 with self._Phase(self, "resort"):
                     self._resort_samples(idx, m, ws)
+        return self._reduce_and_smooth(be, part, use_hist, sigma, pack_rows, entropy_error)
 
+    def _epoch_streamed(self, sigma: float, pack_rows: bool, entropy_error: bool, force_simt: bool) -> dict:
+        """`epoch` on streamed samples: per chunk, fp16 shadows (in the order K2 left the chunk's samples in the
+        epoch before), BMU search and K2 into a chunk `part`, which is added into the epoch's in chunk order; then the
+        all-reduce, K3 and the read-back of the resident epoch."""
+        m, cur = self.M, self.W[self.cur]
+        # the backend follows the whole sample count: small chunks must not turn the tensor search into the SIMT one
+        be = (nat.BMU_SIMT, 0) if force_simt else self._pick_backend(self.N, m)
+        tensor, need_lo = be[0] == nat.BMU_TENSOR, be[1] == 3
+        sorted_ = self._chunks_sorted
+        selective = [sorted_ and self._select_eligible(c1 - c0, m, be) for c0, c1 in self.chunks]
+        with self._Phase(self, "prepare_w"):
+            mpad = self._prepare_w(cur, m, tensor, need_lo, top1=True, map_order=any(selective))
+        part = self.part[: m * self.ldx + 3 * m]
+        cpart = self._cpart[: part.numel()]
+        use_hist = entropy_error and self.labels is not None
+        hist = self.class_hist[:m] if use_hist else None
+        chist = self._chist[:m] if use_hist else None
+        idx = self.idx.view(-1)[: self.N]
+
+        def body(c, c0, c1, x):
+            n = c1 - c0
+            perm = self.row_perm[c0:c1]
+            # like the resident epoch, only the selective search reads the samples in sorted order
+            x16 = self._chunk_x16(x, n, need_lo, perm if selective[c] else None) if tensor else None
+            self._bmu_search(x, n, self.ldx, x16, cur, m, mpad, 1, False, idx[c0:c1], None, be,
+                             row_perm=perm if selective[c] else None, selective=selective[c])
+            first = c == 0
+            ws = self._accumulate(x, n, idx[c0:c1], part if first else cpart,
+                                  self.labels[c0:c1] if use_hist else None,
+                                  self.weight[c0:c1] if self.weight is not None else None,
+                                  (hist if first else chist) if use_hist else None)
+            if not first:
+                with self._Phase(self, "chunk_sum"):
+                    part.add_(cpart)
+                    if use_hist:
+                        hist.add_(chist)
+            # the chunk's samples grouped by winner: the shadow order of its next epoch
+            off = int(self.lib.dbgsom_accumulate_perm_offset(n, m))
+            perm.copy_(ws[off : off + 4 * n].view(self.torch.int32))
+
+        self._stream_pass(body)
+        self._chunks_sorted = True
+        self._sorted_search |= any(selective)
+        return self._reduce_and_smooth(be, part, use_hist, sigma, pack_rows, entropy_error)
+
+    def _reduce_and_smooth(self, be, part, use_hist: bool, sigma: float, pack_rows: bool, entropy_error: bool) -> dict:
+        """All-reduce of the epoch sums -> K3 -> read-back."""
+        torch = self.torch
+        m, cur = self.M, self.W[self.cur]
         # the one collective of the path: per-neuron partial sums (+ class histogram)
         with self._Phase(self, "allreduce"):
             self.comm.allreduce_(part)
@@ -912,6 +1134,15 @@ class DeviceEngine:
             W = self.W[self.cur ^ 1] if previous else self.W[self.cur]
             m = self.n_previous_rows if previous else self.M
             n_bmu = min(n_bmu, m)
+            if self.streaming:
+                dist_h = np.empty((self.N, n_bmu), dtype=np.float64)
+                idx_h = np.empty((self.N, n_bmu), dtype=np.int64)
+
+                def out(c, c0, c1, idx, dist):
+                    dist_h[c0:c1], idx_h[c0:c1] = dist.cpu().numpy(), idx.cpu().numpy()
+
+                self._bmu_pass_streamed(W, m, n_bmu, self.strict_ties, out)
+                return dist_h, idx_h
             be = self._pick_backend(self.N, m)
             x16 = None
             if be[0] == nat.BMU_TENSOR:
@@ -922,6 +1153,34 @@ class DeviceEngine:
             self._run_bmu(self.X, self.N, self.ldx, x16, W, m, n_bmu, True, idx, dist, backend=be,
                           row_perm=self.row_perm if be[0] == nat.BMU_TENSOR else None)
             return dist.cpu().numpy(), idx.cpu().numpy().astype(np.int64)
+
+    def _bmu_pass_streamed(self, W, m: int, n_bmu: int, strict: bool, out) -> None:
+        """BMU search of the streamed samples against W (what `_run_bmu` does on resident ones): per chunk, the
+        chunk's winners idx int32 [n, n_bmu] and distances dist float64 [n, n_bmu] go to out(c, c0, c1, idx, dist),
+        which enqueues what reads them before the next chunk overwrites them."""
+        torch = self.torch
+        be = self._pick_backend(self.N, m)
+        tensor, need_lo = be[0] == nat.BMU_TENSOR, be[1] == 3
+        if W.shape[0] > self.W32.shape[0]:
+            self.W32 = torch.zeros((W.shape[0], self.ldx), dtype=torch.float32, device=self.dev)
+        with self._Phase(self, "prepare_w"):
+            mpad = self._prepare_w(W, m, tensor, need_lo, top1=n_bmu == 1)
+        if getattr(self, "_cidx", None) is None or self._cidx.numel() < self.chunk_rows * n_bmu:
+            self._cidx = torch.empty(self.chunk_rows * max(n_bmu, 2), dtype=torch.int32, device=self.dev)
+            self._cdist = torch.empty(self.chunk_rows * max(n_bmu, 2), dtype=torch.float64, device=self.dev)
+        # sorted shadows where the resident fit has them: once the selective search has sorted the samples
+        sorted_ = self._chunks_sorted and self._sorted_search
+
+        def body(c, c0, c1, x):
+            n = c1 - c0
+            perm = self.row_perm[c0:c1] if (tensor and sorted_) else None
+            x16 = self._chunk_x16(x, n, need_lo, perm) if tensor else None
+            idx = self._cidx[: n * n_bmu].view(n, n_bmu)
+            dist = self._cdist[: n * n_bmu].view(n, n_bmu)
+            self._bmu_search(x, n, self.ldx, x16, W, m, mpad, n_bmu, True, idx, dist, be, strict=strict, row_perm=perm)
+            out(c, c0, c1, idx, dist)
+
+        self._stream_pass(body)
 
     # ------------------------------------------------------------------ post-training passes
     def _bmu_train_device(self, n_bmu: int, previous: bool):
@@ -949,8 +1208,12 @@ class DeviceEngine:
         and the node statistics (:181-211); the u-matrix (:320-337) uses the updated prototypes."""
         torch = self.torch
         with torch.cuda.device(self.dev):
-            idx, dist, m = self._bmu_train_device(2, previous=True)
-            n_bmu = int(idx.shape[1])
+            if self.streaming:
+                m = self.n_previous_rows  # the chunks are searched below, once the bandwidth is known
+                n_bmu = min(2, m)
+            else:
+                idx, dist, m = self._bmu_train_device(2, previous=True)
+                n_bmu = int(idx.shape[1])
             M, cur = self.M, self.W[self.cur]
             total = float(np.sum(degrees))
             if total > 0:
@@ -968,23 +1231,20 @@ class DeviceEngine:
             pos = torch.from_numpy(np.ascontiguousarray(positions[:m], dtype=np.int32)).to(self.dev)
             out = torch.empty(2 + 2 * m, dtype=torch.float64, device=self.dev)
             ok = bandwidth > 0 and math.isfinite(bandwidth)
-            if self.weight is None:
-                nat.check(
-                    self.lib.dbgsom_node_stats(
-                        idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, self.N, pos.data_ptr(), m,
-                        bandwidth if ok else 1.0, out.data_ptr(), self._stream(),
-                    ),
-                    "dbgsom_node_stats",
-                )
+            if self.streaming:
+                # per chunk into `cout`, added into `out` in chunk order
+                cout = torch.empty_like(out)
+
+                def stats(c, c0, c1, idx, dist):
+                    w = self.weight[c0:c1] if self.weight is not None else None
+                    self._node_stats(idx, dist, n_bmu, c1 - c0, pos, m, bandwidth if ok else 1.0, w,
+                                     out if c == 0 else cout)
+                    if c > 0:
+                        out.add_(cout)
+
+                self._bmu_pass_streamed(self.W[self.cur ^ 1], m, n_bmu, True, stats)
             else:
-                nat.check(
-                    self.lib.dbgsom_node_stats_weighted(
-                        idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, self.N, pos.data_ptr(), m,
-                        bandwidth if ok else 1.0, self.weight.data_ptr(), out.data_ptr(), self._stream(),
-                    ),
-                    "dbgsom_node_stats_weighted",
-                )
-            self.launches += 2
+                self._node_stats(idx, dist, n_bmu, self.N, pos, m, bandwidth if ok else 1.0, self.weight, out)
             self.comm.allreduce_(out)
             o = out.cpu().numpy()
             dens = o[2 + m :].copy()
@@ -993,9 +1253,36 @@ class DeviceEngine:
             return {"te_count": float(o[0]), "qe_sum": float(o[1]), "hits": o[2 : 2 + m].copy(), "dens_sum": dens,
                     "avg_dist": avg_host, "weights": self.weights(), "n_rows": m}
 
+    def _node_stats(self, idx, dist, n_bmu: int, n: int, pos, m: int, bandwidth: float, weight, out) -> None:
+        if weight is None:
+            nat.check(
+                self.lib.dbgsom_node_stats(
+                    idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, n, pos.data_ptr(), m,
+                    bandwidth, out.data_ptr(), self._stream(),
+                ),
+                "dbgsom_node_stats",
+            )
+        else:
+            nat.check(
+                self.lib.dbgsom_node_stats_weighted(
+                    idx.data_ptr(), n_bmu, dist.data_ptr(), n_bmu, n, pos.data_ptr(), m,
+                    bandwidth, weight.data_ptr(), out.data_ptr(), self._stream(),
+                ),
+                "dbgsom_node_stats_weighted",
+            )
+        self.launches += 2
+
     def final_winners(self) -> None:
         """Top-1 BMU of the training samples on the current (reduced) map; stays on the device."""
         with self.torch.cuda.device(self.dev):
+            if self.streaming:
+                self._final_idx = self.torch.empty((self.N, 1), dtype=self.torch.int32, device=self.dev)
+
+                def keep(c, c0, c1, idx, dist):
+                    self._final_idx[c0:c1].copy_(idx)
+
+                self._bmu_pass_streamed(self.W[self.cur], self.M, 1, True, keep)
+                return
             self._final_idx, _, _ = self._bmu_train_device(1, previous=False)
 
     def winners_host(self) -> np.ndarray:
@@ -1008,6 +1295,8 @@ class DeviceEngine:
         torch = self.torch
         with torch.cuda.device(self.dev):
             m = self.M
+            if self.streaming:
+                return self._label_histogram_chunked(n_classes)
             if self.weight is not None:
                 counts = torch.empty((m, n_classes), dtype=torch.float64, device=self.dev)
                 first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
@@ -1038,16 +1327,56 @@ class DeviceEngine:
             self.comm.allreduce_(first, "min")
             return counts.cpu().numpy().astype(np.float64), first.cpu().numpy()
 
+    def _label_histogram_chunked(self, n_classes: int):
+        """`label_histogram` of a streamed fit: the same kernels per chunk (global sample offset + c0), counts added
+        in chunk order, `first` the minimum over the chunks."""
+        torch = self.torch
+        m, weighted = self.M, self.weight is not None
+        counts = torch.zeros((m, n_classes), dtype=torch.float64 if weighted else torch.int64, device=self.dev)
+        first = torch.full((m, n_classes), np.iinfo(np.int64).max, dtype=torch.int64, device=self.dev)
+        c_counts = torch.empty((m, n_classes), dtype=torch.float64 if weighted else torch.int32, device=self.dev)
+        c_first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
+        for c0, c1 in self.chunks:
+            n, idx = c1 - c0, self._final_idx[c0:c1]
+            if weighted:
+                ws = self._workspace("labels", self.lib.dbgsom_label_hist_weighted_workspace_bytes(n, m))
+                nat.check(
+                    self.lib.dbgsom_label_hist_weighted(
+                        idx.data_ptr(), self.labels[c0:c1].data_ptr(), self.weight[c0:c1].data_ptr(), n,
+                        self.sample_offset + c0, m, n_classes, c_counts.data_ptr(), c_first.data_ptr(), ws.data_ptr(),
+                        ws.numel(), self._stream(),
+                    ),
+                    "dbgsom_label_hist_weighted",
+                )
+            else:
+                nat.check(
+                    self.lib.dbgsom_label_hist(
+                        idx.data_ptr(), 1, self.labels[c0:c1].data_ptr(), n, self.sample_offset + c0, m, n_classes,
+                        c_counts.data_ptr(), c_first.data_ptr(), self._stream(),
+                    ),
+                    "dbgsom_label_hist",
+                )
+            self.launches += 3
+            counts.add_(c_counts)
+            torch.minimum(first, c_first, out=first)
+        self.comm.allreduce_(counts)
+        self.comm.allreduce_(first, "min")
+        return counts.cpu().numpy().astype(np.float64), first.cpu().numpy()
+
     def bmu(self, X: np.ndarray, W: np.ndarray, n_bmu: int):
-        """Stand-alone BMU search (predict path): host samples against host prototypes."""
+        """Stand-alone BMU search (predict path): host samples against host prototypes.
+
+        Samples whose upload would not fit in device memory (or `stream_rows` > 0) are searched in row chunks; the
+        shadow shift and scale still come from all of X, so every row gets the winner and distance of one call."""
         torch = self.torch
         with torch.cuda.device(self.dev):
             n, d = int(X.shape[0]), int(X.shape[1])
             if d != W.shape[1]:
                 raise ValueError(f"X has {d} features, the map has {W.shape[1]}")
-            self.N, self.D = n, d
-            self.X = self._upload_matrix(np.asarray(X))
-            self.ldx = int(self.X.shape[1])
+            rows = self._plan_rows(n, d, 0, False, capacity=W.shape[0])
+            chunks = [(0, n)] if rows is None else streaming.chunk_bounds(n, rows)
+            self.N, self.D = chunks[0][1] - chunks[0][0], d
+            self.ldx = _round_up(d, 4)
             self.ld16 = _round_up(self.ldx, 64)
             self.labels, self.n_classes = None, 0
             self.row_perm = None
@@ -1057,27 +1386,36 @@ class DeviceEngine:
             self.set_map(np.asarray(W))
             # shadows for the tensor path: centre on the prototypes' mean, scale from both operands
             be = self._pick_backend(n, self.M)
-            x16 = None
-            if be[0] == nat.BMU_TENSOR:
+            tensor = be[0] == nat.BMU_TENSOR
+            if tensor:
                 centre = np.asarray(W, dtype=np.float64).mean(axis=0)
                 shift = np.zeros(self.ldx, dtype=np.float32)
                 shift[:d] = centre
                 self.shift = torch.from_numpy(shift).to(self.dev)
-                maxabs = float(max(np.abs(np.asarray(X) - centre).max(), np.abs(np.asarray(W) - centre).max()))
+                x_max = max(float(np.abs(np.asarray(X[c0:c1]) - centre).max()) for c0, c1 in chunks)
+                maxabs = float(max(x_max, np.abs(np.asarray(W) - centre).max()))
                 self.scale = 1.0 if not (maxabs > 0 and math.isfinite(maxabs)) else 2.0 ** math.floor(
                     math.log2(2.0**14 / maxabs)
                 )  # both operands are in hand here, so the bound is exact
-                self.X16_hi = None
-                self._ensure_x16(be[1] == 3)
-                x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
             else:
                 self.shift = torch.zeros(self.ldx, dtype=torch.float32, device=self.dev)
                 self.scale = 1.0
             n_bmu = min(n_bmu, self.M)
-            idx = torch.empty((n, n_bmu), dtype=torch.int32, device=self.dev)
-            dist = torch.empty((n, n_bmu), dtype=torch.float64, device=self.dev)
-            self._run_bmu(self.X, n, self.ldx, x16, self.W[0], self.M, n_bmu, True, idx, dist, backend=be)
-            return dist.cpu().numpy(), idx.cpu().numpy().astype(np.int64)
+            dist_h = np.empty((n, n_bmu), dtype=np.float64)
+            idx_h = np.empty((n, n_bmu), dtype=np.int64)
+            for c0, c1 in chunks:
+                self.N = c1 - c0
+                self.X = self._upload_matrix(np.asarray(X[c0:c1]))
+                x16 = None
+                if tensor:
+                    self.X16_hi = None
+                    self._ensure_x16(be[1] == 3)
+                    x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
+                idx = torch.empty((self.N, n_bmu), dtype=torch.int32, device=self.dev)
+                dist = torch.empty((self.N, n_bmu), dtype=torch.float64, device=self.dev)
+                self._run_bmu(self.X, self.N, self.ldx, x16, self.W[0], self.M, n_bmu, True, idx, dist, backend=be)
+                dist_h[c0:c1], idx_h[c0:c1] = dist.cpu().numpy(), idx.cpu().numpy()
+            return dist_h, idx_h
 
     # ------------------------------------------------------------------ sparse coding (transform)
     def sparse_code(self, Xn: np.ndarray, Wn: np.ndarray, max_iter: int = 1000) -> np.ndarray:
