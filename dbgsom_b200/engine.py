@@ -118,8 +118,92 @@ class Comm:
         return int(counts[: self.rank].sum()), int(counts.sum())
 
 
+class ResidentSamples:
+    """Every sample in HBM for the whole fit: X float32 [N, ldx] and its fp16 shadows, which persist between epochs;
+    a pass over the samples is one chunk, X itself (streaming.StreamedSamples has the same operations).  Once the
+    selective search applies, the shadows are rebuilt in the order K2 grouped the samples by winner (`row_perm`) at
+    its first epoch and then every `resort_every` epochs, since each rebuild is a pass over X."""
+
+    streaming = False
+    winner_cols = 2  # the epoch winners are [N, 2] (streaming.resident_bytes counts them so)
+
+    def __init__(self, eng, X):
+        self.eng, self.X = eng, X
+        self.N = int(X.shape[0])
+        self.chunks = [(0, self.N)]
+        self.X16_hi = self.X16_lo = self.xnorm16 = None
+        self.row_perm = None  # int32 [N]: shadow row p holds sample row_perm[p] (None = natural order)
+        self.age = 0          # selective-eligible epochs since the shadows were last sorted
+
+    def chunk_pass(self, body) -> None:
+        body(0, 0, self.N, self.X)
+
+    def reserve_shadows(self, need_lo: bool) -> bool:
+        """Allocate the shadows unless they exist (with the low half when `need_lo`); True when they were allocated,
+        in natural order and not yet built."""
+        if self.X16_hi is not None and (self.X16_lo is not None or not need_lo):
+            return False
+        torch, dev, ld16 = self.eng.torch, self.eng.dev, self.eng.ld16
+        self.row_perm = None
+        self.X16_hi = torch.empty((self.N, ld16), dtype=torch.float16, device=dev)
+        self.X16_lo = torch.empty((self.N, ld16), dtype=torch.float16, device=dev) if need_lo else None
+        self.xnorm16 = torch.empty(self.N, dtype=torch.float32, device=dev)
+        return True
+
+    def shadows(self, c: int, x, backend, selective):
+        """(shadows, row order) for a search of chunk c with `backend`; (None, None) for the SIMT search.  Every
+        tensor search reads the persistent shadows in their current order, selective (`selective`) or not."""
+        if backend[0] != nat.BMU_TENSOR:
+            return None, None
+        if self.reserve_shadows(backend[1] == 3):
+            self.eng._prepare_x16(self.X, self.N, self.X16_hi, self.X16_lo, self.xnorm16)
+        return (self.X16_hi, self.X16_lo, self.xnorm16), self.row_perm
+
+    def has_order(self, c: int) -> bool:
+        return self.row_perm is not None
+
+    def after_k2(self, c: int, order, eligible: bool) -> None:
+        """`order`: K2's winner-sorted permutation of the epoch; `eligible`: the selective search applied to it."""
+        if not eligible:
+            return
+        eng = self.eng
+        self.age += 1
+        if self.row_perm is None or self.age >= eng.resort_every:
+            with eng._Phase(eng, "resort"):
+                if self.row_perm is None:
+                    self.row_perm = eng.torch.empty(self.N, dtype=eng.torch.int32, device=eng.dev)
+                self.row_perm.copy_(order)
+                eng._prepare_x16(self.X, self.N, self.X16_hi, self.X16_lo, self.xnorm16, self.row_perm)
+            self.age = 0
+
+    def shift_row(self):
+        return self.X[0].clone()
+
+    def start_rows(self, rows: np.ndarray):
+        """float64 [len(rows), ldx] copies of the given local sample rows."""
+        eng, torch = self.eng, self.eng.torch
+        src = torch.from_numpy(rows).to(eng.dev)
+        out = torch.zeros((len(rows), eng.ldx), dtype=torch.float64, device=eng.dev)
+        nat.check(eng.lib.dbgsom_gather_rows(self.X.data_ptr(), eng.ldx, eng.ldx, src.data_ptr(), len(rows),
+                                             out.data_ptr(), eng._stream()),
+                  "dbgsom_gather_rows")
+        eng.launches += 1
+        return out
+
+    def close(self) -> None:
+        self.X = self.X16_hi = self.X16_lo = self.xnorm16 = self.row_perm = None
+
+
+def _sample_buffer(name: str):
+    """Engine attribute read from the sample source: the resident X, its shadows, the shadow-row order (None where
+    the source has no such buffer)."""
+    return property(lambda self: getattr(self.samples, name, None))
+
+
 class DeviceEngine:
     """One fit's worth of device state.  See module docstring."""
+
+    X, X16_hi, X16_lo, xnorm16, row_perm = map(_sample_buffer, ("X", "X16_hi", "X16_lo", "xnorm16", "row_perm"))
 
     # M^2 D above which the smoothing rows are split over the ranks (DBGSOM_K3_SHARD_MIN_WORK overrides; tests)
     K3_SHARD_MIN_WORK = int(os.environ.get("DBGSOM_K3_SHARD_MIN_WORK", 1 << 36))
@@ -162,9 +246,7 @@ class DeviceEngine:
         self.tile_bound = None
         self._tile_ready = False
         self.resort_every = int(os.environ.get("DBGSOM_RESORT_EVERY", "8"))
-        self.row_perm = None      # int32 [N]: shadow row p holds sample row_perm[p] (None = natural order)
         self.tile_mask = None
-        self._sort_age = 0
         self._map_order = None    # prototype indices in map-patch order (from the topology)
         self._perm_cache = {}
         self._epoch_kinds = {"selective": 0, "classic": 0}
@@ -178,7 +260,7 @@ class DeviceEngine:
         self._prof = None
         self.last_bmu_stats = None
         self._ws = {}
-        self.X = None
+        self.samples = None       # ResidentSamples or streaming.StreamedSamples: where the fit's samples live
         self.W = None
         self.M = 0
         self.n_previous_rows = 0
@@ -187,11 +269,21 @@ class DeviceEngine:
         # automatically (stream only when the resident fit would not fit); DBGSOM_STREAM_ROWS=n forces chunks of n rows.
         self.stream_rows = streaming.stream_rows_from_env()
         self.capacity_hint = int(capacity_hint)  # map capacity the fit will ask for (sizes the plan)
-        self.streaming = False
-        self.chunks = None        # [(c0, c1)] row ranges of the chunks when streaming
-        self._host_X = None
-        self._stager = None
-        self._copy_stream = None
+        self._copy_stream = None  # side stream of `epoch_from_host`
+
+    @property
+    def streaming(self) -> bool:
+        """The samples stay in host memory and pass through the device in chunks every epoch."""
+        return self.samples is not None and self.samples.streaming
+
+    @property
+    def chunks(self):
+        """[(c0, c1)] row ranges of one pass over the samples ([(0, N)] when resident)."""
+        return None if self.samples is None else self.samples.chunks
+
+    @property
+    def chunk_rows(self) -> int:
+        return self.samples.chunk_rows
 
     # ------------------------------------------------------------------ helpers
     def _stream(self):
@@ -245,42 +337,42 @@ class DeviceEngine:
         return out
 
     def close(self) -> None:
-        if self._stager is not None:
-            # no copy may still read the page-locked ring when it is unregistered
-            self.torch.cuda.synchronize(self.dev)
-            self._stager.close()
-            self._stager = None
-        self._host_X = None
+        if self.samples is not None:
+            self.samples.close()
         self._ws.clear()
         self._perm_cache.clear()
-        for name in ("X", "X16_hi", "X16_lo", "xnorm16", "W", "W32", "W16_hi", "W16_lo", "Wb16", "_row_hash", "labels", "weight",
-                     "part", "hop", "_final_idx", "row_perm", "tile_mask", "tile_bound", "_slots", "_cx16", "_cpart",
-                     "_chist", "_cidx", "_cdist"):
+        for name in ("W", "W32", "W16_hi", "W16_lo", "Wb16", "_row_hash", "labels", "weight", "part", "hop", "_final_idx",
+                     "tile_mask", "tile_bound", "_cpart", "_chist"):
             if hasattr(self, name):
                 setattr(self, name, None)
 
     # ------------------------------------------------------------------ data
     def load_data(self, X: np.ndarray, y, n_classes: int, sample_weight=None) -> dict:
-        """Upload the samples and reduce the column statistics `fit` needs (K4).
+        """Upload the samples and reduce the column statistics `fit` needs (K4).  Samples that would not fit in
+        device memory (or `stream_rows` > 0) stay in X and are streamed in chunks every epoch.
 
         `sample_weight` (float64 [N], finite, >= 0; this rank's shard): frequency weights -- a sample of weight w
         counts like w copies of it in every sum of the fit.  None runs the unweighted kernels."""
         torch = self.torch
         with torch.cuda.device(self.dev):
             self.N, self.D = int(X.shape[0]), int(X.shape[1])
+            self.ldx = _round_up(self.D, 4)
             rows = self._plan_rows(self.N, self.D, int(n_classes) if y is not None else 0, sample_weight is not None)
-            if rows is not None:
-                return self._load_streamed(X, y, n_classes, sample_weight, rows)
-            self.X = self._upload_matrix(X)
-            self.ldx = int(self.X.shape[1])
-            self.n_classes = int(n_classes)
-            self.labels = None
-            if y is not None:
-                self.labels = torch.from_numpy(np.ascontiguousarray(y, dtype=np.int32)).to(self.dev)
-            self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
-            self._set_weights(None if sample_weight is None else torch.from_numpy(
-                np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev))
-            return self._column_statistics()
+            samples = ResidentSamples(self, self._upload_matrix(X)) if rows is None else streaming.StreamedSamples(
+                self, X, rows)
+            labels = None if y is None else torch.from_numpy(np.ascontiguousarray(y, dtype=np.int32)).to(self.dev)
+            weight = None if sample_weight is None else torch.from_numpy(
+                np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev)
+            return self._use_samples(samples, labels, n_classes, weight)
+
+    def _use_samples(self, samples, labels, n_classes: int, weight) -> dict:
+        self.samples = samples
+        self.ld16 = _round_up(self.ldx, 64)
+        self.n_classes, self.labels = int(n_classes), labels
+        self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
+        self._set_weights(weight)
+        self.idx = self.torch.empty((self.N, samples.winner_cols), dtype=self.torch.int32, device=self.dev)
+        return self._column_statistics()
 
     def free_device_bytes(self) -> int:
         """Device bytes a fit may still allocate: free memory plus what torch has cached but not handed out, less
@@ -330,30 +422,20 @@ class DeviceEngine:
 
     def _column_statistics(self) -> dict:
         torch = self.torch
-        # K4: moments about a common data row (rank 0's first row)
-        if self.streaming:
-            shift_row = torch.zeros(self.ldx, dtype=torch.float32, device=self.dev)
-            shift_row[: self.D] = torch.from_numpy(np.asarray(self._host_X[0], dtype=np.float32)).to(self.dev)
-        else:
-            shift_row = self.X[0].clone()
+        # K4: moments about a common data row (rank 0's first row, as float32)
+        shift_row = self.samples.shift_row()
         self.comm.broadcast_(shift_row, 0)
-        # the row-block parts are added on the host in a fixed order: the same statistics on every run
-        if not self.streaming:
-            p = self._colstats_parts(self.X, self.N, shift_row, self.weight)
+        # the row-block parts of a chunk are added on the host, then the chunk sums in chunk order: the same
+        # statistics on every run
+        acc = []
+
+        def body(c, c0, c1, x):
+            p = self._colstats_parts(x, c1 - c0, shift_row, self.weight[c0:c1] if self.weight is not None else None)
             sums, maxabs = p[:, : 2 * self.ldx].sum(axis=0), p[:, 2 * self.ldx].max()
-        else:
-            # streamed: each chunk's parts are added, then the chunk sums in chunk order
-            acc = {"sums": np.zeros(2 * self.ldx), "max": 0.0}
+            acc[:] = [sums, maxabs] if c == 0 else [acc[0] + sums, max(acc[1], maxabs)]
 
-            def body(c, c0, c1, x):
-                w = self.weight[c0:c1] if self.weight is not None else None
-                p = self._colstats_parts(x, c1 - c0, shift_row, w)
-                acc["sums"] = acc["sums"] + p[:, : 2 * self.ldx].sum(axis=0)
-                acc["max"] = max(acc["max"], float(p[:, 2 * self.ldx].max()))
-
-            self._stream_pass(body)
-            sums, maxabs = acc["sums"], acc["max"]
-        moments = torch.from_numpy(np.append(sums, maxabs)).to(self.dev)
+        self.samples.chunk_pass(body)
+        moments = torch.from_numpy(np.append(*acc)).to(self.dev)
         self.comm.allreduce_(moments[: 2 * self.ldx])
         self.comm.allreduce_(moments[2 * self.ldx :], "max")
         m = moments.cpu().numpy()
@@ -384,8 +466,6 @@ class DeviceEngine:
         self.scale = 1.0 if not (maxabs > 0 and math.isfinite(maxabs)) else 2.0 ** math.floor(
             math.log2(2.0**12 / (2.0 * maxabs))
         )
-        self.X16_hi = self.X16_lo = self.xnorm16 = None
-        self.ld16 = _round_up(self.ldx, 64)
         return stats
 
     def load_device_data(self, X_dev, labels_dev=None, n_classes: int = 0, weight_dev=None) -> dict:
@@ -395,122 +475,23 @@ class DeviceEngine:
             raise ValueError("X_dev must be a contiguous float32 [N, D] CUDA tensor with D % 4 == 0")
         with torch.cuda.device(self.dev):
             self.N, self.D = int(X_dev.shape[0]), int(X_dev.shape[1])
-            self.X, self.ldx = X_dev, int(X_dev.shape[1])
-            self.n_classes, self.labels = int(n_classes), labels_dev
-            self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
-            self._set_weights(weight_dev)
-            return self._column_statistics()
+            self.ldx = self.D
+            return self._use_samples(ResidentSamples(self, X_dev), labels_dev, n_classes, weight_dev)
 
-    # ------------------------------------------------------------------ streamed data
-    def _load_streamed(self, X, y, n_classes: int, sample_weight, rows: int) -> dict:
-        """`load_data` for a streamed fit: only per-sample vectors go to the device (labels, weights; the winners and
-        the chunk-local sort permutation are allocated here), the rows stay in the caller's array."""
-        torch = self.torch
-        if X.dtype not in (np.float32, np.float64):
-            raise ValueError("streamed samples must be float32 or float64")
-        self.streaming = True
-        self._host_X = X
-        self.ldx = _round_up(self.D, 4)
-        self.ld16 = _round_up(self.ldx, 64)
-        self.chunk_rows = int(min(rows, _round_up(max(self.N, 1), streaming.ROW_GRANULE)))
-        self.chunks = streaming.chunk_bounds(self.N, self.chunk_rows)
-        self.n_classes = int(n_classes)
-        self.labels = None
-        if y is not None:
-            self.labels = torch.from_numpy(np.ascontiguousarray(y, dtype=np.int32)).to(self.dev)
-        self.sample_offset, self.n_samples_global = self.comm.exclusive_offset(self.N, self.dev)
-        self._set_weights(None if sample_weight is None else torch.from_numpy(
-            np.ascontiguousarray(sample_weight, dtype=np.float64)).to(self.dev))
-        # two float32 chunk slots (one is filled while the other is computed on); every other chunk buffer is single,
-        # because all compute runs on one stream
-        self._slots = [torch.empty((self.chunk_rows, self.ldx), dtype=torch.float32, device=self.dev) for _ in range(2)]
-        self._slot_ready = [torch.cuda.Event() for _ in range(2)]
-        self._slot_free = [torch.cuda.Event() for _ in range(2)]
-        self.row_perm = torch.empty(self.N, dtype=torch.int32, device=self.dev)  # chunk-local K2 order per chunk
-        self._chunks_sorted = False  # row_perm holds every chunk's K2 order (after the first epoch)
-        self._sorted_search = False  # some chunk's search read its samples sorted (the post passes then do too)
-        self._cx16 = None
-        self._copy_stream = torch.cuda.Stream(self.dev)
-        self._stager = streaming.HostStager(torch, streaming.HostStager.piece_rows_for(self.chunk_rows, self.ldx),
-                                            self.D, self.ldx)
-        return self._column_statistics()
-
-    def _stream_pass(self, body) -> None:
-        """One pass over the samples in chunks: body(c, c0, c1, x) enqueues the work on chunk c, whose float32 rows
-        x [c1 - c0, ldx] are in a device slot.  The rows of chunk c + 1 are staged by the host threads and copied on
-        a side stream into the other slot while chunk c is computed; a slot is overwritten only after the work on
-        the chunk before has been enqueued and has run (event `_slot_free`)."""
-        torch = self.torch
-        main = torch.cuda.current_stream(self.dev)
-        copy = self._copy_stream
-        copy.wait_stream(main)  # earlier readers of the slots are done before they are overwritten
-        with self._stager.pieces(self._host_X, self.chunks) as pieces:
-            pieces = iter(pieces)
-
-            def upload(c):
-                s, (c0, c1) = c % 2, self.chunks[c]
-                if c >= 2:
-                    copy.wait_event(self._slot_free[s])
-                done = c0
-                with torch.cuda.stream(copy):
-                    while done < c1:
-                        _, r0, r1, host, release = next(pieces)
-                        self._slots[s][r0 - c0 : r1 - c0].copy_(host, non_blocking=True)
-                        ev = torch.cuda.Event()
-                        ev.record(copy)
-                        release(ev)
-                        done = r1
-                    self._slot_ready[s].record(copy)
-
-            upload(0)
-            for c, (c0, c1) in enumerate(self.chunks):
-                s = c % 2
-                main.wait_event(self._slot_ready[s])
-                body(c, c0, c1, self._slots[s][: c1 - c0])
-                self._slot_free[s].record(main)
-                if c + 1 < len(self.chunks):
-                    upload(c + 1)
-
-    def _chunk_x16(self, x, n: int, need_lo: bool, perm=None):
-        """fp16 shadows of one chunk's rows (in the order `perm`, chunk-local, when given)."""
-        torch = self.torch
-        if self._cx16 is None or (need_lo and self._cx16[1] is None):
-            self._cx16 = (torch.empty((self.chunk_rows, self.ld16), dtype=torch.float16, device=self.dev),
-                          torch.empty((self.chunk_rows, self.ld16), dtype=torch.float16, device=self.dev) if need_lo else None,
-                          torch.empty(self.chunk_rows, dtype=torch.float32, device=self.dev))
-        hi, lo, xn = self._cx16
-        lo_ptr = lo.data_ptr() if need_lo else None
-        with self._Phase(self, "prepare_x16"):
-            if perm is None:
-                nat.check(self.lib.dbgsom_prepare_x16(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(), self.scale,
-                                                      hi.data_ptr(), lo_ptr, self.ld16, xn.data_ptr(), self._stream()),
-                          "dbgsom_prepare_x16")
-                self.launches += 1
-            else:
-                nat.check(self.lib.dbgsom_prepare_x16_sorted(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(),
-                                                             self.scale, perm.data_ptr(), hi.data_ptr(), lo_ptr, self.ld16,
-                                                             xn.data_ptr(), self._stream()),
-                          "dbgsom_prepare_x16_sorted")
-                self.launches += 2
-        return hi[:n], (lo[:n] if need_lo else None), xn[:n]
-
-    def _ensure_x16(self, need_lo: bool) -> None:
-        torch = self.torch
-        if self.X16_hi is not None and (self.X16_lo is not None or not need_lo):
-            return
-        self.row_perm = None  # (re)built in natural sample order
-        self.X16_hi = torch.empty((self.N, self.ld16), dtype=torch.float16, device=self.dev)
-        self.X16_lo = torch.empty((self.N, self.ld16), dtype=torch.float16, device=self.dev) if need_lo else None
-        self.xnorm16 = torch.empty(self.N, dtype=torch.float32, device=self.dev)
-        nat.check(
-            self.lib.dbgsom_prepare_x16(
-                self.X.data_ptr(), self.N, self.ldx, self.ldx, self.shift.data_ptr(), self.scale,
-                self.X16_hi.data_ptr(), self.X16_lo.data_ptr() if need_lo else None, self.ld16,
-                self.xnorm16.data_ptr(), self._stream(),
-            ),
-            "dbgsom_prepare_x16",
-        )
-        self.launches += 1
+    def _prepare_x16(self, x, n: int, hi, lo, xnorm, perm=None) -> None:
+        """fp16 shadows hi (and lo, when given) and xnorm of n rows of x, in the order `perm` when given."""
+        lo_ptr = lo.data_ptr() if lo is not None else None
+        if perm is None:
+            nat.check(self.lib.dbgsom_prepare_x16(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(), self.scale,
+                                                  hi.data_ptr(), lo_ptr, self.ld16, xnorm.data_ptr(), self._stream()),
+                      "dbgsom_prepare_x16")
+            self.launches += 1
+        else:
+            nat.check(self.lib.dbgsom_prepare_x16_sorted(x.data_ptr(), n, self.ldx, self.ldx, self.shift.data_ptr(),
+                                                         self.scale, perm.data_ptr(), hi.data_ptr(), lo_ptr, self.ld16,
+                                                         xnorm.data_ptr(), self._stream()),
+                      "dbgsom_prepare_x16_sorted")
+            self.launches += 2
 
     # ------------------------------------------------------------------ map state
     def _alloc_map(self, capacity: int) -> None:
@@ -526,15 +507,13 @@ class DeviceEngine:
         self.wmax = torch.zeros(4, dtype=torch.float32, device=self.dev)  # see dbgsom_prepare_w
         self.part = torch.zeros(cap * self.ldx + 3 * cap, dtype=torch.float64, device=self.dev)
         self.change = torch.zeros(1, dtype=torch.float64, device=self.dev)
-        # the epoch's winners (streamed fits keep only the int32 winner of every sample resident)
-        self.idx = torch.empty((self.N, 1 if self.streaming else 2), dtype=torch.int32, device=self.dev)
         self.bmu_stats = torch.zeros(8, dtype=torch.int64, device=self.dev)
         # weighted fits sum the class histogram as float64 weights
         hist_dtype = torch.int32 if self.weight is None else torch.float64
         self.class_hist = (
             torch.zeros((cap, self.n_classes), dtype=hist_dtype, device=self.dev) if self.labels is not None else None
         )
-        if self.streaming:
+        if self.samples is not None and len(self.samples.chunks) > 1:
             # one chunk's K2 sums and class histogram, added into the epoch's in chunk order
             self._cpart = torch.empty_like(self.part)
             self._chist = torch.empty_like(self.class_hist) if self.class_hist is not None else None
@@ -557,22 +536,8 @@ class DeviceEngine:
             local = rows - self.sample_offset
             owned = (local >= 0) & (local < self.N)
             W0 = self.W[0]
-            if owned.any() and self.streaming:
-                # the rows the device gather would read, rounded through float32 like the device copy of X
-                tmp = np.zeros((len(rows), self.ldx), dtype=np.float64)
-                tmp[:, : self.D] = np.asarray(self._host_X[np.where(owned, local, 0)]).astype(np.float32)
-                tmp[~owned] = 0
-                W0[: len(rows)] = torch.from_numpy(tmp).to(self.dev)
-            elif owned.any():
-                src = torch.from_numpy(np.where(owned, local, 0)).to(self.dev)
-                tmp = torch.zeros((len(rows), self.ldx), dtype=torch.float64, device=self.dev)
-                nat.check(
-                    self.lib.dbgsom_gather_rows(
-                        self.X.data_ptr(), self.ldx, self.ldx, src.data_ptr(), len(rows), tmp.data_ptr(), self._stream()
-                    ),
-                    "dbgsom_gather_rows",
-                )
-                self.launches += 1
+            if owned.any():
+                tmp = self.samples.start_rows(np.where(owned, local, 0))
                 tmp[torch.from_numpy(~owned).to(self.dev)] = 0
                 W0[: len(rows)] = tmp
             else:
@@ -786,13 +751,18 @@ class DeviceEngine:
     def _run_bmu(self, X, n: int, ldx: int, x16, W, m: int, n_bmu: int, want_dist: bool, idx, dist, backend=None,
                  strict=None, row_perm=None, selective=False):
         """prepare_w + candidate search + exact re-score for samples X against prototypes W."""
-        be, n_pass = self._pick_backend(n, m) if backend is None else backend
+        backend = self._pick_backend(n, m) if backend is None else backend
+        mpad = self._prepare_search(W, m, backend, n_bmu, map_order=selective)
+        self._bmu_search(X, n, ldx, x16, W, m, mpad, n_bmu, want_dist, idx, dist, backend, strict=strict,
+                         row_perm=row_perm, selective=selective)
+
+    def _prepare_search(self, W, m: int, backend, n_bmu: int, map_order: bool = False) -> int:
+        """prepare_w for searches of `backend` against the first m rows of W; returns mpad."""
         if W.shape[0] > self.W32.shape[0]:
             self.W32 = self.torch.zeros((W.shape[0], self.ldx), dtype=self.torch.float32, device=self.dev)
         with self._Phase(self, "prepare_w"):
-            mpad = self._prepare_w(W, m, be == nat.BMU_TENSOR, n_pass == 3, top1=n_bmu == 1, map_order=selective)
-        self._bmu_search(X, n, ldx, x16, W, m, mpad, n_bmu, want_dist, idx, dist, (be, n_pass), strict=strict,
-                         row_perm=row_perm, selective=selective)
+            return self._prepare_w(W, m, backend[0] == nat.BMU_TENSOR, backend[1] == 3, top1=n_bmu == 1,
+                                   map_order=map_order)
 
     def _select_eligible(self, n: int, m: int, backend) -> bool:
         """The selective search applies: tensor search with three passes, one winner, shapes the kernels cover, and a
@@ -872,102 +842,90 @@ class DeviceEngine:
                         chunk_rows: int = 1 << 20) -> dict:
         """One epoch whose samples arrive from (pinned) host memory: row chunks are copied on a side
         stream while the previous chunk's fp16 shadow and BMU search run, so only the update pass waits
-        for the whole upload.  `host_X` is a float32 torch tensor [N, ldx] with the layout of `self.X`."""
+        for the whole upload.  `host_X` is a float32 torch tensor [N, ldx] with the layout of the resident X."""
         torch = self.torch
         with torch.cuda.device(self.dev):
-            if tuple(host_X.shape) != tuple(self.X.shape) or host_X.dtype != torch.float32:
+            S = self.samples
+            X = S.X
+            if tuple(host_X.shape) != tuple(X.shape) or host_X.dtype != torch.float32:
                 raise ValueError("host_X must match the resident sample matrix (float32, same shape)")
             m, cur = self.M, self.W[self.cur]
             be = self._pick_backend(self.N, m)
             tensor = be[0] == nat.BMU_TENSOR
             need_lo = be[1] == 3
-            self.row_perm = None  # the shadows are rebuilt chunk by chunk in natural sample order
-            if tensor and (self.X16_hi is None or (need_lo and self.X16_lo is None)):
-                self.X16_hi = torch.empty((self.N, self.ld16), dtype=torch.float16, device=self.dev)
-                self.X16_lo = torch.empty((self.N, self.ld16), dtype=torch.float16, device=self.dev) if need_lo else None
-                self.xnorm16 = torch.empty(self.N, dtype=torch.float32, device=self.dev)
+            S.row_perm = None  # the shadows are rebuilt chunk by chunk in natural sample order
+            if tensor:
+                S.reserve_shadows(need_lo)
             main = torch.cuda.current_stream(self.dev)
-            if getattr(self, "_copy_stream", None) is None:
+            if self._copy_stream is None:
                 self._copy_stream = torch.cuda.Stream(self.dev)
             self._copy_stream.wait_stream(main)  # earlier readers of X are done before it is overwritten
-            with self._Phase(self, "prepare_w"):
-                mpad = self._prepare_w(cur, m, tensor, need_lo)
+            mpad = self._prepare_search(cur, m, be, 1)
             idx = self.idx.view(-1)[: self.N]
             for c0 in range(0, self.N, chunk_rows):
                 c1 = min(self.N, c0 + chunk_rows)
                 with torch.cuda.stream(self._copy_stream):
-                    self.X[c0:c1].copy_(host_X[c0:c1], non_blocking=True)
+                    X[c0:c1].copy_(host_X[c0:c1], non_blocking=True)
                     ready = torch.cuda.Event()
                     ready.record(self._copy_stream)
                 main.wait_event(ready)
                 x16 = None
                 if tensor:
-                    xh, xl, xn = self.X16_hi[c0:c1], (self.X16_lo[c0:c1] if need_lo else None), self.xnorm16[c0:c1]
-                    nat.check(
-                        self.lib.dbgsom_prepare_x16(
-                            self.X[c0:c1].data_ptr(), c1 - c0, self.ldx, self.ldx, self.shift.data_ptr(), self.scale,
-                            xh.data_ptr(), xl.data_ptr() if need_lo else None, self.ld16, xn.data_ptr(), self._stream(),
-                        ),
-                        "dbgsom_prepare_x16",
-                    )
-                    self.launches += 1
-                    x16 = (xh, xl, xn)
-                self._bmu_search(self.X[c0:c1], c1 - c0, self.ldx, x16, cur, m, mpad, 1, False, idx[c0:c1], None, be,
+                    x16 = (S.X16_hi[c0:c1], S.X16_lo[c0:c1] if need_lo else None, S.xnorm16[c0:c1])
+                    self._prepare_x16(X[c0:c1], c1 - c0, *x16)
+                self._bmu_search(X[c0:c1], c1 - c0, self.ldx, x16, cur, m, mpad, 1, False, idx[c0:c1], None, be,
                                  ws_key="bmu_chunk")
-            return self._update_and_smooth(be, idx, sigma, pack_rows, entropy_error)
+            part, hist = self._epoch_sums(entropy_error)
+            self._accumulate(0, 0, self.N, X, idx, part, hist)
+            return self._reduce_and_smooth(be, part, hist is not None, sigma, pack_rows, entropy_error)
 
     def epoch(self, sigma: float, pack_rows: bool, entropy_error: bool, _force_simt: bool = False) -> dict:
-        """One training epoch on the resident data; returns per-neuron error, counts, change."""
+        """One training epoch: per chunk of the samples, fp16 shadows, BMU search and K2; then the all-reduce, K3 and
+        the read-back.  Returns per-neuron error, counts, change."""
         torch = self.torch
         with torch.cuda.device(self.dev):
-            if self.streaming:
-                return self._epoch_streamed(sigma, pack_rows, entropy_error, _force_simt)
-            m, cur = self.M, self.W[self.cur]
+            S, m, cur = self.samples, self.M, self.W[self.cur]
+            # the backend follows the whole sample count: small chunks must not turn the tensor search into the SIMT one
             be = (nat.BMU_SIMT, 0) if _force_simt else self._pick_backend(self.N, m)
-            x16 = None
-            if be[0] == nat.BMU_TENSOR:
-                self._ensure_x16(be[1] == 3)
-                x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
+            eligible = [self._select_eligible(c1 - c0, m, be) for c0, c1 in S.chunks]
+            # the selective search needs the samples in sorted order, i.e. the winners of an earlier epoch
+            selective = [e and S.has_order(c) for c, e in enumerate(eligible)]
+            mpad = self._prepare_search(cur, m, be, 1, map_order=any(selective))
+            part, hist = self._epoch_sums(entropy_error)
             idx = self.idx.view(-1)[: self.N]
-            eligible = self._select_eligible(self.N, m, be)
-            # the selective search needs the sorted sample order, i.e. the winners of an earlier epoch
-            selective = eligible and self.row_perm is not None
-            self._run_bmu(self.X, self.N, self.ldx, x16, cur, m, 1, False, idx, None, backend=be,
-                          row_perm=self.row_perm if be[0] == nat.BMU_TENSOR else None, selective=selective)
-            return self._update_and_smooth(be, idx, sigma, pack_rows, entropy_error, resort=eligible)
 
-    def _resort_samples(self, idx, m: int, acc_ws) -> None:
-        """Rebuild the fp16 shadows in the order K2 has just grouped the samples in (by winner, ascending index): row
-        tiles of the tensor search then hold samples that compete for the same few prototypes.  One pass over X."""
-        torch = self.torch
-        off = int(self.lib.dbgsom_accumulate_perm_offset(self.N, m))
-        perm = acc_ws[off : off + 4 * self.N].view(torch.int32)
-        if self.row_perm is None:
-            self.row_perm = torch.empty(self.N, dtype=torch.int32, device=self.dev)
-        self.row_perm.copy_(perm)
-        nat.check(
-            self.lib.dbgsom_prepare_x16_sorted(
-                self.X.data_ptr(), self.N, self.ldx, self.ldx, self.shift.data_ptr(), self.scale, self.row_perm.data_ptr(),
-                self.X16_hi.data_ptr(), self.X16_lo.data_ptr() if self.X16_lo is not None else None, self.ld16,
-                self.xnorm16.data_ptr(), self._stream(),
-            ),
-            "dbgsom_prepare_x16_sorted",
-        )
-        self.launches += 2
-        self._sort_age = 0
+            def body(c, c0, c1, x):
+                x16, perm = S.shadows(c, x, be, selective[c])
+                self._bmu_search(x, c1 - c0, self.ldx, x16, cur, m, mpad, 1, False, idx[c0:c1], None, be,
+                                 row_perm=perm, selective=selective[c])
+                S.after_k2(c, self._accumulate(c, c0, c1, x, idx, part, hist), eligible[c])
 
-    def _accumulate(self, X, n: int, idx, part, labels, weight, hist):
-        """K2 over n rows of X with winners idx into `part` (and the class histogram `hist` when labels are given);
-        returns the workspace, which holds the samples' order grouped by winner."""
-        m, cur = self.M, self.W[self.cur]
+            S.chunk_pass(body)
+            return self._reduce_and_smooth(be, part, hist is not None, sigma, pack_rows, entropy_error)
+
+    def _epoch_sums(self, entropy_error: bool):
+        """The epoch's K2 sums `part` and class histogram (None unless the entropy error needs it)."""
+        m = self.M
+        use_hist = entropy_error and self.labels is not None
+        return self.part[: m * self.ldx + 3 * m], self.class_hist[:m] if use_hist else None
+
+    def _accumulate(self, c: int, c0: int, c1: int, x, idx, part, hist):
+        """K2 over chunk c (rows x of samples c0..c1, winners idx[c0:c1]).  Chunk 0 writes the epoch's `part` and class
+        histogram `hist` (None: no histogram), later chunks write the chunk buffers, which are then added.  Returns
+        the chunk's samples grouped by winner (chunk-local int32 [c1 - c0])."""
+        n, m, first = c1 - c0, self.M, c == 0
+        k_part = part if first else self._cpart[: part.numel()]
+        k_hist = hist if first or hist is None else self._chist[:m]
+        labels = self.labels[c0:c1] if hist is not None else None
+        weight = self.weight[c0:c1] if self.weight is not None else None
         acc = nat.AccumulateArgs()
-        acc.d_X, acc.N, acc.D, acc.ldx = X.data_ptr(), n, self.ldx, self.ldx
-        acc.d_bmu, acc.d_W, acc.M = idx.data_ptr(), cur.data_ptr(), m
+        acc.d_X, acc.N, acc.D, acc.ldx = x.data_ptr(), n, self.ldx, self.ldx
+        acc.d_bmu, acc.d_W, acc.M = idx[c0:c1].data_ptr(), self.W[self.cur].data_ptr(), m
         acc.inv_total_variance = 1.0 / self.total_variance if self.total_variance > 0 else float("inf")
-        acc.d_part = part.data_ptr()
+        acc.d_part = k_part.data_ptr()
         acc.d_labels = labels.data_ptr() if labels is not None else None
         acc.n_classes = self.n_classes if labels is not None else 0
-        acc.d_class_hist = hist.data_ptr() if labels is not None and weight is None else None
+        acc.d_class_hist = k_hist.data_ptr() if labels is not None and weight is None else None
         ws = self._workspace("acc", self.lib.dbgsom_accumulate_workspace_bytes(n, m, self.ldx))
         acc.d_workspace, acc.workspace_bytes = ws.data_ptr(), ws.numel()
         with self._Phase(self, "accumulate"):
@@ -976,72 +934,18 @@ class DeviceEngine:
             else:
                 nat.check(
                     self.lib.dbgsom_accumulate_weighted(
-                        acc, weight.data_ptr(), hist.data_ptr() if labels is not None else None, self._stream()
+                        acc, weight.data_ptr(), k_hist.data_ptr() if labels is not None else None, self._stream()
                     ),
                     "dbgsom_accumulate_weighted",
                 )
         self.launches += (10 if m <= 24576 else 8) + (1 if labels is not None else 0)  # stable scatter: 3 kernels
-        return ws
-
-    def _update_and_smooth(self, be, idx, sigma: float, pack_rows: bool, entropy_error: bool, resort: bool = False) -> dict:
-        """K2 -> all-reduce -> K3 -> read-back, given the winners of the current prototypes."""
-        m = self.M
-        # K2
-        part = self.part[: m * self.ldx + 3 * m]
-        use_hist = entropy_error and self.labels is not None
-        ws = self._accumulate(self.X, self.N, idx, part, self.labels if use_hist else None, self.weight,
-                              self.class_hist if use_hist else None)
-        if resort and self.X16_hi is not None:
-            self._sort_age += 1
-            if self.row_perm is None or self._sort_age >= self.resort_every:
-                with self._Phase(self, "resort"):
-                    self._resort_samples(idx, m, ws)
-        return self._reduce_and_smooth(be, part, use_hist, sigma, pack_rows, entropy_error)
-
-    def _epoch_streamed(self, sigma: float, pack_rows: bool, entropy_error: bool, force_simt: bool) -> dict:
-        """`epoch` on streamed samples: per chunk, fp16 shadows (in the order K2 left the chunk's samples in the
-        epoch before), BMU search and K2 into a chunk `part`, which is added into the epoch's in chunk order; then the
-        all-reduce, K3 and the read-back of the resident epoch."""
-        m, cur = self.M, self.W[self.cur]
-        # the backend follows the whole sample count: small chunks must not turn the tensor search into the SIMT one
-        be = (nat.BMU_SIMT, 0) if force_simt else self._pick_backend(self.N, m)
-        tensor, need_lo = be[0] == nat.BMU_TENSOR, be[1] == 3
-        sorted_ = self._chunks_sorted
-        selective = [sorted_ and self._select_eligible(c1 - c0, m, be) for c0, c1 in self.chunks]
-        with self._Phase(self, "prepare_w"):
-            mpad = self._prepare_w(cur, m, tensor, need_lo, top1=True, map_order=any(selective))
-        part = self.part[: m * self.ldx + 3 * m]
-        cpart = self._cpart[: part.numel()]
-        use_hist = entropy_error and self.labels is not None
-        hist = self.class_hist[:m] if use_hist else None
-        chist = self._chist[:m] if use_hist else None
-        idx = self.idx.view(-1)[: self.N]
-
-        def body(c, c0, c1, x):
-            n = c1 - c0
-            perm = self.row_perm[c0:c1]
-            # like the resident epoch, only the selective search reads the samples in sorted order
-            x16 = self._chunk_x16(x, n, need_lo, perm if selective[c] else None) if tensor else None
-            self._bmu_search(x, n, self.ldx, x16, cur, m, mpad, 1, False, idx[c0:c1], None, be,
-                             row_perm=perm if selective[c] else None, selective=selective[c])
-            first = c == 0
-            ws = self._accumulate(x, n, idx[c0:c1], part if first else cpart,
-                                  self.labels[c0:c1] if use_hist else None,
-                                  self.weight[c0:c1] if self.weight is not None else None,
-                                  (hist if first else chist) if use_hist else None)
-            if not first:
-                with self._Phase(self, "chunk_sum"):
-                    part.add_(cpart)
-                    if use_hist:
-                        hist.add_(chist)
-            # the chunk's samples grouped by winner: the shadow order of its next epoch
-            off = int(self.lib.dbgsom_accumulate_perm_offset(n, m))
-            perm.copy_(ws[off : off + 4 * n].view(self.torch.int32))
-
-        self._stream_pass(body)
-        self._chunks_sorted = True
-        self._sorted_search |= any(selective)
-        return self._reduce_and_smooth(be, part, use_hist, sigma, pack_rows, entropy_error)
+        if not first:
+            with self._Phase(self, "chunk_sum"):
+                part.add_(k_part)
+                if hist is not None:
+                    hist.add_(k_hist)
+        off = int(self.lib.dbgsom_accumulate_perm_offset(n, m))
+        return ws[off : off + 4 * n].view(self.torch.int32)
 
     def _reduce_and_smooth(self, be, part, use_hist: bool, sigma: float, pack_rows: bool, entropy_error: bool) -> dict:
         """All-reduce of the epoch sums -> K3 -> read-back."""
@@ -1129,78 +1033,40 @@ class DeviceEngine:
 
     def bmu_train(self, n_bmu: int, previous: bool = False):
         """BMUs of the training samples against the current (or pre-update) prototypes."""
-        torch = self.torch
-        with torch.cuda.device(self.dev):
+        with self.torch.cuda.device(self.dev):
             W = self.W[self.cur ^ 1] if previous else self.W[self.cur]
             m = self.n_previous_rows if previous else self.M
             n_bmu = min(n_bmu, m)
-            if self.streaming:
-                dist_h = np.empty((self.N, n_bmu), dtype=np.float64)
-                idx_h = np.empty((self.N, n_bmu), dtype=np.int64)
+            dist_h = np.empty((self.N, n_bmu), dtype=np.float64)
+            idx_h = np.empty((self.N, n_bmu), dtype=np.int64)
 
-                def out(c, c0, c1, idx, dist):
-                    dist_h[c0:c1], idx_h[c0:c1] = dist.cpu().numpy(), idx.cpu().numpy()
+            def out(c, c0, c1, idx, dist):
+                dist_h[c0:c1], idx_h[c0:c1] = dist.cpu().numpy(), idx.cpu().numpy()
 
-                self._bmu_pass_streamed(W, m, n_bmu, self.strict_ties, out)
-                return dist_h, idx_h
-            be = self._pick_backend(self.N, m)
-            x16 = None
-            if be[0] == nat.BMU_TENSOR:
-                self._ensure_x16(be[1] == 3)
-                x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
-            idx = torch.empty((self.N, n_bmu), dtype=torch.int32, device=self.dev)
-            dist = torch.empty((self.N, n_bmu), dtype=torch.float64, device=self.dev)
-            self._run_bmu(self.X, self.N, self.ldx, x16, W, m, n_bmu, True, idx, dist, backend=be,
-                          row_perm=self.row_perm if be[0] == nat.BMU_TENSOR else None)
-            return dist.cpu().numpy(), idx.cpu().numpy().astype(np.int64)
+            self._bmu_pass(W, m, n_bmu, self.strict_ties, out)
+            return dist_h, idx_h
 
-    def _bmu_pass_streamed(self, W, m: int, n_bmu: int, strict: bool, out) -> None:
-        """BMU search of the streamed samples against W (what `_run_bmu` does on resident ones): per chunk, the
-        chunk's winners idx int32 [n, n_bmu] and distances dist float64 [n, n_bmu] go to out(c, c0, c1, idx, dist),
-        which enqueues what reads them before the next chunk overwrites them."""
+    def _bmu_pass(self, W, m: int, n_bmu: int, strict: bool, out) -> None:
+        """BMU search of the training samples against W: per chunk, the chunk's winners idx int32 [n, n_bmu] and
+        distances dist float64 [n, n_bmu] go to out(c, c0, c1, idx, dist), which enqueues what reads them before the
+        next chunk overwrites them.  With one chunk they are the whole [N, n_bmu] results."""
         torch = self.torch
         be = self._pick_backend(self.N, m)
-        tensor, need_lo = be[0] == nat.BMU_TENSOR, be[1] == 3
-        if W.shape[0] > self.W32.shape[0]:
-            self.W32 = torch.zeros((W.shape[0], self.ldx), dtype=torch.float32, device=self.dev)
-        with self._Phase(self, "prepare_w"):
-            mpad = self._prepare_w(W, m, tensor, need_lo, top1=n_bmu == 1)
-        if getattr(self, "_cidx", None) is None or self._cidx.numel() < self.chunk_rows * n_bmu:
-            self._cidx = torch.empty(self.chunk_rows * max(n_bmu, 2), dtype=torch.int32, device=self.dev)
-            self._cdist = torch.empty(self.chunk_rows * max(n_bmu, 2), dtype=torch.float64, device=self.dev)
-        # sorted shadows where the resident fit has them: once the selective search has sorted the samples
-        sorted_ = self._chunks_sorted and self._sorted_search
+        mpad = self._prepare_search(W, m, be, n_bmu)
+        rows = max((c1 - c0 for c0, c1 in self.samples.chunks), default=0)
+        idx_buf = torch.empty((rows, n_bmu), dtype=torch.int32, device=self.dev)
+        dist_buf = torch.empty((rows, n_bmu), dtype=torch.float64, device=self.dev)
 
         def body(c, c0, c1, x):
             n = c1 - c0
-            perm = self.row_perm[c0:c1] if (tensor and sorted_) else None
-            x16 = self._chunk_x16(x, n, need_lo, perm) if tensor else None
-            idx = self._cidx[: n * n_bmu].view(n, n_bmu)
-            dist = self._cdist[: n * n_bmu].view(n, n_bmu)
+            x16, perm = self.samples.shadows(c, x, be, None)
+            idx, dist = idx_buf[:n], dist_buf[:n]
             self._bmu_search(x, n, self.ldx, x16, W, m, mpad, n_bmu, True, idx, dist, be, strict=strict, row_perm=perm)
             out(c, c0, c1, idx, dist)
 
-        self._stream_pass(body)
+        self.samples.chunk_pass(body)
 
     # ------------------------------------------------------------------ post-training passes
-    def _bmu_train_device(self, n_bmu: int, previous: bool):
-        """Like `bmu_train`, results stay in HBM: (idx int32 [N, n_bmu], dist float64 [N, n_bmu], m)."""
-        torch = self.torch
-        W = self.W[self.cur ^ 1] if previous else self.W[self.cur]
-        m = self.n_previous_rows if previous else self.M
-        n_bmu = min(n_bmu, m)
-        be = self._pick_backend(self.N, m)
-        x16 = None
-        if be[0] == nat.BMU_TENSOR:
-            self._ensure_x16(be[1] == 3)
-            x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
-        idx = torch.empty((self.N, n_bmu), dtype=torch.int32, device=self.dev)
-        dist = torch.empty((self.N, n_bmu), dtype=torch.float64, device=self.dev)
-        # the post-training passes run once per fit: flagged samples are always re-scored against all prototypes
-        self._run_bmu(self.X, self.N, self.ldx, x16, W, m, n_bmu, True, idx, dist, backend=be, strict=True,
-                      row_perm=self.row_perm if be[0] == nat.BMU_TENSOR else None)
-        return idx, dist, m
-
     def final_statistics(self, positions: np.ndarray, degrees: np.ndarray) -> dict:
         """Everything `fit` measures after the loop, reduced on the device (and over ranks):
         one top-2 BMU search on the PRE-update prototypes (dbgsom/BaseSom.py:116-119 see the
@@ -1208,12 +1074,8 @@ class DeviceEngine:
         and the node statistics (:181-211); the u-matrix (:320-337) uses the updated prototypes."""
         torch = self.torch
         with torch.cuda.device(self.dev):
-            if self.streaming:
-                m = self.n_previous_rows  # the chunks are searched below, once the bandwidth is known
-                n_bmu = min(2, m)
-            else:
-                idx, dist, m = self._bmu_train_device(2, previous=True)
-                n_bmu = int(idx.shape[1])
+            m = self.n_previous_rows  # the samples are searched below, once the bandwidth is known
+            n_bmu = min(2, m)
             M, cur = self.M, self.W[self.cur]
             total = float(np.sum(degrees))
             if total > 0:
@@ -1231,20 +1093,16 @@ class DeviceEngine:
             pos = torch.from_numpy(np.ascontiguousarray(positions[:m], dtype=np.int32)).to(self.dev)
             out = torch.empty(2 + 2 * m, dtype=torch.float64, device=self.dev)
             ok = bandwidth > 0 and math.isfinite(bandwidth)
-            if self.streaming:
-                # per chunk into `cout`, added into `out` in chunk order
-                cout = torch.empty_like(out)
 
-                def stats(c, c0, c1, idx, dist):
-                    w = self.weight[c0:c1] if self.weight is not None else None
-                    self._node_stats(idx, dist, n_bmu, c1 - c0, pos, m, bandwidth if ok else 1.0, w,
-                                     out if c == 0 else cout)
-                    if c > 0:
-                        out.add_(cout)
+            def stats(c, c0, c1, idx, dist):
+                # chunk 0 writes `out`, later chunks a chunk buffer that is added into it
+                k_out = out if c == 0 else torch.empty_like(out)
+                w = self.weight[c0:c1] if self.weight is not None else None
+                self._node_stats(idx, dist, n_bmu, c1 - c0, pos, m, bandwidth if ok else 1.0, w, k_out)
+                if c:
+                    out.add_(k_out)
 
-                self._bmu_pass_streamed(self.W[self.cur ^ 1], m, n_bmu, True, stats)
-            else:
-                self._node_stats(idx, dist, n_bmu, self.N, pos, m, bandwidth if ok else 1.0, self.weight, out)
+            self._bmu_pass(self.W[self.cur ^ 1], m, n_bmu, True, stats)
             self.comm.allreduce_(out)
             o = out.cpu().numpy()
             dens = o[2 + m :].copy()
@@ -1275,15 +1133,17 @@ class DeviceEngine:
     def final_winners(self) -> None:
         """Top-1 BMU of the training samples on the current (reduced) map; stays on the device."""
         with self.torch.cuda.device(self.dev):
-            if self.streaming:
-                self._final_idx = self.torch.empty((self.N, 1), dtype=self.torch.int32, device=self.dev)
+            # one chunk: the pass's own [N, 1] winners are kept
+            chunked = len(self.samples.chunks) > 1
+            self._final_idx = self.torch.empty((self.N, 1), dtype=self.torch.int32, device=self.dev) if chunked else None
 
-                def keep(c, c0, c1, idx, dist):
+            def keep(c, c0, c1, idx, dist):
+                if chunked:
                     self._final_idx[c0:c1].copy_(idx)
+                else:
+                    self._final_idx = idx
 
-                self._bmu_pass_streamed(self.W[self.cur], self.M, 1, True, keep)
-                return
-            self._final_idx, _, _ = self._bmu_train_device(1, previous=False)
+            self._bmu_pass(self.W[self.cur], self.M, 1, True, keep)
 
     def winners_host(self) -> np.ndarray:
         return self._final_idx[:, 0].cpu().numpy().astype(np.int64)
@@ -1291,77 +1151,42 @@ class DeviceEngine:
     def label_histogram(self, n_classes: int):
         """Class counts [M, C] and first global sample index [M, C] of every (winner, class) cell of the
         last `final_winners` search, reduced over ranks (dbgsom/SomClassifier.py:130-152).  Weighted fits: the
-        counts are weight sums and `first` ignores zero-weight samples."""
+        counts are weight sums and `first` ignores zero-weight samples.  Per chunk of the samples: counts added in
+        chunk order, `first` the minimum over the chunks."""
         torch = self.torch
         with torch.cuda.device(self.dev):
-            m = self.M
-            if self.streaming:
-                return self._label_histogram_chunked(n_classes)
-            if self.weight is not None:
-                counts = torch.empty((m, n_classes), dtype=torch.float64, device=self.dev)
-                first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
-                ws = self._workspace("labels", self.lib.dbgsom_label_hist_weighted_workspace_bytes(self.N, m))
-                nat.check(
-                    self.lib.dbgsom_label_hist_weighted(
-                        self._final_idx.data_ptr(), self.labels.data_ptr(), self.weight.data_ptr(), self.N,
-                        self.sample_offset, m, n_classes, counts.data_ptr(), first.data_ptr(), ws.data_ptr(),
-                        ws.numel(), self._stream(),
-                    ),
-                    "dbgsom_label_hist_weighted",
-                )
-                self.comm.allreduce_(counts)
-                self.comm.allreduce_(first, "min")
-                return counts.cpu().numpy(), first.cpu().numpy()
-            counts = torch.empty((m, n_classes), dtype=torch.int32, device=self.dev)
-            first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
-            nat.check(
-                self.lib.dbgsom_label_hist(
-                    self._final_idx.data_ptr(), int(self._final_idx.shape[1]), self.labels.data_ptr(), self.N,
-                    self.sample_offset, m, n_classes, counts.data_ptr(), first.data_ptr(), self._stream(),
-                ),
-                "dbgsom_label_hist",
-            )
-            self.launches += 3
-            counts = counts.to(torch.int64)
-            self.comm.allreduce_(counts)
+            m, weighted = self.M, self.weight is not None
+            for c, (c0, c1) in enumerate(self.samples.chunks):
+                n, idx = c1 - c0, self._final_idx[c0:c1]
+                counts = torch.empty((m, n_classes), dtype=torch.float64 if weighted else torch.int32, device=self.dev)
+                k_first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
+                if weighted:
+                    ws = self._workspace("labels", self.lib.dbgsom_label_hist_weighted_workspace_bytes(n, m))
+                    nat.check(
+                        self.lib.dbgsom_label_hist_weighted(
+                            idx.data_ptr(), self.labels[c0:c1].data_ptr(), self.weight[c0:c1].data_ptr(), n,
+                            self.sample_offset + c0, m, n_classes, counts.data_ptr(), k_first.data_ptr(),
+                            ws.data_ptr(), ws.numel(), self._stream(),
+                        ),
+                        "dbgsom_label_hist_weighted",
+                    )
+                else:
+                    nat.check(
+                        self.lib.dbgsom_label_hist(
+                            idx.data_ptr(), int(idx.shape[1]), self.labels[c0:c1].data_ptr(), n, self.sample_offset + c0,
+                            m, n_classes, counts.data_ptr(), k_first.data_ptr(), self._stream(),
+                        ),
+                        "dbgsom_label_hist",
+                    )
+                self.launches += 3
+                if c == 0:  # int32 counts are summed as int64
+                    total, first = counts.to(torch.float64 if weighted else torch.int64), k_first
+                else:
+                    total.add_(counts)
+                    torch.minimum(first, k_first, out=first)
+            self.comm.allreduce_(total)
             self.comm.allreduce_(first, "min")
-            return counts.cpu().numpy().astype(np.float64), first.cpu().numpy()
-
-    def _label_histogram_chunked(self, n_classes: int):
-        """`label_histogram` of a streamed fit: the same kernels per chunk (global sample offset + c0), counts added
-        in chunk order, `first` the minimum over the chunks."""
-        torch = self.torch
-        m, weighted = self.M, self.weight is not None
-        counts = torch.zeros((m, n_classes), dtype=torch.float64 if weighted else torch.int64, device=self.dev)
-        first = torch.full((m, n_classes), np.iinfo(np.int64).max, dtype=torch.int64, device=self.dev)
-        c_counts = torch.empty((m, n_classes), dtype=torch.float64 if weighted else torch.int32, device=self.dev)
-        c_first = torch.empty((m, n_classes), dtype=torch.int64, device=self.dev)
-        for c0, c1 in self.chunks:
-            n, idx = c1 - c0, self._final_idx[c0:c1]
-            if weighted:
-                ws = self._workspace("labels", self.lib.dbgsom_label_hist_weighted_workspace_bytes(n, m))
-                nat.check(
-                    self.lib.dbgsom_label_hist_weighted(
-                        idx.data_ptr(), self.labels[c0:c1].data_ptr(), self.weight[c0:c1].data_ptr(), n,
-                        self.sample_offset + c0, m, n_classes, c_counts.data_ptr(), c_first.data_ptr(), ws.data_ptr(),
-                        ws.numel(), self._stream(),
-                    ),
-                    "dbgsom_label_hist_weighted",
-                )
-            else:
-                nat.check(
-                    self.lib.dbgsom_label_hist(
-                        idx.data_ptr(), 1, self.labels[c0:c1].data_ptr(), n, self.sample_offset + c0, m, n_classes,
-                        c_counts.data_ptr(), c_first.data_ptr(), self._stream(),
-                    ),
-                    "dbgsom_label_hist",
-                )
-            self.launches += 3
-            counts.add_(c_counts)
-            torch.minimum(first, c_first, out=first)
-        self.comm.allreduce_(counts)
-        self.comm.allreduce_(first, "min")
-        return counts.cpu().numpy().astype(np.float64), first.cpu().numpy()
+            return total.cpu().numpy().astype(np.float64), first.cpu().numpy()
 
     def bmu(self, X: np.ndarray, W: np.ndarray, n_bmu: int):
         """Stand-alone BMU search (predict path): host samples against host prototypes.
@@ -1379,7 +1204,6 @@ class DeviceEngine:
             self.ldx = _round_up(d, 4)
             self.ld16 = _round_up(self.ldx, 64)
             self.labels, self.n_classes = None, 0
-            self.row_perm = None
             self.W = None
             self._alloc_map(W.shape[0])
             self.cur = 0
@@ -1405,15 +1229,11 @@ class DeviceEngine:
             idx_h = np.empty((n, n_bmu), dtype=np.int64)
             for c0, c1 in chunks:
                 self.N = c1 - c0
-                self.X = self._upload_matrix(np.asarray(X[c0:c1]))
-                x16 = None
-                if tensor:
-                    self.X16_hi = None
-                    self._ensure_x16(be[1] == 3)
-                    x16 = (self.X16_hi, self.X16_lo, self.xnorm16)
+                x = self._upload_matrix(np.asarray(X[c0:c1]))
+                x16, _ = ResidentSamples(self, x).shadows(0, x, be, None)
                 idx = torch.empty((self.N, n_bmu), dtype=torch.int32, device=self.dev)
                 dist = torch.empty((self.N, n_bmu), dtype=torch.float64, device=self.dev)
-                self._run_bmu(self.X, self.N, self.ldx, x16, self.W[0], self.M, n_bmu, True, idx, dist, backend=be)
+                self._run_bmu(x, self.N, self.ldx, x16, self.W[0], self.M, n_bmu, True, idx, dist, backend=be)
                 dist_h[c0:c1], idx_h[c0:c1] = dist.cpu().numpy(), idx.cpu().numpy()
             return dist_h, idx_h
 

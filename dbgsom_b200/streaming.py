@@ -3,8 +3,9 @@
 When the resident fit (every sample, its fp16 shadows and the per-sample buffers of the search, K2 and the
 post-training passes in HBM) would not fit in free device memory, `DeviceEngine` keeps only per-sample vectors on
 the device and streams the rows from the user's host array in chunks, every epoch.  `plan_stream` decides which of
-the two a fit takes and how large the chunks are; `HostStager` moves the rows through a fixed ring of page-locked
-buffers.  DESIGN.md, "Streaming fits", describes the pipeline.
+the two a fit takes and how large the chunks are; `StreamedSamples` is the engine's source of such samples, and
+`HostStager` moves the rows through a fixed ring of page-locked buffers.  DESIGN.md, "Streaming fits", describes the
+pipeline.
 """
 
 from __future__ import annotations
@@ -18,6 +19,8 @@ from concurrent.futures import ThreadPoolExecutor
 from typing import Callable
 
 import numpy as np
+
+from . import _native as nat
 
 ROW_GRANULE = 256                 # chunk row counts are multiples of this
 MAX_CHUNK_BYTES = 512 << 20       # float32 rows of one planned chunk (the first chunk's copy is not hidden)
@@ -202,3 +205,116 @@ class HostStager:
             for f in pending:
                 f.cancel()
             pool.shutdown(wait=True)
+
+
+class StreamedSamples:
+    """Samples that stay in the caller's host array (float32 or float64) and pass through the device in chunks of
+    `chunk_rows` rows every epoch; the operations of engine.ResidentSamples.  On the device: two float32 chunk slots,
+    the fp16 shadows of one chunk, rebuilt for every chunk of every pass, and `row_perm`, the chunk-local order K2
+    left each chunk's samples in.  Other chunk buffers are single, because all compute runs on one stream."""
+
+    streaming = True
+    winner_cols = 1  # only the int32 winner of every sample stays resident
+
+    def __init__(self, eng, X, rows: int):
+        if X.dtype not in (np.float32, np.float64):
+            raise ValueError("streamed samples must be float32 or float64")
+        torch = eng.torch
+        self.eng, self.host_X = eng, X
+        n = int(X.shape[0])
+        self.chunk_rows = int(min(rows, _round_up(max(n, 1), ROW_GRANULE)))
+        self.chunks = chunk_bounds(n, self.chunk_rows)
+        self.slots = [torch.empty((self.chunk_rows, eng.ldx), dtype=torch.float32, device=eng.dev) for _ in range(2)]
+        self.slot_ready = [torch.cuda.Event() for _ in range(2)]
+        self.slot_free = [torch.cuda.Event() for _ in range(2)]
+        self.row_perm = torch.empty(n, dtype=torch.int32, device=eng.dev)
+        self._chunks_sorted = False  # row_perm holds every chunk's K2 order (after the first epoch)
+        self._sorted_search = False  # some chunk's search read its samples sorted (the post passes then do too)
+        self._x16 = None
+        self.copy_stream = torch.cuda.Stream(eng.dev)
+        self.stager = HostStager(torch, HostStager.piece_rows_for(self.chunk_rows, eng.ldx), eng.D, eng.ldx)
+
+    def chunk_pass(self, body) -> None:
+        """One pass over the samples in chunks: body(c, c0, c1, x) enqueues the work on chunk c, whose float32 rows
+        x [c1 - c0, ldx] are in a device slot.  The rows of chunk c + 1 are staged by the host threads and copied on
+        a side stream into the other slot while chunk c is computed; a slot is overwritten only after the work on
+        the chunk before has been enqueued and has run (event `slot_free`)."""
+        torch = self.eng.torch
+        main = torch.cuda.current_stream(self.eng.dev)
+        copy = self.copy_stream
+        copy.wait_stream(main)  # earlier readers of the slots are done before they are overwritten
+        with self.stager.pieces(self.host_X, self.chunks) as pieces:
+            pieces = iter(pieces)
+
+            def upload(c):
+                s, (c0, c1) = c % 2, self.chunks[c]
+                if c >= 2:
+                    copy.wait_event(self.slot_free[s])
+                done = c0
+                with torch.cuda.stream(copy):
+                    while done < c1:
+                        _, r0, r1, host, release = next(pieces)
+                        self.slots[s][r0 - c0 : r1 - c0].copy_(host, non_blocking=True)
+                        ev = torch.cuda.Event()
+                        ev.record(copy)
+                        release(ev)
+                        done = r1
+                    self.slot_ready[s].record(copy)
+
+            upload(0)
+            for c, (c0, c1) in enumerate(self.chunks):
+                s = c % 2
+                main.wait_event(self.slot_ready[s])
+                body(c, c0, c1, self.slots[s][: c1 - c0])
+                self.slot_free[s].record(main)
+                if c + 1 < len(self.chunks):
+                    upload(c + 1)
+
+    def shadows(self, c: int, x, backend, selective):
+        """(shadows, row order) for a search of chunk c (rows x) with `backend`; (None, None) for the SIMT search.
+        An epoch search (`selective` True or False) reads them sorted by the chunk's K2 order iff it is selective, a
+        post-training search (`selective` None) iff some epoch's search was.  D > 256 chunks are never selective, so
+        they stay in natural order, where the resident fit keeps them too."""
+        if backend[0] != nat.BMU_TENSOR:
+            return None, None
+        eng, torch = self.eng, self.eng.torch
+        need_lo = backend[1] == 3
+        self._sorted_search |= bool(selective)
+        c0, c1 = self.chunks[c]
+        perm = self.row_perm[c0:c1] if (self._sorted_search if selective is None else selective) else None
+        if self._x16 is None or (need_lo and self._x16[1] is None):
+            self._x16 = (torch.empty((self.chunk_rows, eng.ld16), dtype=torch.float16, device=eng.dev),
+                         torch.empty((self.chunk_rows, eng.ld16), dtype=torch.float16, device=eng.dev) if need_lo else None,
+                         torch.empty(self.chunk_rows, dtype=torch.float32, device=eng.dev))
+        n = c1 - c0
+        hi, lo, xn = self._x16[0][:n], (self._x16[1][:n] if need_lo else None), self._x16[2][:n]
+        with eng._Phase(eng, "prepare_x16"):
+            eng._prepare_x16(x, n, hi, lo, xn, perm)
+        return (hi, lo, xn), perm
+
+    def has_order(self, c: int) -> bool:
+        return self._chunks_sorted
+
+    def after_k2(self, c: int, order, eligible: bool) -> None:
+        """Keep chunk c's K2 order (`order`, chunk-local) for the shadows of its next epoch."""
+        c0, c1 = self.chunks[c]
+        self.row_perm[c0:c1].copy_(order)
+        self._chunks_sorted = True
+
+    def shift_row(self):
+        return self.start_rows(np.zeros(1, dtype=np.int64))[0].float()  # float32 -> float64 -> float32 is exact
+
+    def start_rows(self, rows: np.ndarray):
+        """float64 [len(rows), ldx] copies of the given local sample rows, rounded through float32 like the chunks."""
+        eng = self.eng
+        out = np.zeros((len(rows), eng.ldx), dtype=np.float64)
+        out[:, : eng.D] = np.asarray(self.host_X[rows]).astype(np.float32)
+        return eng.torch.from_numpy(out).to(eng.dev)
+
+    def close(self) -> None:
+        if self.stager is not None:
+            # no copy may still read the page-locked ring when it is unregistered
+            self.eng.torch.cuda.synchronize(self.eng.dev)
+            self.stager.close()
+            self.stager = None
+        self.host_X = self.slots = self.row_perm = self._x16 = None

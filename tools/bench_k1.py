@@ -30,8 +30,7 @@ def main():
         eng = DeviceEngine(device="cuda:0", bmu_backend="tensor")
         eng.load_device_data(X)
         eng.init_map_from_rows(np.random.default_rng(0).choice(rows, m, replace=False), capacity=m)
-        eng._ensure_x16(True)
-        x16 = (eng.X16_hi, eng.X16_lo, eng.xnorm16)
+        x16, _ = eng.samples.shadows(0, eng.X, (nat.BMU_TENSOR, 3), False)
         idx = torch.empty((rows, 1), dtype=torch.int32, device=dev)
         eng.enable_profiling(True)
         for _ in range(2):

@@ -103,7 +103,7 @@ def compare(torch, name, n, d, side, epochs, warmup, stream_rows):
         timed_epoch(torch, res, e, m)
         timed_epoch(torch, st, e, m)
     t_res, t_st = [], []
-    stager = st._stager
+    stager = st.samples.stager
     b0, f0 = stager.bytes_staged, stager.fill_seconds
     for e in range(warmup, warmup + epochs):  # alternately, from the same epoch count
         t_res.append(timed_epoch(torch, res, e, m))

@@ -43,8 +43,7 @@ def main():
     print("epoch  " + "  ".join(f"k={s:<7g}" for s in scales) + "   (mismatching winners with exact rel. gap > 1e-7 | flagged | ambiguous)")
     for e in range(args.epochs):
         W = eng.W[eng.cur]
-        eng._ensure_x16(True)
-        x16 = (eng.X16_hi, eng.X16_lo, eng.xnorm16)
+        x16, _ = eng.samples.shadows(0, eng.X, (nat.BMU_TENSOR, 3), False)
         ref = torch.empty((eng.N, 1), dtype=torch.int32, device=dev)
         eng.strict_ties = True
         eng._run_bmu(eng.X, eng.N, eng.ldx, None, W, eng.M, 1, False, ref, None, backend=(nat.BMU_SIMT, 0))

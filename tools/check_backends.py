@@ -35,8 +35,7 @@ def main():
     total_bad = 0
     for e in range(epochs):
         W = eng.W[eng.cur]
-        eng._ensure_x16(True)
-        x16 = (eng.X16_hi, eng.X16_lo, eng.xnorm16)
+        x16, _ = eng.samples.shadows(0, eng.X, (nat.BMU_TENSOR, 3), False)
         ref = torch.empty((rows, 1), dtype=torch.int32, device=dev)
         got = torch.empty((rows, 1), dtype=torch.int32, device=dev)
         eng.strict_ties = True

@@ -71,7 +71,7 @@ def main():
             total_bad += compare(eng, cls, ref, d, m, W, "classic tensor search on sorted shadows vs simt")
             total_bad += compare(eng, got, ref, d, m, W, "selective search vs simt")
         r = eng.epoch(sigma_at(e, m), True, False)
-        print(f"epoch {e} done: live {int((r['counts'] > 0).sum())} sorted {eng.row_perm is not None} age {eng._sort_age}", flush=True)
+        print(f"epoch {e} done: live {int((r['counts'] > 0).sum())} sorted {eng.row_perm is not None} age {eng.samples.age}", flush=True)
     print("OK" if total_bad == 0 else "MISMATCH")
     eng.close()
 

@@ -24,5 +24,5 @@ print('resident epoch ms', t(lambda: eng.epoch(sigma_at(5,m),True,False)))
 print('epoch_from_host ms', t(lambda: eng.epoch_from_host(host,sigma_at(5,m),True,False)))
 print('epoch_from_host 4M chunks ms', t(lambda: eng.epoch_from_host(host,sigma_at(5,m),True,False,chunk_rows=1<<22)))
 def serial():
-    X.copy_(host,non_blocking=True); eng.X16_hi=None; eng.epoch(sigma_at(5,m),True,False)
+    X.copy_(host,non_blocking=True); eng.samples.X16_hi=eng.samples.row_perm=None; eng.epoch(sigma_at(5,m),True,False)
 print('serial copy+epoch ms', t(serial))
