@@ -1502,6 +1502,14 @@ int launch_cfg_cl(const dbgsom_bmu_args& a, const BmuWorkspace& ws, cudaStream_t
       fprintf(stderr, "dbgsom: K1 takes wnorm through the bias k-step, E = %g\n", e);
     }
   }
+  if (getenv("DBGSOM_TC_VERBOSE")) {  // once per process and kernel form (the static is per instantiation)
+    static bool said = false;
+    if (!said) {
+      said = true;
+      fprintf(stderr, "dbgsom: K1 form npass=%d nb=%d bn=%d res_kb=%d akb=%d cl=%d pair=%d sel=%d tb=%d sgt=%d\n", NPASS, NB,
+              BN, RES_KB, AKB, CL, (int)PAIR, SEL, (int)TB, SGT);
+    }
+  }
   auto kern = bmu_cand_tensor_kernel<NPASS, NB, BN, RES_KB, AKB, CL, PAIR, SEL, TB, SGT>;
   DBGSOM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   const int KB = (int)(a.ld16 / BK);
@@ -1565,14 +1573,7 @@ int launch_cfg(const dbgsom_bmu_args& a, const BmuWorkspace& ws, cudaStream_t s)
   const int cl = ceil_div<int64_t>(a.N, BM) < sm_count() ? 1 : cluster_size();
   if constexpr (AKB > 0) {  // CTA pairs (cta_group::2) whenever the sample tile is tensor-memory resident; DBGSOM_TC_PAIR=0 disables
     static const bool pair = getenv("DBGSOM_TC_PAIR") == nullptr || atoi(getenv("DBGSOM_TC_PAIR")) != 0;
-    if (pair && cl >= 2) {
-      static bool said = false;
-      if (!said && getenv("DBGSOM_TC_VERBOSE")) {
-        said = true;
-        fprintf(stderr, "dbgsom: K1 runs as CTA pairs (cta_group::2)\n");
-      }
-      return launch_cfg_cl<NPASS, NB, BN, RES_KB, AKB, 2, true>(a, ws, s);
-    }
+    if (pair && cl >= 2) return launch_cfg_cl<NPASS, NB, BN, RES_KB, AKB, 2, true>(a, ws, s);
   }
   if (cl == 4) return launch_cfg_cl<NPASS, NB, BN, RES_KB, AKB, 4>(a, ws, s);
   if (cl == 2) return launch_cfg_cl<NPASS, NB, BN, RES_KB, AKB, 2>(a, ws, s);

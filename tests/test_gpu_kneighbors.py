@@ -3,10 +3,10 @@ import numpy as np
 import pytest
 
 import _datasets
+from _topk_reference import GAP, assert_topk_parity, bench_like_maps
 from oracle import som_oracle as O
 
 pytestmark = pytest.mark.gpu
-GAP = 1e-6
 KS = (3, 4, 5, 8, 16)
 
 
@@ -14,58 +14,6 @@ def engine(**kw):
     from dbgsom_b200.engine import DeviceEngine
 
     return DeviceEngine(**kw)
-
-
-def exact_topk(X, W, k):
-    """Indices (lowest index first on exact ties) and squared distances of the k + 1 nearest prototypes, by direct
-    differences in float64.  The float64 expansion preselects k + 65 candidates; it cannot order prototypes whose
-    distances differ by less than its cancellation error (samples sitting on a cluster of near-copies), so the
-    candidates are ranked again by direct differences."""
-    X64 = np.asarray(X, dtype=np.float64)
-    W64 = np.asarray(W, dtype=np.float64)
-    kk = min(k + 65, W.shape[0])
-    _, cand = O.bmu_expansion(X64, W64, kk)
-    cand = np.sort(cand.reshape(len(X), kk), axis=1)
-    d2 = np.empty((len(X), kk))
-    for s in range(0, len(X), 256):
-        diff = X64[s : s + 256, None, :] - W64[cand[s : s + 256]]
-        d2[s : s + 256] = np.einsum("nkd,nkd->nk", diff, diff)
-    order = np.argsort(d2, axis=1, kind="stable")[:, : min(k + 1, kk)]
-    d2 = np.take_along_axis(d2, order, axis=1)
-    return np.take_along_axis(cand, order, axis=1), d2, d2[:, :k]
-
-
-def assert_topk_parity(dist, idx, X, W, k, gap=GAP):
-    """Indices equal at every rank whose squared distance is more than `gap` (relative) away from its neighbours'
-    ranks; distances equal to float64 rounding of the direct-difference sum.  Returns the number of gated rows."""
-    assert idx.shape == dist.shape == (len(X), k)
-    ref_idx, d2, d2_direct = exact_topk(X, W, k)
-    scale = np.maximum(d2, 1e-300)
-    sep = np.ones_like(d2, dtype=bool)  # rank r is separated from rank r + 1
-    sep[:, :-1] = (d2[:, 1:] - d2[:, :-1]) > gap * scale[:, :-1]
-    if d2.shape[1] == k:  # k == M: nothing behind the last rank
-        sep[:, -1] = True
-    ok = sep[:, :k].copy()
-    ok[:, 1:] &= sep[:, : k - 1]
-    bad = np.argwhere((idx != ref_idx[:, :k]) & ok)
-    assert bad.size == 0, f"{len(bad)} (row, rank) mismatches outside near-ties, first {bad[:5].tolist()}"
-    # distances: exact where the index matches, within the gate elsewhere
-    same = idx == ref_idx[:, :k]
-    np.testing.assert_allclose(dist[same], np.sqrt(d2_direct[same]), rtol=1e-12, atol=1e-300)
-    np.testing.assert_allclose(dist, np.sqrt(d2_direct), rtol=gap)
-    assert (np.diff(dist, axis=1) >= 0).all()
-    # every returned index is a distinct prototype
-    srt = np.sort(idx, axis=1)
-    assert (srt[:, 1:] != srt[:, :-1]).all()
-    return int((~ok).any(axis=1).sum())
-
-
-def bench_like_maps(n, d, m, seed=11):
-    X = _datasets.gmm(n, d, 32, seed)
-    rng = np.random.default_rng(5)
-    W = X[rng.choice(n, m, replace=False)].astype(np.float64)
-    W += rng.normal(0.0, 0.01, size=W.shape) * np.abs(W).mean()
-    return X, W
 
 
 # "auto" picks the three-pass tensor search for every shape but the last (N * M * ldx >= 2^31, M >= 128).  The launch

@@ -106,3 +106,83 @@ def test_workspace_bytes():
             wide = lib.dbgsom_bmu_workspace_bytes(n, k)
             assert wide >= n * (4 * 32 + 1 + 4)
             assert wide - base >= n * 4 * (32 - nat.MAX_CAND) - 256  # tables are padded to 256 bytes
+
+
+# Runs in a process without a visible device, so that an argument check that stops refusing cannot launch a kernel on
+# fake pointers: the call then fails on the missing device instead.
+_REFUSALS = r"""
+import json, sys
+sys.path.insert(0, sys.argv[1])
+from dbgsom_b200 import _native as nat
+
+lib = nat.load()
+N, D, M = 1000, 64, 100
+cases = {}
+
+
+def args(n_bmu, backend, **kw):
+    a = nat.BmuArgs()
+    fake = iter(range(0x100000, 0x10000000, 0x10000))  # 16-byte aligned, never dereferenced
+    for name in ("d_X", "d_X16_hi", "d_X16_lo", "d_xnorm16", "d_W", "d_W32", "d_W16_hi", "d_W16_lo", "d_wnorm",
+                 "d_wmax", "d_proto_of_col", "d_idx", "d_dist", "d_stats", "d_workspace"):
+        setattr(a, name, next(fake))
+    a.N, a.D, a.ldx, a.ld16, a.M, a.Mpad = N, D, D, 64, M, 256
+    a.n_bmu, a.backend, a.n_pass, a.want_dist, a.select_granule = n_bmu, backend, 3, 1, 64
+    a.workspace_bytes = lib.dbgsom_bmu_workspace_bytes(N, n_bmu)
+    for name, value in kw.items():
+        setattr(a, name, value)
+    return a
+
+
+def run(a):
+    return [lib.dbgsom_bmu_candidates(a, None), lib.dbgsom_bmu_resolve(a, None), lib.dbgsom_bmu(a, None)]
+
+
+for k in (3, 16):
+    for be, be_name in ((nat.BMU_TENSOR, "tensor"), (nat.BMU_SIMT, "simt")):
+        tag = f"{be_name}-{k}"
+        cases[f"valid-{tag}"] = run(args(k, be))
+        cases[f"select-flag-{tag}"] = run(args(k, be, select=nat.SELECT_FLAG, d_tile_mask=0x20000000))
+        cases[f"select-refine-{tag}"] = run(args(k, be, select=nat.SELECT_REFINE, d_tile_mask=0x20000000))
+        cases[f"ties_any-{tag}"] = run(args(k, be, ties_any=1))
+        cases[f"tile_bound-{tag}"] = run(args(k, be, d_tile_bound=0x20000000))
+        cases[f"row_perm-{tag}"] = run(args(k, be, d_row_perm=0x20000000))
+        cases[f"more-than-M-{tag}"] = run(args(k, be, M=k - 1))
+        cases[f"top2-workspace-{tag}"] = run(args(k, be, workspace_bytes=lib.dbgsom_bmu_workspace_bytes(N, 2)))
+    cases[f"one-pass-tensor-{k}"] = run(args(k, nat.BMU_TENSOR, n_pass=1))
+for be in (nat.BMU_TENSOR, nat.BMU_SIMT):
+    cases[f"n_bmu-17-{be}"] = run(args(17, be, workspace_bytes=lib.dbgsom_bmu_workspace_bytes(N, 16)))
+print(json.dumps(cases))
+"""
+
+
+def test_topk_abi_refusals():
+    """The C ABI refuses what the top-k search (n_bmu > 2) does not support: the selective search, ties_any, tile
+    bounds and a sorted sample order are top-1 tools, the tensor front end runs top-k in its three-pass form only, and
+    the candidate table needs 32 slots per row."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    from dbgsom_b200 import build as builder
+
+    builder.build()
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    res = subprocess.run([sys.executable, "-c", _REFUSALS, root], env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
+                         capture_output=True, text=True, timeout=120)
+    assert res.returncode == 0, res.stderr[-2000:]
+    cases = json.loads(res.stdout.strip().splitlines()[-1])
+    badarg, workspace, unsupported = -1, -2, -3  # DBGSOM_E_*
+    expect = {"select-flag": badarg, "select-refine": badarg, "ties_any": badarg, "tile_bound": badarg,
+              "row_perm": badarg, "more-than-M": badarg, "top2-workspace": workspace, "one-pass-tensor": unsupported,
+              "n_bmu-17": badarg}
+    assert len(cases) == 2 * 2 * 8 + 2 + 2
+    for name, codes in cases.items():
+        if name.startswith("valid"):
+            # passes every argument check and fails only for want of a device: the refusals below are the checks'
+            assert codes[0] not in (0, badarg, workspace, unsupported) and codes[1] not in (0, badarg, workspace,
+                                                                                              unsupported), (name, codes)
+            continue
+        want = next(v for key, v in expect.items() if name.startswith(key + "-"))
+        assert codes == [want] * 3, (name, codes)
